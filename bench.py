@@ -7,7 +7,7 @@ A "step" is one pass of the hot path (frontend -> DFSMN -> on-device post-proces
 segment frame pairs) over one batch of chunks per GPU.  Streams shard across ranks with no
 data-path collective (weak scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--chunks B] [--impl vadx|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--chunks B] [--impl vadx|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 `value`  : device-resident inputs, CUDA-event timed, max over ranks.
@@ -49,7 +49,39 @@ def parse():
     ap.add_argument("--no-families", action="store_true", help="skip the short RTFx runs of the other model families")
     ap.add_argument("--sustain-seconds", type=float, default=4.0,
                     help="extra device-resident leg of about this many seconds (steady-state clocks / power); 0 = skip")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed device-resident step returned (rank 0's streams) as DIR/<name>.npy, "
+                         "float32; inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "vadx":
+        ap.error("--dump-outputs applies to --impl vadx")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, probs, dec, cnt, seg, n_valid):
+    """One step's results of run_vad_streams as float32 .npy files (every value is exact in float32).  Segment slots
+    past a stream's count and decisions past its valid frames were never written by the device and are set to -1 and 0,
+    so the files depend only on what was computed.  Above DUMP_LIMIT_BYTES a fixed seeded sample of streams is written,
+    the same rows of every array, with their indices in stream_index.npy."""
+    import numpy as np
+    probs, dec, cnt, seg, n_valid = (t.cpu().numpy().copy() for t in (probs, dec, cnt, seg, n_valid))
+    seg[np.arange(seg.shape[1])[None, :] >= np.minimum(cnt, seg.shape[1])[:, None]] = -1
+    dec[np.arange(dec.shape[1])[None, :] >= n_valid[:, None]] = 0
+    out = {"frame_probs": probs, "decisions": dec, "seg_count": cnt, "segments": seg}
+    S = cnt.shape[0]
+    per_stream = 4 * (sum(a[0].size for a in out.values()) + 1)
+    if S * per_stream > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.RandomState(0).choice(S, DUMP_LIMIT_BYTES // per_stream, replace=False))
+        out = {k: a[idx] for k, a in out.items()}
+        out["stream_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float32))
 
 
 def ncu_traffic_bytes(kernel_substr):
@@ -475,6 +507,7 @@ def run_vadx(args):
         torch.cuda.synchronize()
 
     sampler = ClockSampler(local_rank)
+    last = {}
 
     def timed(fn, steps, warmup):
         for _ in range(warmup):
@@ -483,8 +516,11 @@ def run_vadx(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sampler.active.set()
         e0.record(stream)
-        for _ in range(steps):
-            fn()
+        for i in range(steps):
+            if i < steps - 1:
+                fn()
+            else:
+                last["out"] = fn()      # kept from the last step only: no two steps' outputs are alive at once
         e1.record(stream)
         barrier()
         sampler.active.clear()
@@ -509,6 +545,9 @@ def run_vadx(args):
     stages = lib.profile_collect()
     kernel_records = lib.profile_collect_kernels()
     lib.profile_enable(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last["out"])
+    last.clear()
     # ---- the same step back to back for a few seconds: the timed region above is ~0.1 s, this leg shows the step time and
     # the clocks once the part sits at its power / thermal steady state (reported next to `value`, not as it)
     sustained = None

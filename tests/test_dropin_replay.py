@@ -2,7 +2,8 @@
 session that answers every run() with what the vadx sessions produced on the B200 for exactly that call
 (tests/golden/dropin_vadx_outputs.npz, written by tests/test_gpu_dropin.py) -- after checking that the feed the script
 built is bit-for-bit the one stage A fed -- and the two text files each script writes must equal the files of the
-all-reference run.  Needs /root/reference (this container); skipped on the GPU box."""
+all-reference run.  The replay needs a checkout of the upstream reference project (oracle/ref_loader.py) and skips
+without one; the check of the committed transcript runs everywhere."""
 import os
 
 import numpy as np
@@ -11,8 +12,8 @@ import pytest
 from oracle import ref_loader as RL
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-pytestmark = pytest.mark.skipif(not RL.reference_available() or not os.path.exists(os.path.join(GOLD, "dropin_vadx_outputs.npz")),
-                                reason="needs /root/reference and the stage-A outputs recorded on a B200")
+needs_reference = pytest.mark.skipif(not RL.reference_available(),
+                                     reason="replays into the upstream reference scripts, which are not part of this repository")
 
 
 @pytest.fixture(scope="module")
@@ -23,6 +24,7 @@ def replayed():
     return tr, vx, dropin.replay_scripts(tr, vx)
 
 
+@needs_reference
 @pytest.mark.parametrize("family,n_calls", [("firered", 6), ("fsmn", 8), ("silero", 175)])
 def test_unmodified_script_on_vadx_outputs_writes_the_reference_files(replayed, family, n_calls):
     tr, vx, res = replayed
