@@ -4,19 +4,15 @@
 #include "model.hpp"
 
 // ------------------------------------------------------------------------------------------ FireRed
-struct FireRedHP {
-  int idim, R, M, H, P, N1, S1, N2, S2, odim, n_fft, win, hop, n_mels;
-  int n_taps() const { return win < n_fft ? win : n_fft; }
-  int n_bins() const { return n_fft / 2 + 1; }
-  int ld_basis() const { return (int)round_up(2 * n_bins(), 4); }
-  int ld_power() const { return (int)round_up(n_bins(), 4); }
+struct FireRedHP : FrontendGeom {
+  int idim, R, M, H, P, N1, S1, N2, S2, odim;
   int frames(int64_t L) const { return L < n_taps() ? 0 : (int)(1 + (L - n_taps()) / hop); }
 };
 
 static int firered_hp(const vadx_model* m, FireRedHP* h) {
   VADX_REQUIRE(m->hp.size() == 14, "firered: expected 14 hyper-parameters, got %zu", m->hp.size());
   const int32_t* v = m->hp.data();
-  *h = FireRedHP{v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8], v[9], v[10], v[11], v[12], v[13]};
+  *h = FireRedHP{{v[10], v[11], v[12], v[13]}, v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8], v[9]};
   VADX_REQUIRE(h->idim == h->n_mels, "firered: idim (%d) must equal n_mels (%d)", h->idim, h->n_mels);
   VADX_REQUIRE(h->R >= 1 && h->M >= 1 && h->H >= 1 && h->P >= 1 && h->N1 >= 1 && h->S1 >= 1 && h->N2 >= 0 &&
                    h->odim >= 1 && h->odim <= 8 && h->hop >= 1 && h->n_fft >= 2,
@@ -24,10 +20,16 @@ static int firered_hp(const vadx_model* m, FireRedHP* h) {
   return VADX_OK;
 }
 
+// DFT over derived.bins_used only; no centre pad: frames start at sample 0
+static Frontend firered_frontend(const vadx_model* m, const FireRedHP& h) {
+  return Frontend{h, (int)m->scalar("derived.bins_used", (double)h.n_bins()), 0, 1.0f, false, VADX_PREEMPH_ZERO_HISTORY,
+                  VADX_TC_FMT_F16, VADX_FLOOR_CLAMP, (float)m->scalar("frontend.log_floor", 1e-7), frontend_rate_scale(m),
+                  false};
+}
+
 int firered_finalize(vadx_model* m) {
   FireRedHP h;
   VADX_TRY(firered_hp(m, &h));
-  VADX_TRY(m->upload_raw("frontend.basis", (int64_t)h.n_taps() * h.ld_basis(), VADX_DT_F32));
   // bins the filterbank actually reads: the Kaldi-style bank gives zero weight to DC and Nyquist, so the
   // DFT only has to produce bins [0, bins_used) (FireRed: 200 of 201 -> 400 columns = exactly five 80-wide tiles)
   int bins_used = 1;
@@ -44,41 +46,7 @@ int firered_finalize(vadx_model* m) {
     bins_used = std::min(bins_used, h.n_bins());
     m->scalars["derived.bins_used"] = bins_used;
   }
-  if (vadx_stft_tc_supported(h.n_taps(), bins_used)) {
-    // tensor-core DFT image: pre-emphasis folded into the 2-term fp16 basis (stft_tc.cu)
-    const double preemph = m->scalar("frontend.preemph", 0.97);
-    size_t bytes = 0;
-    const float* hb = m->find("frontend.basis")->f32();
-    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, h.ld_basis(), h.n_taps(), bins_used, preemph, 1.0, VADX_TC_FMT_F16, nullptr, 0, &bytes));
-    std::vector<uint8_t> img(bytes);
-    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, h.ld_basis(), h.n_taps(), bins_used, preemph, 1.0, VADX_TC_FMT_F16, img.data(),
-                                         img.size(), &bytes));
-    VADX_TRY(m->upload("frontend.basis#TC", img.data(), img.size()));
-  }
-  VADX_TRY(m->upload_raw("frontend.mel_start", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_len", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_w", -1, VADX_DT_F32));
-  {
-    // the filterbank as a dense [n_mels][bins_used] layer for the tensor-core path (log + floor in the epilogue)
-    const HostTensor* ms = m->find("frontend.mel_start");
-    const HostTensor* ml = m->find("frontend.mel_len");
-    const HostTensor* mw = m->find("frontend.mel_w");
-    if (ms && ml && mw && ms->numel() == h.n_mels && ml->numel() == h.n_mels && vadx_tc_supported(bins_used, h.n_mels)) {
-      const int max_len = (int)(mw->numel() / h.n_mels);
-      const int32_t* a = reinterpret_cast<const int32_t*>(ms->bytes.data());
-      const int32_t* b = reinterpret_cast<const int32_t*>(ml->bytes.data());
-      std::vector<float> dense((size_t)h.n_mels * bins_used, 0.f);
-      for (int i = 0; i < h.n_mels; ++i)
-        for (int j = 0; j < b[i] && a[i] + j < bins_used; ++j) dense[(size_t)i * bins_used + a[i] + j] = mw->f32()[(size_t)i * max_len + j];
-      size_t bytes = 0;
-      VADX_TRY(vadx_pack_weight_tc(dense.data(), h.n_mels, bins_used, nullptr, 0, &bytes));
-      std::vector<uint8_t> img(bytes);
-      VADX_TRY(vadx_pack_weight_tc(dense.data(), h.n_mels, bins_used, img.data(), img.size(), &bytes));
-      VADX_TRY(m->upload("frontend.mel#TC", img.data(), img.size()));
-      std::vector<float> floor_v((size_t)h.n_mels, (float)m->scalar("frontend.log_floor", 1e-7));
-      VADX_TRY(m->upload("frontend.mel_floor", floor_v.data(), floor_v.size() * sizeof(float)));
-    }
-  }
+  VADX_TRY(firered_frontend(m, h).finalize(m));
   VADX_TRY(m->upload_linear("dfsmn.fc1.0.weight", h.H, h.idim));
   VADX_TRY(m->upload_raw("dfsmn.fc1.0.bias", h.H, VADX_DT_F32));
   VADX_TRY(m->upload_linear("dfsmn.fc2.0.weight", h.P, h.H));
@@ -113,16 +81,10 @@ int firered_check(const vadx_model* m) {
   FireRedHP h;
   return firered_hp(m, &h);
 }
-// IN_SAMPLE_RATE != 16000 (Export_FireRedVAD.py:389-393): scale = 1 / (in_rate / 16000), samples after the
-// in-graph linear resampler = floor(L * scale)
-static double firered_rate_scale(const vadx_model* m) {
-  const double in_rate = m->scalar("frontend.in_sample_rate", 16000.0);
-  return in_rate == 16000.0 ? 1.0 : 1.0 / (in_rate / 16000.0);
-}
 int firered_frames(const vadx_model* m, int64_t n_samples, int32_t* out) {
   FireRedHP h;
   VADX_TRY(firered_hp(m, &h));
-  const double sc = firered_rate_scale(m);
+  const double sc = frontend_rate_scale(m);
   *out = h.frames(sc == 1.0 ? n_samples : vadx_resample_out_len(n_samples, sc));
   return VADX_OK;
 }
@@ -154,7 +116,8 @@ int firered_run(vadx_model* m, bool dry, const void* const* in, void* const* out
   }
   const int64_t cache_stream = (int64_t)h.P * (h.N1 - 1) * h.S1;
   const int64_t cache_layer = S_all * cache_stream;
-  const double rate_scale = firered_rate_scale(m);
+  const Frontend fe = firered_frontend(m, h);
+  const double rate_scale = fe.rate_scale;
   const int64_t L16 = rate_scale == 1.0 ? L : vadx_resample_out_len(L, rate_scale);   // samples at the model's 16 kHz
   const int T = h.frames(L16);
   VADX_REQUIRE(T >= 1, "firered: %lld samples are shorter than one %d-sample frame", (long long)L16, h.n_taps());
@@ -180,11 +143,6 @@ int firered_run(vadx_model* m, bool dry, const void* const* in, void* const* out
     set_error("firered: workspace of %zu bytes is smaller than the %zu needed", ws_bytes, ws.off);
     return VADX_ENOMEM;
   }
-  const float preemph = (float)m->scalar("frontend.preemph", 0.97);
-  const float floor_v = (float)m->scalar("frontend.log_floor", 1e-7);
-  const HostTensor* melw = m->find("frontend.mel_w");
-  const int mel_max = (int)(melw->numel() / h.n_mels);
-  const int nb_used = (int)m->scalar("derived.bins_used", (double)h.n_bins());
 
   for (int64_t s0 = 0; s0 < S_all; s0 += slab) {
     const int64_t S = std::min(slab, S_all - s0);
@@ -196,39 +154,7 @@ int firered_run(vadx_model* m, bool dry, const void* const* in, void* const* out
     float* memA = memA0;
     float* memB = memB0;
     const bool use_tc = m->scalar("engine.use_tc", 1.0) != 0.0 && rows > kSkinnyMaxRows;
-    const uint8_t* stft_img = use_tc ? m->d<uint8_t>("frontend.basis#TC") : nullptr;
-    if (rate_scale != 1.0) {
-      // in-graph resampler: downsample before the pre-emphasis, upsample after it (Export_FireRedVAD.py:431-449)
-      const int pre = preemph > 0.f ? VADX_PREEMPH_ZERO_HISTORY : 0;
-      if (rate_scale < 1.0) {
-        VADX_TRY(vadx_prep_audio(d_audio, VADX_DT_I16, S, L, L, 1.0f, 0, 0, 0.f, 0, sig2, Lp, st));
-        VADX_TRY(vadx_resample_linear_f32(sig2, Lp, L, S, rate_scale, sig, Lp, 0, st));
-        VADX_TRY(vadx_prep_audio(sig, VADX_DT_F32, S, L16, Lp, 1.0f, 0, pre, preemph, 0, sig2, Lp, st));
-      } else {
-        VADX_TRY(vadx_prep_audio(d_audio, VADX_DT_I16, S, L, L, 1.0f, 0, pre, preemph, 0, sig, Lp, st));
-        VADX_TRY(vadx_resample_linear_f32(sig, Lp, L, S, rate_scale, sig2, Lp, 0, st));
-      }
-      VADX_TRY(vadx_stft_power_f32(sig2, Lp, S, T, h.hop, h.n_taps(), m->d<float>("frontend.basis"), h.ld_basis(),
-                                   nb_used, power, h.ld_power(), st));
-    } else if (stft_img && (L % 8) == 0 && (h.hop % 8) == 0 && aligned16(d_audio)) {
-      // int16 audio -> power in one tensor-core kernel (exact sample split, folded pre-emphasis)
-      VADX_TRY(vadx_stft_power_tc_i16_ex(d_audio, L, L, S, T, h.hop, h.n_taps(), stft_img, nb_used, power, h.ld_power(), 0,
-                                         nullptr, nullptr, nullptr, 0, T, 1.0f, VADX_TC_FMT_F16, st));
-    } else {
-      VADX_TRY(vadx_prep_audio(d_audio, VADX_DT_I16, S, L, L, 1.0f, 0, preemph > 0.f ? VADX_PREEMPH_ZERO_HISTORY : 0,
-                               preemph, 0, sig, Lp, st));
-      VADX_TRY(vadx_stft_power_f32(sig, Lp, S, T, h.hop, h.n_taps(), m->d<float>("frontend.basis"), h.ld_basis(),
-                                   nb_used, power, h.ld_power(), st));
-    }
-    if (use_tc && m->d<uint8_t>("frontend.mel#TC")) {
-      // log-mel as a dense tensor-core layer: [rows][bins] x [bins][n_mels], log(max(., floor)) in the epilogue
-      VADX_TRY(vadx_linear_tc_f32(power, h.ld_power(), m->d<uint8_t>("frontend.mel#TC"), m->d<float>("frontend.mel_floor"),
-                                  nullptr, 0, feat, h.n_mels, rows, nb_used, h.n_mels, VADX_ACT_LOG_CLAMP, st));
-    } else {
-      VADX_TRY(vadx_mel_log_f32(power, h.ld_power(), rows, nb_used, h.n_mels, m->d<int32_t>("frontend.mel_start"),
-                                m->d<int32_t>("frontend.mel_len"), m->d<float>("frontend.mel_w"), mel_max,
-                                VADX_FLOOR_CLAMP, floor_v, feat, h.n_mels, st));
-    }
+    VADX_TRY(fe.run(m, d_audio, S, L, T, FrontendBufs{sig, sig2, Lp, power, nullptr, nullptr, feat}, st));
     auto lin = [&](const float* x, int n_in, const std::string& w, const char* b, const float* res, float* y, int n_out,
                    int act) -> int {
       const uint8_t* img = use_tc ? m->d<uint8_t>(w + "#TC") : nullptr;

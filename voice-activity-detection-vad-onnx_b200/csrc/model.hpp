@@ -243,6 +243,156 @@ struct vadx_model {
   bool has(const std::string& n) const { return host.count(n) != 0; }
 };
 
+// ------------------------------------------------------------------------------------------ log-mel frontend
+// int16 audio -> power spectrum -> log-mel rows, shared by FireRed, FSMN and MarbleNet: the in-graph resampler path, the
+// int16 tensor-core STFT or the fp32 FFMA STFT, then log-mel on the tensor cores or the sparse filterbank kernel.  Its
+// tensors are "frontend.basis" (fp32 [n_taps][ld_basis], re/im interleaved) and the sparse filterbank "frontend.mel_start" /
+// "mel_len" / "mel_w".
+
+// framing: the window's n_taps non-zero taps start first_tap samples into the n_fft-point frame
+struct FrontendGeom {
+  int n_fft, win, hop, n_mels;
+  int n_taps() const { return win < n_fft ? win : n_fft; }
+  int first_tap() const { return win < n_fft ? (n_fft - win) / 2 : 0; }
+  int n_bins() const { return n_fft / 2 + 1; }
+  int ld_basis() const { return (int)round_up(2 * n_bins(), 4); }
+  int ld_power() const { return (int)round_up(n_bins(), 4); }
+  int pad_left() const { return n_fft / 2 - first_tap(); }  // centre pad ahead of the first tap
+};
+
+struct FrontendBufs {  // the caller's workspace
+  float* sig;          // [S][Lp] prepped fp32 signal
+  float* sig2;         // [S][Lp] second signal (resampler only)
+  int64_t Lp;
+  float* power;        // [S*T][ld_power]
+  float* mean;         // [S] row means (remove_dc only)
+  int32_t* mean_int;   // [S]
+  float* mel;          // [S*T][n_mels] log-mel output
+};
+
+// What differs between the models' frontends.  The tensor-core paths run when engine.use_tc is set and S*T exceeds
+// kSkinnyMaxRows; the int16 tensor-core STFT also needs L, hop and pad_left to be multiples of 8 and 16-byte aligned audio.
+struct Frontend {
+  FrontendGeom g;
+  int n_bins;          // DFT bins computed (<= g.n_bins())
+  int pad_left;        // frame t starts at sample t*hop - pad_left, zeros outside the clip
+  float in_scale;      // int16 -> fp32 sample scale; the tensor-core STFT scales the power by its square instead
+  bool remove_dc;      // each row's mean removed before the pre-emphasis
+  int preemph_mode;    // VADX_PREEMPH_* of the fp32 paths
+  int tc_format;       // VADX_TC_FMT_* of the tensor-core DFT image
+  int floor_mode;      // VADX_FLOOR_*: ln(max(mel, floor)) or ln(mel + floor)
+  float floor_value;
+  double rate_scale;   // in-graph resampler, 1 = none
+  bool keep_signal;    // the prepped fp32 signal is produced on every path (read after the frontend)
+
+  // uploads the basis, its tensor-core image, the mel tables and the dense tensor-core mel image
+  int finalize(vadx_model* m) const;
+  // audio [S][L] int16 (L at the input rate) -> b.mel [S*T][n_mels] on stream st
+  int run(vadx_model* m, const int16_t* audio, int64_t S, int64_t L, int T, const FrontendBufs& b, cudaStream_t st) const;
+};
+
+// IN_SAMPLE_RATE != 16000 (Export_FireRedVAD.py:389-393, Export_NVIDIA_MarbleNet_VAD.py:180-183): scale = 1 / (in_rate /
+// 16000), the in-graph linear resampler leaves floor(L * scale) samples at the model's 16 kHz
+inline double frontend_rate_scale(const vadx_model* m) {
+  const double in_rate = m->scalar("frontend.in_sample_rate", 16000.0);
+  return in_rate == 16000.0 ? 1.0 : 1.0 / (in_rate / 16000.0);
+}
+
+inline int Frontend::finalize(vadx_model* m) const {
+  VADX_TRY(m->upload_raw("frontend.basis", (int64_t)g.n_taps() * g.ld_basis(), VADX_DT_F32));
+  if (vadx_stft_tc_supported(g.n_taps(), n_bins)) {
+    // tensor-core DFT image: the pre-emphasis folded into the 2-term basis; a scale such as 1/32768 stays out of it (fp16
+    // range) and multiplies the power instead
+    const double preemph = m->scalar("frontend.preemph", 0.97);
+    const float* hb = m->find("frontend.basis")->f32();
+    size_t bytes = 0;
+    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, g.ld_basis(), g.n_taps(), n_bins, preemph, 1.0, tc_format, nullptr, 0, &bytes));
+    std::vector<uint8_t> img(bytes);
+    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, g.ld_basis(), g.n_taps(), n_bins, preemph, 1.0, tc_format, img.data(), img.size(),
+                                         &bytes));
+    VADX_TRY(m->upload("frontend.basis#TC", img.data(), img.size()));
+  }
+  VADX_TRY(m->upload_raw("frontend.mel_start", g.n_mels, VADX_DT_I32));
+  VADX_TRY(m->upload_raw("frontend.mel_len", g.n_mels, VADX_DT_I32));
+  VADX_TRY(m->upload_raw("frontend.mel_w", -1, VADX_DT_F32));
+  return m->upload_mel_dense_tc(g.n_mels, n_bins, floor_value);
+}
+
+inline int Frontend::run(vadx_model* m, const int16_t* audio, int64_t S, int64_t L, int T, const FrontendBufs& b,
+                         cudaStream_t st) const {
+  const int64_t rows = S * T;
+  const bool use_tc = m->scalar("engine.use_tc", 1.0) != 0.0 && rows > kSkinnyMaxRows;
+  const float preemph = (float)m->scalar("frontend.preemph", 0.97);
+  const int pre = preemph > 0.f ? preemph_mode : 0;
+  const int64_t Lp = b.Lp;
+  const uint8_t* stft_img = use_tc ? m->d<uint8_t>("frontend.basis#TC") : nullptr;
+  if (rate_scale != 1.0) {
+    // in-graph resampler (Export_FireRedVAD.py:431-449, Export_NVIDIA_MarbleNet_VAD.py:236-254): downsample before the
+    // scale + pre-emphasis, upsample after it
+    if (rate_scale < 1.0) {
+      VADX_TRY(vadx_prep_audio(audio, VADX_DT_I16, S, L, L, 1.0f, 0, 0, 0.f, 0, b.sig2, Lp, st));
+      VADX_TRY(vadx_resample_linear_f32(b.sig2, Lp, L, S, rate_scale, b.sig, Lp, 0, st));
+      VADX_TRY(vadx_prep_audio(b.sig, VADX_DT_F32, S, vadx_resample_out_len(L, rate_scale), Lp, in_scale, remove_dc, pre,
+                               preemph, pad_left, b.sig2, Lp, st));
+    } else {
+      VADX_TRY(vadx_prep_audio(audio, VADX_DT_I16, S, L, L, in_scale, remove_dc, pre, preemph, 0, b.sig, Lp, st));
+      if (pad_left > 0) {  // centre pad around the resampled signal
+        cudaError_t e = cudaMemsetAsync(b.sig2, 0, (size_t)S * Lp * sizeof(float), st);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(frontend centre pad)");
+      }
+      VADX_TRY(vadx_resample_linear_f32(b.sig, Lp, L, S, rate_scale, b.sig2, Lp, pad_left, st));
+    }
+    VADX_TRY(vadx_stft_power_f32(b.sig2, Lp, S, T, g.hop, g.n_taps(), m->d<float>("frontend.basis"), g.ld_basis(), n_bins,
+                                 b.power, g.ld_power(), st));
+  } else {
+    const bool tc = stft_img && (L % 8) == 0 && (g.hop % 8) == 0 && (pad_left % 8) == 0 && aligned16(audio);
+    if (keep_signal || !tc)
+      VADX_TRY(vadx_prep_audio(audio, VADX_DT_I16, S, L, L, in_scale, remove_dc, pre, preemph, pad_left, b.sig, Lp, st));
+    if (tc) {
+      // framed DFT on the tensor cores straight from the int16 samples.  Frames reaching outside the clip and the mean
+      // removal take per-frame correction tables (vadx_pack_stft_dc_tc), built per chunk length at first use
+      const float* dc = nullptr;
+      int lo = 0, hi = T;
+      if (remove_dc || pad_left > 0) {
+        const std::string key = "frontend.dc#" + std::to_string((long long)L);
+        const std::string k_lo = key + ".lo", k_hi = key + ".hi";
+        if (!m->d<float>(key)) {
+          size_t n = 0;
+          const float* hb = m->find("frontend.basis")->f32();
+          VADX_TRY(vadx_pack_stft_dc_tc(hb, g.ld_basis(), g.n_taps(), n_bins, preemph, 1.0, L, g.hop, pad_left, T, nullptr, 0,
+                                        &n, &lo, &hi));
+          std::vector<float> tab(n);
+          VADX_TRY(vadx_pack_stft_dc_tc(hb, g.ld_basis(), g.n_taps(), n_bins, preemph, 1.0, L, g.hop, pad_left, T, tab.data(),
+                                        tab.size(), &n, &lo, &hi));
+          VADX_TRY(m->upload(key, tab.data(), tab.size() * sizeof(float)));
+          m->scalars[k_lo] = lo;
+          m->scalars[k_hi] = hi;
+        }
+        dc = m->d<float>(key);
+        lo = (int)m->scalar(k_lo.c_str(), 0.0);
+        hi = (int)m->scalar(k_hi.c_str(), (double)T);
+      }
+      if (remove_dc) VADX_TRY(vadx_stream_mean_i16(audio, L, L, S, b.mean, b.mean_int, st));
+      VADX_TRY(vadx_stft_power_tc_i16_ex(audio, L, L, S, T, g.hop, g.n_taps(), stft_img, n_bins, b.power, g.ld_power(), pad_left,
+                                         remove_dc ? b.mean : nullptr, remove_dc ? b.mean_int : nullptr, dc, lo, hi,
+                                         in_scale * in_scale, tc_format, st));
+    } else {
+      VADX_TRY(vadx_stft_power_f32(b.sig, Lp, S, T, g.hop, g.n_taps(), m->d<float>("frontend.basis"), g.ld_basis(), n_bins,
+                                   b.power, g.ld_power(), st));
+    }
+  }
+  if (use_tc && m->d<uint8_t>("frontend.mel#TC")) {
+    // log-mel as a dense tensor-core layer: [rows][bins] x [bins][n_mels], the floor / epsilon in the bias slot
+    return vadx_linear_tc_f32(b.power, g.ld_power(), m->d<uint8_t>("frontend.mel#TC"), m->d<float>("frontend.mel_floor"),
+                              nullptr, 0, b.mel, g.n_mels, rows, n_bins, g.n_mels,
+                              floor_mode == VADX_FLOOR_CLAMP ? VADX_ACT_LOG_CLAMP : VADX_ACT_LOG, st);
+  }
+  const int mel_max = (int)(m->find("frontend.mel_w")->numel() / g.n_mels);
+  return vadx_mel_log_f32(b.power, g.ld_power(), rows, n_bins, g.n_mels, m->d<int32_t>("frontend.mel_start"),
+                          m->d<int32_t>("frontend.mel_len"), m->d<float>("frontend.mel_w"), mel_max, floor_mode, floor_value,
+                          b.mel, g.n_mels, st);
+}
+
 
 // per-kind entry points
 int firered_check(const vadx_model* m);

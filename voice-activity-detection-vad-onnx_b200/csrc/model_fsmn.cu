@@ -25,28 +25,28 @@ int vadx_gather_windows_i16(const int16_t*, int64_t, int64_t, int, int64_t, int6
 }
 
 namespace {
-struct FsmnHP {
-  int input_dim, affine, layers, linear, proj, lorder, rorder, lstride, rstride, out_affine, out_dim, n_fft, win, hop,
-      n_mels, lfr_m, lfr_n;
-  int n_taps() const { return win < n_fft ? win : n_fft; }
-  int first_tap() const { return win < n_fft ? (n_fft - win) / 2 : 0; }
-  int n_bins() const { return n_fft / 2 + 1; }
-  int ld_basis() const { return (int)round_up(2 * n_bins(), 4); }
-  int ld_power() const { return (int)round_up(n_bins(), 4); }
-  int pad_left() const { return n_fft / 2 - first_tap(); }
+struct FsmnHP : FrontendGeom {
+  int input_dim, affine, layers, linear, proj, lorder, rorder, lstride, rstride, out_affine, out_dim, lfr_m, lfr_n;
   int frames(int64_t L) const { return (int)(L / hop + 1); }
 };
 
 int fsmn_hp(const vadx_model* m, FsmnHP* h) {
   VADX_REQUIRE(m->hp.size() == 17, "fsmn: expected 17 hyper-parameters, got %zu", m->hp.size());
   const int32_t* v = m->hp.data();
-  *h = FsmnHP{v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8], v[9], v[10], v[11], v[12], v[13], v[14], v[15], v[16]};
+  *h = FsmnHP{{v[11], v[12], v[13], v[14]}, v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7], v[8], v[9], v[10], v[15], v[16]};
   VADX_REQUIRE(h->input_dim == h->n_mels * h->lfr_m, "fsmn: input_dim %d != n_mels*lfr_m", h->input_dim);
   VADX_REQUIRE(h->layers >= 1 && h->layers <= 8 && h->proj >= 1 && h->lorder >= 1 && h->lstride >= 1 && h->hop >= 1 &&
                    h->lfr_n == 1 && h->out_dim >= 2,
                "fsmn: hyper-parameter out of range");
   VADX_REQUIRE(h->rorder == 0, "fsmn: the reference never applies conv_right (encoder.py:78-83); rorder must be 0");
   return VADX_OK;
+}
+
+// the mean removed before the pre-emphasis (the tensor-core STFT corrects for it in the frequency domain); the fp32 signal
+// is prepped on every path because the frame energy reads it
+Frontend fsmn_frontend(const vadx_model* m, const FsmnHP& h) {
+  return Frontend{h, h.n_bins(), h.pad_left(), 1.0f, true, VADX_PREEMPH_KEEP_FIRST, VADX_TC_FMT_BF16, VADX_FLOOR_CLAMP,
+                  (float)m->scalar("frontend.log_floor", 1e-5), 1.0, true};
 }
 }  // namespace
 
@@ -64,22 +64,7 @@ int fsmn_frames(const vadx_model* m, int64_t n_samples, int32_t* out) {
 int fsmn_finalize(vadx_model* m) {
   FsmnHP h;
   VADX_TRY(fsmn_hp(m, &h));
-  VADX_TRY(m->upload_raw("frontend.basis", (int64_t)h.n_taps() * h.ld_basis(), VADX_DT_F32));
-  if (vadx_stft_tc_supported(h.n_taps(), h.n_bins())) {
-    // tensor-core DFT image: pre-emphasis folded into the 2-term bf16 basis; the DC removal is applied in the
-    // frequency domain by the kernel's epilogue (tables built per chunk length at first use)
-    const double preemph = m->scalar("frontend.preemph", 0.97);
-    const float* hb = m->find("frontend.basis")->f32();
-    size_t bytes = 0;
-    VADX_TRY(vadx_pack_stft_basis_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, nullptr, 0, &bytes));
-    std::vector<uint8_t> img(bytes);
-    VADX_TRY(vadx_pack_stft_basis_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, img.data(), img.size(), &bytes));
-    VADX_TRY(m->upload("frontend.basis#TC", img.data(), img.size()));
-  }
-  VADX_TRY(m->upload_raw("frontend.mel_start", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_len", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_w", -1, VADX_DT_F32));
-  VADX_TRY(m->upload_mel_dense_tc(h.n_mels, h.n_bins(), (float)m->scalar("frontend.log_floor", 1e-5)));
+  VADX_TRY(fsmn_frontend(m, h).finalize(m));
   VADX_TRY(m->upload_raw("cmvn_means", h.input_dim, VADX_DT_F32));
   VADX_TRY(m->upload_raw("cmvn_vars", h.input_dim, VADX_DT_F32));
   VADX_TRY(m->upload_linear("in_linear1.linear.weight", h.affine, h.input_dim));
@@ -155,12 +140,8 @@ int fsmn_run(vadx_model* m, bool dry, const void* const* in, void* const* out, v
   float* noisy = static_cast<float*>(out[1]);
   float* p_sil = out[2] ? static_cast<float*>(out[2]) : p_sil_ws;
   float* power_db = out[3] ? static_cast<float*>(out[3]) : power_db_ws;
-  const float preemph = (float)m->scalar("frontend.preemph", 0.97);
-  const float floor_v = (float)m->scalar("frontend.log_floor", 1e-5);
   const float thr = (float)m->scalar("one_minus_speech_threshold", 1.0);
   const float ratio = (float)m->scalar("speech_2_noise_ratio", 1.0);
-  const bool use_tc = m->scalar("engine.use_tc", 1.0) != 0.0 && rows > kSkinnyMaxRows;
-  const int mel_max = (int)(m->find("frontend.mel_w")->numel() / h.n_mels);
 
   const int16_t* audio = static_cast<const int16_t*>(in[0]);
   if (W > 1) {
@@ -168,44 +149,7 @@ int fsmn_run(vadx_model* m, bool dry, const void* const* in, void* const* out, v
     VADX_TRY(vadx_gather_windows_i16(audio, sstride, S_streams, W, wstride, L, win16, st));
     audio = win16;
   }
-  VADX_TRY(vadx_prep_audio(audio, VADX_DT_I16, S, L, L, 1.0f, 1, preemph > 0.f ? VADX_PREEMPH_KEEP_FIRST : 0, preemph,
-                           h.pad_left(), sig, Lp, st));
-  const uint8_t* stft_img = use_tc ? m->d<uint8_t>("frontend.basis#TC") : nullptr;
-  if (stft_img && (L % 8) == 0 && (h.hop % 8) == 0 && (h.pad_left() % 8) == 0 && aligned16(audio)) {
-    // framed DFT on the tensor cores straight from the int16 samples; the mean is removed in the epilogue
-    const std::string key = "frontend.dc#" + std::to_string((long long)L);
-    const std::string k_lo = key + ".lo", k_hi = key + ".hi";
-    if (!m->d<float>(key)) {
-      size_t n = 0;
-      int lo = 0, hi = 0;
-      const float* hb = m->find("frontend.basis")->f32();
-      VADX_TRY(vadx_pack_stft_dc_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, L, h.hop, h.pad_left(), T, nullptr,
-                                    0, &n, &lo, &hi));
-      std::vector<float> tab(n);
-      VADX_TRY(vadx_pack_stft_dc_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, L, h.hop, h.pad_left(), T,
-                                    tab.data(), tab.size(), &n, &lo, &hi));
-      VADX_TRY(m->upload(key, tab.data(), tab.size() * sizeof(float)));
-      m->scalars[k_lo] = lo;
-      m->scalars[k_hi] = hi;
-    }
-    VADX_TRY(vadx_stream_mean_i16(audio, L, L, S, mean_ws, mean_int_ws, st));
-    VADX_TRY(vadx_stft_power_tc_i16_ex(audio, L, L, S, T, h.hop, h.n_taps(), stft_img, h.n_bins(),
-                                       power, h.ld_power(), h.pad_left(), mean_ws, mean_int_ws, m->d<float>(key),
-                                       (int)m->scalar(k_lo.c_str(), 0.0), (int)m->scalar(k_hi.c_str(), (double)T), 1.0f,
-                                       VADX_TC_FMT_BF16, st));
-  } else {
-    VADX_TRY(vadx_stft_power_f32(sig, Lp, S, T, h.hop, h.n_taps(), m->d<float>("frontend.basis"), h.ld_basis(),
-                                 h.n_bins(), power, h.ld_power(), st));
-  }
-  if (use_tc && m->d<uint8_t>("frontend.mel#TC")) {
-    // log-mel as a dense tensor-core layer, log(max(., floor)) in the epilogue
-    VADX_TRY(vadx_linear_tc_f32(power, h.ld_power(), m->d<uint8_t>("frontend.mel#TC"), m->d<float>("frontend.mel_floor"),
-                                nullptr, 0, mel, h.n_mels, rows, h.n_bins(), h.n_mels, VADX_ACT_LOG_CLAMP, st));
-  } else {
-    VADX_TRY(vadx_mel_log_f32(power, h.ld_power(), rows, h.n_bins(), h.n_mels, m->d<int32_t>("frontend.mel_start"),
-                              m->d<int32_t>("frontend.mel_len"), m->d<float>("frontend.mel_w"), mel_max, VADX_FLOOR_CLAMP,
-                              floor_v, mel, h.n_mels, st));
-  }
+  VADX_TRY(fsmn_frontend(m, h).run(m, audio, S, L, T, FrontendBufs{sig, nullptr, Lp, power, mean_ws, mean_int_ws, mel}, st));
   VADX_TRY(vadx_lfr_cmvn_f32(mel, h.n_mels, m->d<float>("cmvn_means"), m->d<float>("cmvn_vars"), feat, h.input_dim, S,
                              T, h.n_mels, h.lfr_m, h.lfr_n, st));
   const bool tc_rows = m->scalar("engine.use_tc", 1.0) != 0.0;

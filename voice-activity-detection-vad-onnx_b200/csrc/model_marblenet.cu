@@ -13,16 +13,10 @@ namespace {
 struct Block {
   int filters, repeat, kernel, stride, dilation, residual;
 };
-struct MarbleHP {
+struct MarbleHP : FrontendGeom {
   int feat_in;
   std::vector<Block> blocks;
-  int n_classes, n_fft, win, hop, n_mels;
-  int n_taps() const { return win < n_fft ? win : n_fft; }
-  int first_tap() const { return win < n_fft ? (n_fft - win) / 2 : 0; }
-  int n_bins() const { return n_fft / 2 + 1; }
-  int ld_basis() const { return (int)round_up(2 * n_bins(), 4); }
-  int ld_power() const { return (int)round_up(n_bins(), 4); }
-  int pad_left() const { return n_fft / 2 - first_tap(); }
+  int n_classes;
   int stft_frames(int64_t L) const { return (int)(L / hop + 1); }
   static int conv_len(int t, int k, int stride, int dil) {
     int pad = (dil * (k - 1)) / 2;
@@ -58,22 +52,22 @@ int marble_hp(const vadx_model* m, MarbleHP* h) {
   VADX_REQUIRE(h->n_classes >= 2 && h->n_classes <= 8 && h->feat_in == h->n_mels, "marblenet: head/frontend mismatch");
   return VADX_OK;
 }
+
+// samples scaled by 1/32768, log(mel + eps); the resampler zeroes the centre pad before writing the upsampled signal
+Frontend marble_frontend(const vadx_model* m, const MarbleHP& h) {
+  return Frontend{h, h.n_bins(), h.pad_left(), 1.0f / 32768.0f, false, VADX_PREEMPH_ZERO_HISTORY, VADX_TC_FMT_F16,
+                  VADX_FLOOR_ADD, (float)m->scalar("frontend.log_eps", 1e-7), frontend_rate_scale(m), false};
+}
 }  // namespace
 
 int marblenet_check(const vadx_model* m) {
   MarbleHP h;
   return marble_hp(m, &h);
 }
-// IN_SAMPLE_RATE != 16000 (Export_NVIDIA_MarbleNet_VAD.py:180-183): scale = 1 / (in_rate / 16000), the in-graph
-// linear resampler leaves floor(L * scale) samples at the model's 16 kHz
-static double marble_rate_scale(const vadx_model* m) {
-  const double in_rate = m->scalar("frontend.in_sample_rate", 16000.0);
-  return in_rate == 16000.0 ? 1.0 : 1.0 / (in_rate / 16000.0);
-}
 int marblenet_frames(const vadx_model* m, int64_t n_samples, int32_t* out) {
   MarbleHP h;
   VADX_TRY(marble_hp(m, &h));
-  const double sc = marble_rate_scale(m);
+  const double sc = frontend_rate_scale(m);
   *out = h.out_frames(sc == 1.0 ? n_samples : vadx_resample_out_len(n_samples, sc));
   return VADX_OK;
 }
@@ -81,24 +75,7 @@ int marblenet_frames(const vadx_model* m, int64_t n_samples, int32_t* out) {
 int marblenet_finalize(vadx_model* m) {
   MarbleHP h;
   VADX_TRY(marble_hp(m, &h));
-  VADX_TRY(m->upload_raw("frontend.basis", (int64_t)h.n_taps() * h.ld_basis(), VADX_DT_F32));
-  if (vadx_stft_tc_supported(h.n_taps(), h.n_bins())) {
-    // tensor-core DFT image: the pre-emphasis folded into the 2-term basis
-    const double preemph = m->scalar("frontend.preemph", 0.97);
-    const float* hb = m->find("frontend.basis")->f32();
-    size_t bytes = 0;
-    // fp16 operands; the 1/32768 stays out of the basis (fp16 range) and multiplies the power instead
-    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, VADX_TC_FMT_F16, nullptr, 0,
-                                         &bytes));
-    std::vector<uint8_t> img(bytes);
-    VADX_TRY(vadx_pack_stft_basis_tc_fmt(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, VADX_TC_FMT_F16, img.data(),
-                                         img.size(), &bytes));
-    VADX_TRY(m->upload("frontend.basis#TC", img.data(), img.size()));
-  }
-  VADX_TRY(m->upload_raw("frontend.mel_start", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_len", h.n_mels, VADX_DT_I32));
-  VADX_TRY(m->upload_raw("frontend.mel_w", -1, VADX_DT_F32));
-  VADX_TRY(m->upload_mel_dense_tc(h.n_mels, h.n_bins(), (float)m->scalar("frontend.log_eps", 1e-7)));
+  VADX_TRY(marble_frontend(m, h).finalize(m));
   int c_in = h.feat_in;
   for (size_t b = 0; b < h.blocks.size(); ++b) {
     const Block& k = h.blocks[b];
@@ -156,7 +133,8 @@ int marblenet_run(vadx_model* m, bool dry, const void* const* in, void* const* o
   (void)state;
   MarbleHP h;
   VADX_TRY(marble_hp(m, &h));
-  const double rate_scale = marble_rate_scale(m);
+  const Frontend fe = marble_frontend(m, h);
+  const double rate_scale = fe.rate_scale;
   const int64_t L_in = L;
   if (rate_scale != 1.0) L = vadx_resample_out_len(L_in, rate_scale);   // from here on L counts 16 kHz samples
   const int T0 = h.stft_frames(L);
@@ -179,63 +157,9 @@ int marblenet_run(vadx_model* m, bool dry, const void* const* in, void* const* o
   VADX_REQUIRE(out[1], "marblenet: outputs are {score_silence, score_active}");
   VADX_REQUIRE((char*)out[1] == (char*)out[0] + (size_t)S * Tout * sizeof(float),
                "marblenet: score_active must directly follow score_silence ([2][S][T'] planes)");
-  const float preemph = (float)m->scalar("frontend.preemph", 0.97);
-  const float eps = (float)m->scalar("frontend.log_eps", 1e-7);
   const bool use_tc = m->scalar("engine.use_tc", 1.0) != 0.0;
-  const int mel_max = (int)(m->find("frontend.mel_w")->numel() / h.n_mels);
-
-  const uint8_t* stft_img = use_tc && rows0 > kSkinnyMaxRows ? m->d<uint8_t>("frontend.basis#TC") : nullptr;
-  if (rate_scale != 1.0) {
-    // in-graph resampler (Export_NVIDIA_MarbleNet_VAD.py:236-254): down before the scale + pre-emphasis conv, up after it
-    const int pre = preemph > 0.f ? VADX_PREEMPH_ZERO_HISTORY : 0;
-    if (rate_scale < 1.0) {
-      VADX_TRY(vadx_prep_audio(in[0], VADX_DT_I16, S, L_in, L_in, 1.0f, 0, 0, 0.f, 0, sig2, Lp, st));
-      VADX_TRY(vadx_resample_linear_f32(sig2, Lp, L_in, S, rate_scale, sig, Lp, 0, st));
-      VADX_TRY(vadx_prep_audio(sig, VADX_DT_F32, S, L, Lp, 1.0f / 32768.0f, 0, pre, preemph, h.pad_left(), sig2, Lp, st));
-    } else {
-      VADX_TRY(vadx_prep_audio(in[0], VADX_DT_I16, S, L_in, L_in, 1.0f / 32768.0f, 0, pre, preemph, 0, sig, Lp, st));
-      cudaError_t e = cudaMemsetAsync(sig2, 0, (size_t)S * Lp * sizeof(float), st);   // centre pad around the resampled signal
-      if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(marblenet centre pad)");
-      VADX_TRY(vadx_resample_linear_f32(sig, Lp, L_in, S, rate_scale, sig2, Lp, h.pad_left(), st));
-    }
-    VADX_TRY(vadx_stft_power_f32(sig2, Lp, S, T0, h.hop, h.n_taps(), m->d<float>("frontend.basis"), h.ld_basis(),
-                                 h.n_bins(), power, h.ld_power(), st));
-  } else if (stft_img && (L % 8) == 0 && (h.hop % 8) == 0 && (h.pad_left() % 8) == 0 && aligned16(in[0])) {
-    // centre-padded framed DFT on the tensor cores straight from the int16 samples (zeros outside the clip)
-    const std::string key = "frontend.dc#" + std::to_string((long long)L);
-    const std::string k_lo = key + ".lo", k_hi = key + ".hi";
-    if (!m->d<float>(key)) {
-      size_t n = 0;
-      int lo = 0, hi = 0;
-      const float* hb = m->find("frontend.basis")->f32();
-      VADX_TRY(vadx_pack_stft_dc_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, L, h.hop, h.pad_left(), T0,
-                                    nullptr, 0, &n, &lo, &hi));
-      std::vector<float> tab(n);
-      VADX_TRY(vadx_pack_stft_dc_tc(hb, h.ld_basis(), h.n_taps(), h.n_bins(), preemph, 1.0, L, h.hop, h.pad_left(), T0,
-                                    tab.data(), tab.size(), &n, &lo, &hi));
-      VADX_TRY(m->upload(key, tab.data(), tab.size() * sizeof(float)));
-      m->scalars[k_lo] = lo;
-      m->scalars[k_hi] = hi;
-    }
-    VADX_TRY(vadx_stft_power_tc_i16_ex(static_cast<const int16_t*>(in[0]), L, L, S, T0, h.hop, h.n_taps(), stft_img, h.n_bins(),
-                                       power, h.ld_power(), h.pad_left(), nullptr, nullptr, m->d<float>(key),
-                                       (int)m->scalar(k_lo.c_str(), 0.0), (int)m->scalar(k_hi.c_str(), (double)T0),
-                                       (float)(1.0 / (32768.0 * 32768.0)), VADX_TC_FMT_F16, st));
-  } else {
-    VADX_TRY(vadx_prep_audio(in[0], VADX_DT_I16, S, L, L, 1.0f / 32768.0f, 0,
-                             preemph > 0.f ? VADX_PREEMPH_ZERO_HISTORY : 0, preemph, h.pad_left(), sig, Lp, st));
-    VADX_TRY(vadx_stft_power_f32(sig, Lp, S, T0, h.hop, h.n_taps(), m->d<float>("frontend.basis"), h.ld_basis(),
-                                 h.n_bins(), power, h.ld_power(), st));
-  }
-  if (use_tc && rows0 > kSkinnyMaxRows && m->d<uint8_t>("frontend.mel#TC")) {
-    // log-mel as a dense tensor-core layer, log(. + eps) in the epilogue (the bias slot carries eps)
-    VADX_TRY(vadx_linear_tc_f32(power, h.ld_power(), m->d<uint8_t>("frontend.mel#TC"), m->d<float>("frontend.mel_floor"),
-                                nullptr, 0, B[0], h.n_mels, rows0, h.n_bins(), h.n_mels, VADX_ACT_LOG, st));
-  } else {
-    VADX_TRY(vadx_mel_log_f32(power, h.ld_power(), rows0, h.n_bins(), h.n_mels, m->d<int32_t>("frontend.mel_start"),
-                              m->d<int32_t>("frontend.mel_len"), m->d<float>("frontend.mel_w"), mel_max, VADX_FLOOR_ADD, eps,
-                              B[0], h.n_mels, st));
-  }
+  VADX_TRY(fe.run(m, static_cast<const int16_t*>(in[0]), S, L_in, T0, FrontendBufs{sig, sig2, Lp, power, nullptr, nullptr, B[0]},
+                  st));
   auto lin = [&](const float* a, int n_in, const std::string& w, const std::string& b, const float* res, float* y,
                  int n_out, int64_t rows, int act) -> int {
     const uint8_t* img = use_tc && rows > kSkinnyMaxRows ? m->d<uint8_t>(w + "#TC") : nullptr;

@@ -58,6 +58,14 @@ class _Engine:
     def set_scalar(self, name: str, v: float):
         lib.check(self._lib.vadx_set_scalar(self._h, name.encode(), float(v)))
 
+    def set_frontend(self, basis: np.ndarray, bank: np.ndarray):
+        """The log-mel frontend's tensors: the interleaved DFT basis and the mel bank [n_bins, n_mels] in sparse form."""
+        st, ln, w = tables.sparse_bank(bank)
+        self.set_tensor("frontend.basis", basis)
+        self.set_tensor("frontend.mel_start", st)
+        self.set_tensor("frontend.mel_len", ln)
+        self.set_tensor("frontend.mel_w", w)
+
     def output_frames(self, n_samples: int) -> int:
         out = C.c_int32()
         lib.check(self._lib.vadx_output_frames(self._h, n_samples, C.byref(out)))
@@ -119,11 +127,7 @@ class FireRedSession:
         basis, first, _ = tables.interleaved_basis(cfg.n_fft, cfg.win_length, cfg.window, "v2")
         assert first == 0
         bank = constants.kaldi_like_mel_bank(cfg.n_fft, cfg.n_mels, 16000).numpy()
-        st, ln, w = tables.sparse_bank(bank)
-        self._e.set_tensor("frontend.basis", basis)
-        self._e.set_tensor("frontend.mel_start", st)
-        self._e.set_tensor("frontend.mel_len", ln)
-        self._e.set_tensor("frontend.mel_w", w)
+        self._e.set_frontend(basis, bank)
         self._e.set_scalar("frontend.preemph", cfg.pre_emphasis)
         self._e.set_scalar("frontend.log_floor", cfg.log_floor)
         self._e.set_scalar("engine.use_tc", 1.0 if tensor_cores else 0.0)
@@ -244,42 +248,6 @@ class FireRedStreamSession(FireRedSession):
         self._e.forward([audio], [out], [caches_in, caches_out], S, L, stream)
         return out, caches_out
 
-    def run_windows(self, aligned, stride: int, caches, stream=None):
-        """Whole-file mode: aligned cuda int16 [S, n] (chunk-aligned recordings, audio_io.align_overlapping), windows of
-        chunk_len samples `stride` apart.  ONE forward covers all W = (n - chunk_len) // stride + 1 windows of every stream
-        (the caches across windows are a causal FIR over the concatenated frames, see csrc/model_fsmn.cu).
-        -> (p_silence [S, W, T], power_dB [S, W, T], new_caches); the gate and the look-ahead machine, which depend on the
-        running background level, follow in postprocess.fsmn_gate_hysteresis_windows."""
-        import torch
-        if not (torch.is_tensor(aligned) and aligned.is_cuda and aligned.dtype == torch.int16 and aligned.dim() == 2
-                and aligned.is_contiguous()):
-            raise ValueError("run_windows: aligned must be a contiguous CUDA int16 tensor [S, n]")
-        S, n = aligned.shape
-        L = self.chunk_len
-        if n < L or stride < 1:
-            raise ValueError(f"run_windows: recordings of {n} samples are shorter than one {L}-sample window")
-        Wn = (n - L) // stride + 1
-        key = (Wn, int(stride), int(n))
-        if getattr(self, "_win_key", None) != key:
-            self._e.set_scalar("input.n_windows", float(Wn))
-            self._e.set_scalar("input.window_stride", float(stride))
-            self._e.set_scalar("input.stream_stride", float(n))
-            self._win_key = key
-        dev = aligned.device
-        p_sil = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
-        power = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
-        new = [torch.empty_like(c) for c in caches]
-        try:
-            self._e.forward([aligned, None], [p_sil, None, p_sil, power], list(caches) + new, S, L, stream)
-        finally:
-            pass
-        return p_sil, power, new
-
-    def _leave_window_mode(self):
-        if getattr(self, "_win_key", None) is not None:
-            self._e.set_scalar("input.n_windows", 1.0)
-            self._win_key = None
-
     def run(self, output_names, input_feed: dict):
         import torch
         names = [o.name for o in self._outputs_meta]
@@ -335,11 +303,7 @@ class FsmnSession:
         self._e = _Engine("fsmn", hp)
         basis, _first, _ = tables.interleaved_basis(cfg.n_fft, cfg.win_length, cfg.window, "v1")
         bank = constants.torchaudio_mel_bank(cfg.n_fft // 2 + 1, 20.0, 8000.0, cfg.n_mels, 16000, None, "htk").numpy()
-        st, ln, w = tables.sparse_bank(bank)
-        self._e.set_tensor("frontend.basis", basis)
-        self._e.set_tensor("frontend.mel_start", st)
-        self._e.set_tensor("frontend.mel_len", ln)
-        self._e.set_tensor("frontend.mel_w", w)
+        self._e.set_frontend(basis, bank)
         self._e.set_scalar("frontend.preemph", cfg.pre_emphasis)
         self._e.set_scalar("frontend.log_floor", cfg.log_floor)
         self._e.set_scalar("speech_2_noise_ratio", cfg.speech_2_noise_ratio)
@@ -434,10 +398,7 @@ class FsmnSession:
         p_sil = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
         power = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
         new = [torch.empty_like(c) for c in caches]
-        try:
-            self._e.forward([aligned, None], [p_sil, None, p_sil, power], list(caches) + new, S, L, stream)
-        finally:
-            pass
+        self._e.forward([aligned, None], [p_sil, None, p_sil, power], list(caches) + new, S, L, stream)
         return p_sil, power, new
 
     def _leave_window_mode(self):
@@ -499,11 +460,7 @@ class MarbleNetSession:
         self._e = _Engine("marblenet", hp)
         basis, _first, _ = tables.interleaved_basis(cfg.n_fft, cfg.win_length, cfg.window, "v2")
         bank = constants.torchaudio_mel_bank(cfg.n_fft // 2 + 1, 0.0, 8000.0, cfg.n_mels, 16000, "slaney", "slaney").numpy()
-        st, ln, w = tables.sparse_bank(bank)
-        self._e.set_tensor("frontend.basis", basis)
-        self._e.set_tensor("frontend.mel_start", st)
-        self._e.set_tensor("frontend.mel_len", ln)
-        self._e.set_tensor("frontend.mel_w", w)
+        self._e.set_frontend(basis, bank)
         self._e.set_scalar("frontend.preemph", cfg.pre_emphasis)
         self._e.set_scalar("frontend.log_eps", cfg.log_eps)
         self._e.set_scalar("engine.use_tc", 1.0 if tensor_cores else 0.0)
@@ -557,42 +514,6 @@ class MarbleNetSession:
             self._e.forward([audio[s0:s1]], [part[0], part[1]], [], s1 - s0, L, stream)
             out[:, s0:s1] = part
         return out
-
-    def run_windows(self, aligned, stride: int, caches, stream=None):
-        """Whole-file mode: aligned cuda int16 [S, n] (chunk-aligned recordings, audio_io.align_overlapping), windows of
-        chunk_len samples `stride` apart.  ONE forward covers all W = (n - chunk_len) // stride + 1 windows of every stream
-        (the caches across windows are a causal FIR over the concatenated frames, see csrc/model_fsmn.cu).
-        -> (p_silence [S, W, T], power_dB [S, W, T], new_caches); the gate and the look-ahead machine, which depend on the
-        running background level, follow in postprocess.fsmn_gate_hysteresis_windows."""
-        import torch
-        if not (torch.is_tensor(aligned) and aligned.is_cuda and aligned.dtype == torch.int16 and aligned.dim() == 2
-                and aligned.is_contiguous()):
-            raise ValueError("run_windows: aligned must be a contiguous CUDA int16 tensor [S, n]")
-        S, n = aligned.shape
-        L = self.chunk_len
-        if n < L or stride < 1:
-            raise ValueError(f"run_windows: recordings of {n} samples are shorter than one {L}-sample window")
-        Wn = (n - L) // stride + 1
-        key = (Wn, int(stride), int(n))
-        if getattr(self, "_win_key", None) != key:
-            self._e.set_scalar("input.n_windows", float(Wn))
-            self._e.set_scalar("input.window_stride", float(stride))
-            self._e.set_scalar("input.stream_stride", float(n))
-            self._win_key = key
-        dev = aligned.device
-        p_sil = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
-        power = torch.empty((S, Wn, self.T), dtype=torch.float32, device=dev)
-        new = [torch.empty_like(c) for c in caches]
-        try:
-            self._e.forward([aligned, None], [p_sil, None, p_sil, power], list(caches) + new, S, L, stream)
-        finally:
-            pass
-        return p_sil, power, new
-
-    def _leave_window_mode(self):
-        if getattr(self, "_win_key", None) is not None:
-            self._e.set_scalar("input.n_windows", 1.0)
-            self._win_key = None
 
     def run(self, output_names, input_feed: dict):
         import torch
