@@ -271,7 +271,8 @@ struct FrontendBufs {  // the caller's workspace
 };
 
 // What differs between the models' frontends.  The tensor-core paths run when engine.use_tc is set and S*T exceeds
-// kSkinnyMaxRows; the int16 tensor-core STFT also needs L, hop and pad_left to be multiples of 8 and 16-byte aligned audio.
+// kSkinnyMaxRows; the int16 tensor-core STFT also needs L and pad_left to be multiples of 8, hop a multiple of 16 and
+// 16-byte aligned audio.
 struct Frontend {
   FrontendGeom g;
   int n_bins;          // DFT bins computed (<= g.n_bins())
@@ -345,7 +346,7 @@ inline int Frontend::run(vadx_model* m, const int16_t* audio, int64_t S, int64_t
     VADX_TRY(vadx_stft_power_f32(b.sig2, Lp, S, T, g.hop, g.n_taps(), m->d<float>("frontend.basis"), g.ld_basis(), n_bins,
                                  b.power, g.ld_power(), st));
   } else {
-    const bool tc = stft_img && (L % 8) == 0 && (g.hop % 8) == 0 && (pad_left % 8) == 0 && aligned16(audio);
+    const bool tc = stft_img && (L % 8) == 0 && (g.hop % 16) == 0 && (pad_left % 8) == 0 && aligned16(audio);
     if (keep_signal || !tc)
       VADX_TRY(vadx_prep_audio(audio, VADX_DT_I16, S, L, L, in_scale, remove_dc, pre, preemph, pad_left, b.sig, Lp, st));
     if (tc) {

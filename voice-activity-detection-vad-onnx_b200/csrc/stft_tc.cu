@@ -1,45 +1,61 @@
 // stft_tc.cu -- framed real DFT + power (a1 + a2) on the tensor cores, straight from int16 audio.
 //
-//   power[(s*T + t)][f] = | sum_n y[s][t*hop + n] * w[n] e^{-i 2 pi f n / n_fft} |^2 ,
+//   power[(s*T + t)][f] = | sum_n y[s][t*hop - pad_left + n] * w[n] e^{-i 2 pi f n / n_fft} |^2 ,
 //   y[i] = scale * (x[i] - c * x[i-1])            (x int16, x[-1] = 0: the reference's pad(1,0)+conv)
 //
-// as ONE bf16 tensor-core GEMM with fp32-grade accuracy and no prepared-signal round trip:
-//   * an int16 sample splits EXACTLY into two bf16 terms, x = 256*(x >> 8) + (x & 255);
+// as ONE tensor-core GEMM with fp32-grade accuracy and no prepared-signal round trip:
+//   * an int16 sample splits EXACTLY into two bf16 / fp16 terms, x = 256*(x >> 8) + (x & 255);
 //   * pre-emphasis and the int16 scale are folded into the basis on the host, in double:
 //       B'[k][col] = scale * (b[k-8][col] - c * b[k-7][col])      (k-8 = tap index; 8 leading zero
 //     rows keep every 8-sample group of a frame 16-byte aligned and make room for the x[i-1] tap);
-//   * B' is split into THREE bf16 terms (24 bits), and x_hi*b0 + x_lo*b0 + x_hi*b1 + x_lo*b1 + x_hi*b2
-//     is accumulated in fp32 TMEM -- the dropped x_lo*b2 is < 2^-23 of full scale.
-// Valid when every frame lies inside [0, L) and no DC removal is requested (FireRedVAD); the
-// centre-padded / DC-removed frontends keep the fp32 kernel.
+//   * B' is split into TWO terms b0 + b1, stacked as one N = 160 operand, so x_hi * [b0|b1] and x_lo * [b0|b1] are the two
+//     MMAs of a K = 16 step; the epilogue adds the two column blocks of the fp32 TMEM accumulator.
+// Centre-padded frontends (frames reaching outside [0, L): zero samples) and DC removal (integer part of the mean taken
+// off the samples by the loaders, the fractional part and the pre-emphasised pad's tail put back from per-frame tables in
+// the epilogue) are the EX variant.
 //
-// Work decomposition: the (re, im)-interleaved output columns are cut into N-tiles of 48; a CTA keeps
-// the 3-term basis image of ITS N-tile resident in shared memory (129 KB, fetched once with
-// cp.async.bulk) and streams 128-frame row tiles through a 2-deep mbarrier ring.  Same warp roles
-// as gemm_tc.cu: 8 loader warps (int16 -> (hi, lo) bf16, swizzled; three register buffers, i.e. the
-// loads of two stages in flight), 4 epilogue warps (TMEM -> re^2+im^2 -> global), 1 MMA issuer, two
-// TMEM accumulators in ping-pong.
+// Hop rows instead of frames.  With hop % 16 == 0, K16 step k = (hop/16)*q + j of frame t reads samples
+// [origin(t) + 16k, +16), origin(t) = t*hop - pad_left - 8: slice j of HOP ROW t + q, where hop row h holds the hop samples
+// from h*hop - pad_left - 8.  The A operand is stored without swizzle, K-major, one 8-sample slice of all rows at a time
+// with the rows 16 B apart, so "hop row t + q" for the 128 frames of a tile is the same slice 16*q bytes further on.  A
+// tile of 128 M rows therefore needs its 128 + Q - 1 hop rows (Q = hop rows a frame spans) converted once, instead of
+// 128 frames that overlap Q-fold.  M rows are SLOTS: T + Q - 1 per stream, so a frame's hop rows never cross into the
+// next stream; the Q - 1 extra slots compute rows that are never stored.
+//
+// Work decomposition: the (re, im)-interleaved output columns are cut into N-tiles of 80; a CTA keeps the 2-term basis
+// image of ITS N-tile resident in shared memory (143 KB for 400 taps, fetched once with cp.async.bulk) and streams
+// 128-slot tiles through a 3-deep ring of stages, each holding kStJ K16 columns of all the tile's hop rows as (hi, lo).
+// Warp roles: 16 loader warps (int16 -> (hi, lo), register buffers keep the loads of several stages in flight), 4
+// epilogue warps (TMEM -> re^2+im^2 -> global), 1 MMA issuer, two TMEM accumulators in ping-pong.
 #include "tc_ptx.cuh"
 
 namespace vadx {
 
 constexpr int kStNPad = 80;                          // columns per N-tile (40 bins)
-constexpr int kStTerms = 2;                          // bf16 terms of the folded basis
+constexpr int kStTerms = 2;                          // terms of the folded basis
 constexpr int kStLead = 8;                           // leading zero rows of the folded basis
-constexpr int kStStageBytes = 2 * kTcTileBytes;      // x_hi + x_lo
-constexpr int kStStages = 2;
+constexpr int kStJ = 2;                              // K16 columns of the hop rows per ring stage
+constexpr int kStSlices = 2 * kStJ;                  // 8-sample slices per stage
+constexpr int kStStages = 3;
+constexpr int kStLoaderWarps = 16;
 constexpr int kStOutLd = 44;                         // floats per staged output row (40 used; 44 keeps float4 stores conflict-free)
-// loader warps LW (8 or 16, a template parameter): epilogue warps LW..LW+3 ((warp & 3) = TMEM lane quarter), MMA warp LW+4
+// epilogue warps kStLoaderWarps..+3 ((warp & 3) = TMEM lane quarter), MMA warp kStLoaderWarps + 4
 
 struct StftTcArgs {
   const int16_t* X;
   int64_t in_stride;   // samples between streams
   int64_t L;           // valid samples per stream
+  int64_t S;           // streams
   int n_frames, hop;
-  const uint8_t* Wimg;  // [n_ntiles][kc][3][kStNPad*128]
+  int h16;             // hop / 16: K16 columns per hop row
+  int n_q;             // Q: hop rows one frame's n_k16 steps span
+  int tq;              // slots per stream (n_frames + Q - 1)
+  int rows;            // hop rows of one tile (kTcBM + Q - 1)
+  int slice_units;     // 16-byte units between two 8-sample slices of a stage (>= rows)
+  int n_st;            // ring stages per tile (ceil(h16 / kStJ))
+  const uint8_t* Wimg;  // [n_ntiles][kc][2][kStNPad*128]
   float* P;
   int64_t ldp;
-  int64_t M;           // S * n_frames
   int n_bins, kc, n_k16, n_tiles, vec_p;
   int pad_left;          // zero samples before sample 0 (centre pad minus the window's dead taps); multiple of 8
   const float* mean;     // [S] FRACTIONAL part of the per-stream mean (removed in the epilogue), or null
@@ -50,11 +66,9 @@ struct StftTcArgs {
                          // pad -- then one tail row per frame that runs past the end of the stream
   int n_edge_lo, t_edge_hi;   // frames t < n_edge_lo and t >= t_edge_hi are edge frames
   float power_scale;     // multiplies re^2 + im^2 (a scale kept out of an fp16 basis, e.g. (1/32768)^2)
-  int stack;       // 1: both basis terms as one N = 160 operand (two MMAs per K step, each sample term read once)
   int stage_out;   // 1: the epilogue transposes each warp's 32 x 40 powers through shared memory (coalesced stores)
   unsigned backoff_ld, backoff_epi;   // nanoseconds between mbarrier probes of the loader / epilogue warps
-  int k_live;      // columns < k_live are read by the MMA (n_k16 * 16)
-  int debug;  // VADX_TC_DEBUG perf experiments: 1 no stores, 2 no loads, 4 one product only
+  int debug;  // VADX_TC_DEBUG perf experiments: 1 no stores, 4 x_hi product only, 8 loaders write no shared memory
 };
 
 // Exact int -> bf16 without the (quarter-rate) conversion pipe: for 0 <= v < 2^23,
@@ -101,15 +115,19 @@ __device__ __forceinline__ void split17(int d, float& hi, float& lo) {
 
 // EX = false: every frame inside the stream, no DC removal (FireRed) -- the padded / mean-removing code is compiled out
 // F16 = true: fp16 operands (cheaper exact conversion; not with the 17-bit mean-removed samples)
-template <bool EX, bool F16, int LW>
-__global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const StftTcArgs g) {
-  constexpr int kStLoaderWarps = LW, kStEpiWarp0 = LW, kStMmaWarp = LW + 4;
+template <bool EX, bool F16>
+__global__ void __launch_bounds__((kStLoaderWarps + 5) * 32, 1) stft_power_tc_kernel(const StftTcArgs g) {
+  constexpr int kStEpiWarp0 = kStLoaderWarps, kStMmaWarp = kStLoaderWarps + 4;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* w_smem = smem_raw;
   const uint32_t img_bytes = kStNPad * 128u;
   const int w_bytes = g.kc * kStTerms * (int)img_bytes;
   uint8_t* a_smem = w_smem + w_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(a_smem + (size_t)kStStages * kStStageBytes);
+  // stage = [x_hi | x_lo], each [kStSlices][slice_units * 16 B]: slice i of a stage holds 8 samples of every hop row
+  const uint32_t slice_bytes = (uint32_t)g.slice_units * 16u;
+  const uint32_t term_bytes = kStSlices * slice_bytes;
+  const uint32_t stage_bytes = 2u * term_bytes;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(a_smem + (size_t)kStStages * stage_bytes);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 13);
   float* out_stage = reinterpret_cast<float*>(bars + 16);   // [4 warps][32 rows][kStOutLd], only when g.stage_out
 
@@ -120,10 +138,11 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
   auto tfull_bar = [&](int b) { return bar0 + 8u * (8 + b); };
   auto tempty_bar = [&](int b) { return bar0 + 8u * (10 + b); };
   const uint32_t wbar = bar0 + 8u * 12;
-  constexpr uint32_t kTmemCols = 512;  // 2 accumulators of 80 (or, stacked, 160) columns
+  constexpr int kAccN = 2 * kStNPad;   // x * b0 | x * b1
+  constexpr uint32_t kTmemCols = 512;  // 2 accumulators of 160 columns
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < 4; ++s) {
+    for (int s = 0; s < kStStages; ++s) {
       mbar_init(full_bar(s), kStLoaderWarps);     // one elected lane per loader warp
       mbar_init(empty_bar(s), 1);
     }
@@ -152,8 +171,21 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       const uint8_t* src = g.Wimg + (size_t)ntile * w_bytes;
       for (int t = 0; t < g.kc * kStTerms; ++t) bulk_g2s(smem_u32(w_smem) + t * img_bytes, src + (size_t)t * img_bytes, img_bytes, wbar);
       mbar_wait(wbar, 0);
-      const int acc_n = g.stack ? 2 * kStNPad : kStNPad;
-      const uint32_t idesc = F16 ? umma_idesc_f16(acc_n) : umma_idesc_bf16(acc_n);
+      const uint32_t idesc = F16 ? umma_idesc_f16(kAccN) : umma_idesc_bf16(kAccN);
+      // descriptors advance in their 16-byte address units: B by one 64-wide basis chunk (both terms) per 4 K16 steps and
+      // 32 B per step inside it (the SW128 image, as umma_k64 reads it); A by one row per q, two slices per K16 column
+      const uint64_t dw = umma_desc_sw128(smem_u32(w_smem));
+      const uint64_t da0 = umma_desc_noswz(smem_u32(a_smem), slice_bytes, 128u);
+      const uint32_t chunk_units = (kStTerms * img_bytes) >> 4, lo_units = term_bytes >> 4, stage_units = stage_bytes >> 4;
+      const uint32_t col_units = (2u * slice_bytes) >> 4;
+      const int h16 = g.h16, n_k16 = g.n_k16;
+      const uint32_t lo_on = (g.debug & 4) ? 0u : 1u;
+      // Issue pacing, measured on a B200 (bench.py, tools/stft_microbench.py): with fp16 operands and no padding or mean
+      // removal -- the cheapest loader -- the issuing thread bounds the kernel, and a column's up to three MMA pairs from
+      // one asm block take FireRed's STFT from 1.28 to 1.10 ms per 8192 chunks.  A build that issued every variant that
+      // way was 10-20 % slower in the bf16 and the padded / mean-removing variants, so those issue one pair at a time.
+      constexpr bool kBurst = F16 && !EX;
+      auto b_desc = [&](int k) { return dw + (uint64_t)((uint32_t)(k >> 2) * chunk_units + 2u * (uint32_t)(k & 3)); };
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -162,28 +194,31 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
         const uint32_t use = (uint32_t)(it >> 1);
         mbar_wait(tempty_bar(b), (use & 1u) ^ 1u);
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(b * acc_n);
-        for (int c = 0; c < g.kc; ++c) {
+        const uint32_t d_tmem = tmem_base + (uint32_t)(b * kAccN);
+        for (int st = 0; st < g.n_st; ++st) {
           mbar_wait(full_bar(stage), phase);
           tc_fence_after();
-          const uint32_t a_hi = smem_u32(a_smem) + (uint32_t)stage * kStStageBytes;
-          const uint32_t a_lo = a_hi + kTcTileBytes;
-          const uint32_t w0 = smem_u32(w_smem) + (uint32_t)(c * kStTerms) * img_bytes;
-          const uint32_t w1 = w0 + img_bytes;
-          const int nk = min(4, g.n_k16 - c * 4);
-          // smallest contributions first would be numerically nicer, but the first MMA of a tile must
-          // overwrite the accumulator; the order below keeps that one the dominant x_hi * b0 term
-          const uint64_t da_hi = umma_desc_sw128(a_hi), da_lo = umma_desc_sw128(a_lo);
-          const uint64_t dw0 = umma_desc_sw128(w0), dw1 = umma_desc_sw128(w1);
-          umma_k64(d_tmem, da_hi, dw0, idesc, c ? 1u : 0u, nk);
-          if (g.stack) {
-            // the two basis terms sit back to back in shared memory: as one 160-row operand they give x_hi*b0 | x_hi*b1
-            // in two column blocks of the accumulator (the epilogue adds them) and every sample term is read once
-            umma_k64(d_tmem, da_lo, dw0, idesc, 1u, nk);
-          } else if (!(g.debug & 4)) {
-            umma_k64(d_tmem, da_lo, dw0, idesc, 1u, nk);
-            umma_k64(d_tmem, da_hi, dw1, idesc, 1u, nk);
-            umma_k64(d_tmem, da_lo, dw1, idesc, 1u, nk);
+          const uint64_t da_st = da0 + (uint64_t)stage * stage_units;
+#pragma unroll
+          for (int jj = 0; jj < kStJ; ++jj) {
+            const int j = st * kStJ + jj;
+            if (j >= h16) break;
+            const uint64_t da_j = da_st + (uint64_t)jj * col_units;
+            // column j, K16 steps k = j + h16 * q: the frame's q-th hop row is 16 bytes (one row) further on.  The first
+            // MMA of a tile (k = 0, the dominant x_hi * b0 | x_hi * b1 term) overwrites the accumulator
+            if (kBurst) {
+              for (int q0 = 0, k = j; k < n_k16; q0 += 3, k += 3 * h16) {
+                const int n_pairs = 1 + (k + h16 < n_k16 ? 1 : 0) + (k + 2 * h16 < n_k16 ? 1 : 0);
+                umma_split_x3(d_tmem, da_j + (uint64_t)q0, 1u, lo_units, b_desc(k), b_desc(k + h16), b_desc(k + 2 * h16),
+                              idesc, k ? 1u : 0u, n_pairs, lo_on);
+              }
+            } else {
+              for (int q = 0, k = j; k < n_k16; ++q, k += h16) {
+                const uint64_t da = da_j + (uint64_t)q;
+                if (g.debug & 4) umma_bf16(d_tmem, da, b_desc(k), idesc, k ? 1u : 0u);
+                else umma_x2(d_tmem, da, da + lo_units, b_desc(k), idesc, k ? 1u : 0u);
+              }
+            }
           }
           umma_commit(empty_bar(stage));
           if (++stage == kStStages) { stage = 0; phase ^= 1u; }
@@ -192,50 +227,52 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       }
     }
   } else if (warp < kStLoaderWarps) {
-    // ===================== loaders: int16 frames -> exact (hi, lo) bf16 =====================
-    // 256 threads: thread = (group of 8 samples, row mod 32), 4 rows per stage.  Three register buffers
-    // rotate (issue for step i+2, convert step i): the loads of two stages are always in flight, so the
-    // L2/HBM latency is hidden instead of being paid once per stage.
-    constexpr int kPasses = kTcBM / (kStLoaderWarps * 4);   // 4
+    // ===================== loaders: int16 hop rows -> exact (hi, lo) =====================
+    // thread = (slice of the stage, row mod 128): the 4 lanes of a row read its 64 contiguous bytes of the stage, 8 rows
+    // per warp.  A quarter-warp's 16-byte stores land on 2 rows x 4 slices; slice_units = 2 (mod 4) spreads them over all
+    // 8 16-byte bank groups.  Rows 128.. (the Q - 1 halo rows) take a second pass on the first warp.
+    constexpr int kRowsPerPass = kStLoaderWarps * 32 / kStSlices;   // 128
+    constexpr int kPasses = 2;                                      // rows <= 256
     const int t = threadIdx.x;
-    const int kq = t & 7;      // group of 8 consecutive samples
-    const int r_in = t >> 3;   // 0..31
-    // frame origins of this thread's rows in the tile being PREFETCHED (recomputed once per tile:
-    // the 64-bit divisions must not sit on the per-stage path)
+    const int sl = t % kStSlices;
+    const int r_in = t / kStSlices;
+    // per row of the tile being PREFETCHED: stream base and first sample of the hop row (recomputed once per tile: the
+    // 64-bit divisions must not sit on the per-stage path)
     const int16_t* xs_n[kPasses];
-    int forig_n[kPasses];
+    int h0_n[kPasses];
+    uint32_t rok_n = 0u;
     int tile_cached = -1;
-    struct Seq { int tile, c; };
+    struct Seq { int tile, st; };
     auto valid = [&](const Seq& q) { return q.tile < g.n_tiles; };
-    auto advance = [&](Seq& q) { if (++q.c == g.kc) { q.c = 0; q.tile += gridDim.x; } };
-    // columns at and beyond the last K16 step the MMA issues are never read: neither load nor store them (the last
-    // 64-wide chunk of a 408-tap frame has 32 such columns, 7 % of the loader's traffic)
-    const int k_live = g.k_live;
+    auto advance = [&](Seq& q) { if (++q.st == g.n_st) { q.st = 0; q.tile += gridDim.x; } };
+    const int n_groups = 2 * g.h16;   // 8-sample groups of a hop row
     auto issue = [&](const Seq& q, uint4* raw, uint32_t& msk) {
       msk = 0u;
       if (q.tile != tile_cached) {
-        const int64_t row0 = (int64_t)q.tile * kTcBM;
+        rok_n = 0u;
 #pragma unroll
         for (int pass = 0; pass < kPasses; ++pass) {
-          const int64_t row = min_i64(row0 + pass * (kStLoaderWarps * 4) + r_in, g.M - 1);
-          const int64_t s = row / g.n_frames;
-          const int fr = (int)(row - s * g.n_frames);
-          xs_n[pass] = g.X + s * g.in_stride;
-          forig_n[pass] = fr * g.hop - (EX ? g.pad_left : 0) - kStLead;
+          const int r = pass * kRowsPerPass + r_in;
+          const int64_t slot = (int64_t)q.tile * kTcBM + r;
+          const int64_t s = slot / g.tq;
+          const int h = (int)(slot - s * g.tq);
+          const bool ok = r < g.rows && s < g.S;
+          xs_n[pass] = g.X + (ok ? s : 0) * g.in_stride;
+          h0_n[pass] = h * g.hop - (EX ? g.pad_left : 0) - kStLead;
+          if (ok) rok_n |= 1u << pass;
         }
         tile_cached = q.tile;
       }
-      const int k = q.c * kTcBK + kq * 8;
+      const int grp = q.st * kStSlices + sl;
 #pragma unroll
       for (int pass = 0; pass < kPasses; ++pass) {
-        const int16_t* xs = xs_n[pass];
-        const int i0 = forig_n[pass] + k;  // first of 8 consecutive samples (stream-relative)
+        const int i0 = h0_n[pass] + 8 * grp;  // first of 8 consecutive samples (stream-relative)
         // hop, pad_left, the lead (8) and the stream length are all multiples of 8 samples, so an 8-sample group lies
         // either entirely inside [0, L) or entirely outside it (zero pad): no element-wise edge path
         uint4 v = make_uint4(0u, 0u, 0u, 0u);
-        if (i0 >= 0 && i0 + 7 < g.L && k < k_live) {
-          v = __ldg(reinterpret_cast<const uint4*>(xs + i0));
-          if (EX) msk |= 0xffu << (8 * pass);
+        if (((rok_n >> pass) & 1u) && grp < n_groups && i0 >= 0 && i0 + 7 < g.L) {
+          v = __ldg(reinterpret_cast<const uint4*>(xs_n[pass] + i0));
+          msk |= 1u << pass;
         }
         raw[pass] = v;
       }
@@ -243,35 +280,36 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
     int stage = 0;
     uint32_t phase = 0;
     int mi_c[kPasses];        // integer mean of each row's stream, for the tile being CONSUMED
+#pragma unroll
+    for (int pass = 0; pass < kPasses; ++pass) mi_c[pass] = 0;
     int tile_cached_c = -1;
     auto consume = [&](const Seq& q, const uint4* raw, uint32_t msk) {
-      const int64_t row0 = (int64_t)q.tile * kTcBM;
       if (EX && g.mean_int && q.tile != tile_cached_c) {
 #pragma unroll
         for (int pass = 0; pass < kPasses; ++pass) {
-          const int64_t row = min_i64(row0 + pass * (kStLoaderWarps * 4) + r_in, g.M - 1);
-          mi_c[pass] = __ldg(g.mean_int + row / g.n_frames);
+          const int64_t s = ((int64_t)q.tile * kTcBM + pass * kRowsPerPass + r_in) / g.tq;
+          mi_c[pass] = s < g.S ? __ldg(g.mean_int + s) : 0;
         }
         tile_cached_c = q.tile;
       }
       mbar_wait(empty_bar(stage), phase ^ 1u, g.backoff_ld);
-      uint8_t* st_hi = a_smem + (size_t)stage * kStStageBytes;
-      uint8_t* st_lo = st_hi + kTcTileBytes;
-      if (!(g.debug & 8) && q.c * kTcBK + kq * 8 < k_live)
+      uint8_t* st_hi = a_smem + (size_t)stage * stage_bytes + sl * slice_bytes;
+      uint8_t* st_lo = st_hi + term_bytes;
+      if (!(g.debug & 8) && q.st * kStSlices + sl < n_groups)
 #pragma unroll
       for (int pass = 0; pass < kPasses; ++pass) {
-        const int r = pass * (kStLoaderWarps * 4) + r_in;
+        const int r = pass * kRowsPerPass + r_in;
+        if (r >= g.rows) break;
         const uint32_t wds[4] = {raw[pass].x, raw[pass].y, raw[pass].z, raw[pass].w};
         uint32_t hi[4], lo[4];
         if (EX && g.mean_int) {
           // integer part of the stream's mean removed from the real samples only (the zero pad stays zero)
-          const int mi = mi_c[pass];
-          const uint32_t vm = (msk >> (8 * pass)) & 0xffu;
+          const int mi = ((msk >> pass) & 1u) ? mi_c[pass] : 0;
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
-            const uint32_t w = wds[j];   // rows past M repeat row M-1 and are never stored
-            const int a = ((vm >> (2 * j)) & 1u) ? ((int)(w << 16) >> 16) - mi : 0;
-            const int b = ((vm >> (2 * j + 1)) & 1u) ? ((int)w >> 16) - mi : 0;
+            const uint32_t w = wds[j];
+            const int a = ((int)(w << 16) >> 16) - mi;
+            const int b = ((int)w >> 16) - mi;
             float ah, al, bh, bl;
             split17(a, ah, al);
             split17(b, bh, bl);
@@ -281,14 +319,13 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
         } else {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          const uint32_t w = wds[j];   // rows past M repeat row M-1 and are never stored
+          const uint32_t w = wds[j];
           hi[j] = F16 ? f16x2_hi(w) : bf16x2_hi(w);
           lo[j] = F16 ? f16x2_lo(w) : bf16x2_lo(w);
         }
         }
-        const int off = r * 128 + ((kq ^ (r & 7)) << 4);
-        *reinterpret_cast<uint4*>(st_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-        *reinterpret_cast<uint4*>(st_lo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        *reinterpret_cast<uint4*>(st_hi + r * 16) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+        *reinterpret_cast<uint4*>(st_lo + r * 16) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
       }
       if (!(g.debug & 16)) fence_proxy_async();
       __syncwarp();
@@ -296,8 +333,8 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       if (++stage == kStStages) { stage = 0; phase ^= 1u; }
     };
     // kStBufs register buffers rotate: the loads of kStBufs - 1 stages are in flight while one is converted
-    // (the padded / mean-removing variant carries more live state per thread and keeps one buffer fewer)
-    constexpr int kStBufs = EX ? 4 : (LW > 8 ? 6 : 5);
+    // (the padded / mean-removing variant carries more live state per thread and keeps fewer)
+    constexpr int kStBufs = EX ? 4 : 6;
     uint4 bufs[kStBufs][kPasses];
     uint32_t msks[kStBufs];
 #pragma unroll
@@ -325,9 +362,13 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       const uint32_t use = (uint32_t)(it >> 1);
       mbar_wait(tfull_bar(b), use & 1u, g.backoff_epi);   // a tile takes microseconds: poll rarely
       tc_fence_after();
-      const int64_t row = (int64_t)tile * kTcBM + q * 32 + lane;
-      const bool row_ok = row < g.M;
-      const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * (g.stack ? 2 * kStNPad : kStNPad));
+      // slot -> (stream, frame); the Q - 1 slots past a stream's last frame hold no frame
+      const int64_t slot = (int64_t)tile * kTcBM + q * 32 + lane;
+      const int64_t sidx = slot / g.tq;
+      const int t = (int)(slot - sidx * g.tq);
+      const bool row_ok = sidx < g.S && t < g.n_frames;
+      const int64_t row = row_ok ? sidx * g.n_frames + t : -1;
+      const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(b * kAccN);
       float* const my_out = out_stage + (size_t)q * 32 * kStOutLd;
       // DC removal in the frequency domain: X(x - m) = X(x) - m * (folded basis applied to the mean's
       // coefficient pattern), exact in fp32; only frames touching the zero pad need their own row of the table
@@ -337,8 +378,6 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       const float* dc_row = nullptr;
       const float* tail_row = nullptr;
       if (EX && g.dc && row_ok) {
-        const int64_t sidx = row / g.n_frames;
-        const int t = (int)(row - sidx * g.n_frames);
         const int n_edge = g.n_edge_lo + (g.n_frames - g.t_edge_hi);
         if (g.mean) {
           m_row = __ldg(g.mean + sidx);
@@ -352,14 +391,11 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       }
 #pragma unroll
       for (int c0 = 0; c0 < kStNPad; c0 += 16) {
-        float v[16];
+        float v[16], v2[16];
         tmem_ld16(taddr + (uint32_t)c0, v);
-        if (g.stack) {
-          float v2[16];
-          tmem_ld16(taddr + (uint32_t)(kStNPad + c0), v2);
+        tmem_ld16(taddr + (uint32_t)(kStNPad + c0), v2);
 #pragma unroll
-          for (int j = 0; j < 16; ++j) v[j] += v2[j];
-        }
+        for (int j = 0; j < 16; ++j) v[j] += v2[j];
         if (!row_ok || (g.debug & 1)) continue;
         if (EX && dc_row) {
 #pragma unroll
@@ -392,16 +428,16 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
       if (lane == 0) mbar_arrive(tempty_bar(b));   // the accumulator is free; the staged rows still have to go out
       if (g.stage_out && !(g.debug & 1)) {
         // 32 rows x 40 powers, written 16 bytes per lane with consecutive lanes on consecutive columns: a row's 160 bytes
-        // leave in one piece instead of as ten 16-byte stores scattered over ten instructions
-        const int64_t row0 = (int64_t)tile * kTcBM + q * 32;
+        // leave in one piece instead of as ten 16-byte stores scattered over ten instructions.  The warp's 32 slots are
+        // not 32 consecutive output rows (a stream's halo slots sit between streams): each staged row asks its own lane
         constexpr int kC4 = kStNPad / 8;   // 10 float4 per row
 #pragma unroll
         for (int itr = 0; itr < kC4; ++itr) {
           const int idx = itr * 32 + lane;
           const int r = idx / kC4, c4 = idx - r * kC4;
-          const int64_t grow = row0 + r;
+          const long long grow = __shfl_sync(0xffffffffu, (long long)row, r);
           const int fbin = f0 + c4 * 4;
-          if (grow < g.M && fbin < g.n_bins) {
+          if (grow >= 0 && fbin < g.n_bins) {
             const float4 val = *reinterpret_cast<const float4*>(my_out + r * kStOutLd + c4 * 4);
             float* out = g.P + grow * g.ldp + fbin;
             if (fbin + 3 < g.n_bins) {
@@ -425,12 +461,28 @@ __global__ void __launch_bounds__((LW + 5) * 32, 1) stft_power_tc_kernel(const S
   }
 }
 
+// hop rows of a tile and the 16-byte units between two slices of a stage: >= rows and = 2 (mod 4), so that the 8 lanes of
+// a quarter-warp (2 rows x 4 slices) store to 8 different 16-byte bank groups
+struct StftTcRing {
+  int n_q, rows, slice_units;
+  size_t bytes;
+};
+static StftTcRing stft_tc_ring(int n_k16, int h16) {
+  StftTcRing r{};
+  r.n_q = (n_k16 - 1) / h16 + 1;
+  r.rows = kTcBM + r.n_q - 1;
+  r.slice_units = r.rows + ((2 - r.rows % 4) + 4) % 4;
+  r.bytes = (size_t)kStStages * 2 * kStSlices * r.slice_units * 16;
+  return r;
+}
+
 struct StftTcShape {
   int kc, n_k16, n_ntiles;
   size_t tile_bytes, img_bytes, smem_bytes, stage_bytes;   // stage_bytes: optional output staging on top of smem_bytes
   bool ok;
 };
-StftTcShape stft_tc_shape(int n_taps, int n_bins) {
+// hop = 16 sizes the ring for the most hop rows a frame can span: a shape that is supported runs at every hop % 16 == 0
+StftTcShape stft_tc_shape(int n_taps, int n_bins, int hop = 16) {
   StftTcShape s{};
   const int k_used = n_taps + kStLead;
   s.kc = (int)ceil_div(k_used, kTcBK);
@@ -438,7 +490,7 @@ StftTcShape stft_tc_shape(int n_taps, int n_bins) {
   s.n_ntiles = (int)ceil_div(2 * n_bins, kStNPad);
   s.tile_bytes = (size_t)s.kc * kStTerms * kStNPad * 128;
   s.img_bytes = s.tile_bytes * s.n_ntiles;
-  s.smem_bytes = s.tile_bytes + (size_t)kStStages * kStStageBytes + 16 * 8;
+  s.smem_bytes = s.tile_bytes + stft_tc_ring(s.n_k16, std::max(1, hop / 16)).bytes + 16 * 8;
   s.stage_bytes = (size_t)4 * 32 * kStOutLd * sizeof(float);
   s.ok = s.smem_bytes <= (size_t)kTcSmemBudget;
   return s;
@@ -609,9 +661,12 @@ extern "C" int vadx_stft_power_tc_i16_ex(const int16_t* d_audio, int64_t in_stri
   const bool leaves_stream = pad_left > 0 || (int64_t)(n_frames - 1) * hop - pad_left + n_taps > n_samples;
   VADX_REQUIRE(!(d_mean || leaves_stream) || (d_dc_tables && n_edge_lo >= 0 && t_edge_hi >= n_edge_lo && t_edge_hi <= n_frames),
                "vadx_stft_power_tc_i16: padded frames / DC removal need the tables of vadx_pack_stft_dc_tc");
-  VADX_REQUIRE((in_stride % 8) == 0 && (hop % 8) == 0 && aligned16(d_audio) && aligned16(d_img),
-               "vadx_stft_power_tc_i16: stream stride and hop must be multiples of 8 samples, pointers 16-byte aligned");
-  StftTcShape s = stft_tc_shape(n_taps, n_bins);
+  VADX_REQUIRE((hop % 16) == 0,
+               "vadx_stft_power_tc_i16: hop %d is not a multiple of 16 samples (frames are read as shifted rows of 16-sample "
+               "hop slices); use vadx_stft_power_f32", hop);
+  VADX_REQUIRE((in_stride % 8) == 0 && aligned16(d_audio) && aligned16(d_img),
+               "vadx_stft_power_tc_i16: stream stride must be a multiple of 8 samples, pointers 16-byte aligned");
+  StftTcShape s = stft_tc_shape(n_taps, n_bins, hop);
   VADX_REQUIRE(s.ok, "vadx_stft_power_tc_i16: shape not supported");
   if (n_streams == 0) return VADX_OK;
   static PerDevice per_device;
@@ -621,15 +676,18 @@ extern "C" int vadx_stft_power_tc_i16_ex(const int16_t* d_audio, int64_t in_stri
     auto opt_in = [&](auto kern) {
       if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmemBudget);
     };
-    opt_in(stft_power_tc_kernel<false, false, 8>);  opt_in(stft_power_tc_kernel<false, false, 16>);
-    opt_in(stft_power_tc_kernel<true, false, 8>);   opt_in(stft_power_tc_kernel<true, false, 16>);
-    opt_in(stft_power_tc_kernel<false, true, 8>);   opt_in(stft_power_tc_kernel<false, true, 16>);
-    opt_in(stft_power_tc_kernel<true, true, 8>);    opt_in(stft_power_tc_kernel<true, true, 16>);
+    opt_in(stft_power_tc_kernel<false, false>);
+    opt_in(stft_power_tc_kernel<true, false>);
+    opt_in(stft_power_tc_kernel<false, true>);
+    opt_in(stft_power_tc_kernel<true, true>);
     return e;
   }));
+  const StftTcRing ring = stft_tc_ring(s.n_k16, hop / 16);
   StftTcArgs g{};
-  g.X = d_audio; g.in_stride = in_stride; g.L = n_samples; g.n_frames = n_frames; g.hop = hop;
-  g.Wimg = static_cast<const uint8_t*>(d_img); g.P = d_power; g.ldp = ld_power; g.M = n_streams * n_frames;
+  g.X = d_audio; g.in_stride = in_stride; g.L = n_samples; g.S = n_streams; g.n_frames = n_frames; g.hop = hop;
+  g.h16 = hop / 16; g.n_q = ring.n_q; g.tq = n_frames + ring.n_q - 1; g.rows = ring.rows; g.slice_units = ring.slice_units;
+  g.n_st = (int)ceil_div(g.h16, kStJ);
+  g.Wimg = static_cast<const uint8_t*>(d_img); g.P = d_power; g.ldp = ld_power;
   g.n_bins = n_bins; g.kc = s.kc; g.n_k16 = s.n_k16;
   g.pad_left = pad_left; g.mean = d_mean; g.mean_int = d_mean_int; g.dc = d_dc_tables; g.power_scale = power_scale; g.n_edge_lo = n_edge_lo; g.t_edge_hi = t_edge_hi;
   g.vec_p = ((ld_power & 3) == 0) && aligned16(d_power);
@@ -637,33 +695,25 @@ extern "C" int vadx_stft_power_tc_i16_ex(const int16_t* d_audio, int64_t in_stri
     static const int dbg = ab_env("VADX_TC_DEBUG", 0);
     g.debug = dbg;
   }
-  static const int opt = ab_env("VADX_ST_OPT", 3);   // bit 0 stack, bit 1 staged output
+  static const int opt = ab_env("VADX_ST_OPT", 2);   // bit 1 staged output
   {
     static const int bl = ab_env("VADX_TC_BACKOFF_LD", 64);
     static const int be = ab_env("VADX_TC_BACKOFF_EPI", 256);
     g.backoff_ld = (unsigned)bl; g.backoff_epi = (unsigned)be;
-    static const bool all_cols = ab_env("VADX_TC_ALLCOLS", 0) != 0;
-    g.k_live = all_cols ? s.kc * kTcBK : s.n_k16 * 16;
   }
-  g.stack = (opt & 1) ? 1 : 0;
   g.stage_out = ((opt & 2) && g.vec_p && s.smem_bytes + s.stage_bytes <= (size_t)kTcSmemBudget) ? 1 : 0;
   const size_t smem = s.smem_bytes + (g.stage_out ? s.stage_bytes : 0);
-  int64_t tiles = ceil_div(g.M, kTcBM);
+  // M rows are slots: each stream's frames and the Q - 1 halo slots behind them
+  int64_t tiles = ceil_div(n_streams * g.tq, kTcBM);
   VADX_REQUIRE(tiles <= 0x7fffffffLL, "vadx_stft_power_tc_i16: too many rows");
   g.n_tiles = (int)tiles;
   int per = std::max(1, n_sm / s.n_ntiles);
   dim3 grid((unsigned)std::min<int64_t>(tiles, per), (unsigned)s.n_ntiles);
   const bool ex = leaves_stream || d_mean, f16 = operand_format == VADX_TC_FMT_F16;
-  static const int lw = ab_env("VADX_ST_LOADERS", 16) == 8 ? 8 : 16;
-#define VADX_ST_LAUNCH(EXV, F16V)                                                                                   \
-  do {                                                                                                              \
-    if (lw == 8) stft_power_tc_kernel<EXV, F16V, 8><<<grid, 13 * 32, smem, (cudaStream_t)stream>>>(g);              \
-    else stft_power_tc_kernel<EXV, F16V, 16><<<grid, 21 * 32, smem, (cudaStream_t)stream>>>(g);                     \
-  } while (0)
-  if (ex && f16) VADX_ST_LAUNCH(true, true);
-  else if (ex) VADX_ST_LAUNCH(true, false);
-  else if (f16) VADX_ST_LAUNCH(false, true);
-  else VADX_ST_LAUNCH(false, false);
-#undef VADX_ST_LAUNCH
+  constexpr int kThreads = (kStLoaderWarps + 5) * 32;
+  if (ex && f16) stft_power_tc_kernel<true, true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(g);
+  else if (ex) stft_power_tc_kernel<true, false><<<grid, kThreads, smem, (cudaStream_t)stream>>>(g);
+  else if (f16) stft_power_tc_kernel<false, true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(g);
+  else stft_power_tc_kernel<false, false><<<grid, kThreads, smem, (cudaStream_t)stream>>>(g);
   return after_launch("vadx_stft_power_tc_i16");
 }

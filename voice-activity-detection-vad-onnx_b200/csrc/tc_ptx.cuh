@@ -65,6 +65,17 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;                        // SWIZZLE_128B
   return d;
 }
+// no-swizzle K-major operand: 8 x 16-byte core matrices, rows 16 B apart inside one; lbo = bytes between the two 8-element
+// halves of a K = 16 step, sbo = bytes between consecutive 8-row groups.  The start address only needs 16-byte alignment,
+// so an operand can begin any number of rows into a run of back-to-back core matrices (sbo = 128)
+__device__ __forceinline__ uint64_t umma_desc_noswz(uint32_t smem_addr, uint32_t lbo, uint32_t sbo) {
+  uint64_t d = 0;
+  d |= (uint64_t)((smem_addr & 0x3FFFFu) >> 4);  // start address, 16-byte units
+  d |= (uint64_t)((lbo >> 4) & 0x3FFFu) << 16;   // leading byte offset: the next 8 elements along K
+  d |= (uint64_t)((sbo >> 4) & 0x3FFFu) << 32;   // stride byte offset: the next 8 rows
+  d |= (uint64_t)1 << 46;                        // descriptor version (sm_100); layout type 0 (no swizzle) in bits 61-63
+  return d;
+}
 // kind::f16, A = B = bf16, D = fp32, both K-major, M = 128
 __device__ __forceinline__ uint32_t umma_idesc_bf16(int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(kTcBM >> 4) << 24);
@@ -107,6 +118,55 @@ __device__ __forceinline__ void umma_k64(uint32_t tmem_d, uint64_t adesc, uint64
       "@q3 tcgen05.mma.cta_group::1.kind::f16 [%0], a3, b3, %3, pt;\n"
       "}\n" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate_first), "r"(n_steps)
+      : "memory");
+}
+// two MMAs into one accumulator that share the B operand (the hi and lo terms of a split A operand), one predicate
+__device__ __forceinline__ void umma_x2(uint32_t tmem_d, uint64_t adesc0, uint64_t adesc1, uint64_t bdesc, uint32_t idesc,
+                                        uint32_t accumulate_first) {
+  asm volatile(
+      "{\n.reg .pred p, pt;\n"
+      "setp.ne.b32 p, %5, 0;\n"
+      "setp.eq.b32 pt, 0, 0;\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %3, %4, p;\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %2, %3, %4, pt;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc0), "l"(adesc1), "l"(bdesc), "r"(idesc), "r"(accumulate_first)
+      : "memory");
+}
+// Up to three K=16 MMA pairs of a split A operand (hi at a, lo at a + a_lo) in one asm block: pair i reads A at
+// a + i * a_step and B at b_i, so one column of a shifted-row operand is issued with its descriptor deltas added
+// inside the block (the issuing thread's instruction rate bounds short MMAs, see umma_k64).  n_pairs in 1..3; the
+// first MMA accumulates iff accumulate_first; lo_on = 0 drops the lo terms (a measurement switch).
+__device__ __forceinline__ void umma_split_x3(uint32_t tmem_d, uint64_t a, uint32_t a_step, uint32_t a_lo, uint64_t b0,
+                                              uint64_t b1, uint64_t b2, uint32_t idesc, uint32_t accumulate_first,
+                                              int n_pairs, uint32_t lo_on) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p0, pt, q1, q2, l0, l1, l2;\n"
+      ".reg .b64 st, lo, a0h, a1, a1h, a2, a2h;\n"
+      "setp.ne.b32 p0, %7, 0;\n"
+      "setp.eq.b32 pt, 0, 0;\n"
+      "setp.gt.s32 q1, %8, 1;\n"
+      "setp.gt.s32 q2, %8, 2;\n"
+      "setp.ne.b32 l0, %9, 0;\n"
+      "and.pred l1, l0, q1;\n"
+      "and.pred l2, l0, q2;\n"
+      "cvt.u64.u32 st, %2;\n"
+      "cvt.u64.u32 lo, %3;\n"
+      "add.u64 a0h, %1, lo;\n"
+      "add.u64 a1, %1, st;\n"
+      "add.u64 a1h, a1, lo;\n"
+      "add.u64 a2, a1, st;\n"
+      "add.u64 a2h, a2, lo;\n"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %4, %6, p0;\n"
+      "@l0 tcgen05.mma.cta_group::1.kind::f16 [%0], a0h, %4, %6, pt;\n"
+      "@q1 tcgen05.mma.cta_group::1.kind::f16 [%0], a1, %5, %6, pt;\n"
+      "@l1 tcgen05.mma.cta_group::1.kind::f16 [%0], a1h, %5, %6, pt;\n"
+      "@q2 tcgen05.mma.cta_group::1.kind::f16 [%0], a2, %10, %6, pt;\n"
+      "@l2 tcgen05.mma.cta_group::1.kind::f16 [%0], a2h, %10, %6, pt;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(a), "r"(a_step), "r"(a_lo), "l"(b0), "l"(b1), "r"(idesc), "r"(accumulate_first), "r"(n_pairs), "r"(lo_on),
+      "l"(b2)
       : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
