@@ -459,6 +459,49 @@ int vadx_stream_postprocess(const float* d_probs, int64_t ld_probs, const int32_
                             int n_frames, const vadx_stream_post_cfg* cfg, int32_t* d_state, int32_t* d_seg_count,
                             int32_t* d_segments, int max_segments, int32_t* d_open, void* stream);
 
+/* Stream-VAD slot server: n_slots independent streams, one tick per chunk of chunk_samples.  Per tick and slot s the
+ * caller gives d_n_samples[s] in [0, chunk_samples] and d_last[s] (uint8, != 0 = the stream's last chunk):
+ *   n > 0, last 0: feed a full chunk (n == chunk_samples; anything shorter is rejected);
+ *   n > 0, last 1: feed the stream's last chunk, which may be short, then finalize the slot;
+ *   n = 0, last 0: hold -- caches and segmenter state unchanged, no frames consumed;
+ *   n = 0, last 1: finalize now without new audio.
+ * Frames per chunk follow the reference loop (Inference_FireRed_ONNX.py:786-811): 1 + (n - frame_len) / frame_hop, one
+ * frame for a chunk shorter than frame_len, and the stream's total cut at the frames of its samples so far (a 64-bit
+ * sample counter in the state words 10..11).  Finalize emits a still-open segment's end at the last frame consumed and
+ * zeroes the slot's state and caches_out rows, so the next stream in the slot starts fresh.
+ *
+ * vadx_stream_serve_zero_tail runs BEFORE the model forward on the tick's chunk [n_slots][ld_chunk] int16: it zeroes
+ * samples [n, frame_len) of every chunk with 0 < n < frame_len (the reference zero-pads such a chunk to one frame);
+ * every other sample past n only reaches frames the server discards.
+ *
+ * vadx_stream_serve_step runs AFTER the forward on its probabilities d_probs [n_slots][ld_probs] (n_frames columns):
+ *   - runs the vadx_stream_postprocess segmenter (same state layout) over the tick's frames of every slot, writing the
+ *     frames consumed to d_frames [n_slots];
+ *   - applies the slot lifecycle to the caches (layout [n_cache_blocks][n_slots][cache_row] fp32, distinct buffers): a
+ *     held slot's caches_out rows <- its caches_in rows, a finalized slot's caches_out rows <- 0.  Both may be NULL
+ *     (segmenter and lifecycle without a model);
+ *   - writes the tick's events to d_events [n][3] int32 (slot, kind, frame), ordered by slot, then emission order, and
+ *     the header d_header[2] = {n, error bits}.  kind: VADX_SERVE_START (the segmenter confirmed a segment starting at
+ *     `frame`), VADX_SERVE_END (closed by min-silence or max-speech), VADX_SERVE_END_OF_STREAM (open at finalize);
+ *     frames are 0-based from the stream's first frame.  d_events must hold n_slots * (2 * n_frames + 1) triples.
+ *     A slot whose control words break the rules above is left unchanged and sets VADX_SERVE_ERR_* in the header.
+ *   - h_events / h_header (optional, together): page-locked host memory of the same sizes that receives the same
+ *     events and header from the device, so the bytes sent to the host grow with the events, not with n_slots.
+ * d_scratch = NULL: only writes the scratch size to *scratch_needed and returns. */
+#define VADX_SERVE_START 0
+#define VADX_SERVE_END 1
+#define VADX_SERVE_END_OF_STREAM 2
+#define VADX_SERVE_ERR_RANGE 1 /* n_samples outside [0, chunk_samples] */
+#define VADX_SERVE_ERR_SHORT 2 /* a short chunk that is not the stream's last */
+int vadx_stream_serve_zero_tail(int16_t* d_chunk, int64_t ld_chunk, const int32_t* d_n_samples, int64_t n_slots,
+                                int chunk_samples, int frame_len, void* stream);
+int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, int n_frames, const int32_t* d_n_samples,
+                           const uint8_t* d_last, int64_t n_slots, int chunk_samples, int frame_len, int frame_hop,
+                           const vadx_stream_post_cfg* cfg, int32_t* d_state, const float* d_caches_in,
+                           float* d_caches_out, int n_cache_blocks, int64_t cache_row, int32_t* d_frames,
+                           int32_t* d_events, int32_t* d_header, int32_t* h_events, int32_t* h_header, void* d_scratch,
+                           size_t scratch_bytes, size_t* scratch_needed, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Model-level API: the replacement for InferenceSession(...).run(...)
  * ------------------------------------------------------------------------------------------ */

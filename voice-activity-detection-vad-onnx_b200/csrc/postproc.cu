@@ -529,8 +529,84 @@ __global__ void __launch_bounds__(kPpWarps * 32) postprocess_frames_runs_kernel(
 // ---- Stream-VAD segmenter (FireRedVAD/Inference_FireRed_ONNX.py:307-490) ----
 // state words per stream: 0 head, 1 fill, 2 frame (1-based, last consumed), 3 mode, 4 speech run, 5 silence run,
 // 6 re-arm flag, 7 first frame of the open segment (0 = none), 8 last frame of the latest closed segment
-// (0 = none), 9 ring sum (float bits), 10..15 spare, 16.. ring of smooth_window floats.
+// (0 = none), 9 ring sum (float bits), 10..11 samples consumed (int64, low word first; the slot server's
+// counter, stream_serve_seg_kernel), 12..15 spare, 16.. ring of smooth_window floats.
 constexpr int kSpHeader = 16;
+
+// One stream's segmenter state in registers (the ring in local memory); load / store move it from / to its state words.
+struct SpState {
+  float ring[kMaxSmooth];
+  int head, fill, frame, mode, n_sp, n_si, open_from, closed_at;
+  bool rearm;
+  float acc;
+
+  __device__ __forceinline__ void load(const int32_t* st, int ws) {
+    for (int i = 0; i < ws; ++i) ring[i] = __int_as_float(st[kSpHeader + i]);
+    head = st[0]; fill = st[1]; frame = st[2]; mode = st[3]; n_sp = st[4]; n_si = st[5];
+    rearm = st[6] != 0;
+    open_from = st[7]; closed_at = st[8];
+    acc = __int_as_float(st[9]);
+  }
+  __device__ __forceinline__ void store(int32_t* st, int ws) const {
+    st[0] = head; st[1] = fill; st[2] = frame; st[3] = mode; st[4] = n_sp; st[5] = n_si; st[6] = rearm ? 1 : 0;
+    st[7] = open_from; st[8] = closed_at; st[9] = __float_as_int(acc);
+    for (int i = 0; i < ws; ++i) st[kSpHeader + i] = __float_as_int(ring[i]);
+  }
+};
+
+// One frame of the segmenter.  On return (all 1-based, 0 = not set): `opened` is the first frame of a segment
+// the segmenter confirmed on this frame; a segment closed on this frame iff begin > 0 && end > 0, and is
+// [begin, end].  At most one segment opens and at most one closes per frame; when both happen the open comes first.
+__device__ __forceinline__ void sp_frame(SpState& g, float pt, const vadx_stream_post_cfg& cfg, int ws, int pad,
+                                         int& opened, int& begin, int& end) {
+  ++g.frame;
+  float sm = pt;
+  if (ws > 1) {
+    const float gone = g.ring[g.head];
+    g.ring[g.head] = pt;
+    g.acc = __fadd_rn(g.acc, __fsub_rn(pt, gone));
+    g.head = g.head + 1 == ws ? 0 : g.head + 1;
+    if (g.fill < ws) ++g.fill;
+    sm = __fdiv_rn(g.acc, (float)g.fill);
+  }
+  const bool speech = sm >= cfg.threshold;
+  opened = begin = end = 0;
+  bool force_close = false;
+  if (g.rearm) { opened = begin = g.open_from = g.frame; g.rearm = false; }
+  if (g.mode == 0) {
+    if (speech) { g.mode = 1; g.n_sp = 1; }
+    else { ++g.n_si; g.n_sp = 0; }
+  } else if (g.mode == 1) {
+    if (speech) {
+      if (++g.n_sp >= cfg.min_speech_frame) {
+        g.mode = 2;
+        int b = g.frame - g.n_sp + 1 - pad;
+        if (b < 1) b = 1;
+        if (b < g.closed_at + 1) b = g.closed_at + 1;
+        opened = begin = g.open_from = b;
+        g.n_si = 0;
+      }
+    } else { g.mode = 0; g.n_si = 1; g.n_sp = 0; }
+  } else if (g.mode == 2) {
+    ++g.n_sp;
+    if (speech) { g.n_si = 0; force_close = g.n_sp >= cfg.max_speech_frame; }
+    else { g.mode = 3; g.n_si = 1; }
+  } else {
+    ++g.n_sp;
+    if (speech) { g.mode = 2; g.n_si = 0; force_close = g.n_sp >= cfg.max_speech_frame; }
+    else if (++g.n_si >= cfg.min_silence_frame) {
+      g.mode = 0;
+      begin = g.open_from; end = g.frame;
+      g.open_from = 0; g.closed_at = g.frame; g.n_sp = 0;
+    }
+  }
+  if (force_close) {
+    g.rearm = true;
+    g.n_sp = 0;
+    begin = g.open_from; end = g.frame;
+    g.open_from = 0; g.closed_at = g.frame;
+  }
+}
 
 __global__ void __launch_bounds__(128) stream_post_kernel(const float* __restrict__ probs, int64_t ld_probs,
                                                           const int32_t* __restrict__ n_frames_per_stream,
@@ -546,76 +622,190 @@ __global__ void __launch_bounds__(128) stream_post_kernel(const float* __restric
   const int ws = cfg.smooth_window < 1 ? 1 : cfg.smooth_window;
   const int pad = cfg.pad_start_frame > ws ? cfg.pad_start_frame : ws;
   int32_t* st = state + s * (int64_t)(kSpHeader + ws);
-  float ring[kMaxSmooth];
-  for (int i = 0; i < ws; ++i) ring[i] = __int_as_float(st[kSpHeader + i]);
-  int head = st[0], fill = st[1], frame = st[2], mode = st[3], n_sp = st[4], n_si = st[5];
-  bool rearm = st[6] != 0;
-  int open_from = st[7], closed_at = st[8];
-  float acc = __int_as_float(st[9]);
+  SpState g;
+  g.load(st, ws);
   int count = seg_count ? seg_count[s] : 0;
   int32_t* seg = segments ? segments + s * (int64_t)max_segments * 2 : nullptr;
   const float* p = probs + s * ld_probs;
   for (int t = 0; t < n; ++t) {
-    const float pt = __ldg(p + t);
-    ++frame;
-    float sm = pt;
-    if (ws > 1) {
-      const float gone = ring[head];
-      ring[head] = pt;
-      acc = __fadd_rn(acc, __fsub_rn(pt, gone));
-      head = head + 1 == ws ? 0 : head + 1;
-      if (fill < ws) ++fill;
-      sm = __fdiv_rn(acc, (float)fill);
-    }
-    const bool speech = sm >= cfg.threshold;
-    int begin = 0, end = 0;  // 1-based, 0 = not set
-    bool force_close = false;
-    if (rearm) { begin = open_from = frame; rearm = false; }
-    if (mode == 0) {
-      if (speech) { mode = 1; n_sp = 1; }
-      else { ++n_si; n_sp = 0; }
-    } else if (mode == 1) {
-      if (speech) {
-        if (++n_sp >= cfg.min_speech_frame) {
-          mode = 2;
-          int b = frame - n_sp + 1 - pad;
-          if (b < 1) b = 1;
-          if (b < closed_at + 1) b = closed_at + 1;
-          begin = open_from = b;
-          n_si = 0;
-        }
-      } else { mode = 0; n_si = 1; n_sp = 0; }
-    } else if (mode == 2) {
-      ++n_sp;
-      if (speech) { n_si = 0; force_close = n_sp >= cfg.max_speech_frame; }
-      else { mode = 3; n_si = 1; }
-    } else {
-      ++n_sp;
-      if (speech) { mode = 2; n_si = 0; force_close = n_sp >= cfg.max_speech_frame; }
-      else if (++n_si >= cfg.min_silence_frame) {
-        mode = 0;
-        begin = open_from; end = frame;
-        open_from = 0; closed_at = frame; n_sp = 0;
-      }
-    }
-    if (force_close) {
-      rearm = true;
-      n_sp = 0;
-      begin = open_from; end = frame;
-      open_from = 0; closed_at = frame;
-    }
+    int opened, begin, end;
+    sp_frame(g, __ldg(p + t), cfg, ws, pad, opened, begin, end);
     if (begin > 0 && end > 0) {
       if (seg && count < max_segments) { seg[2 * count] = begin - 1; seg[2 * count + 1] = end - 1; }
       ++count;
     }
   }
-  st[0] = head; st[1] = fill; st[2] = frame; st[3] = mode; st[4] = n_sp; st[5] = n_si; st[6] = rearm ? 1 : 0;
-  st[7] = open_from; st[8] = closed_at; st[9] = __float_as_int(acc);
-  for (int i = 0; i < ws; ++i) st[kSpHeader + i] = __float_as_int(ring[i]);
+  g.store(st, ws);
   if (seg_count) seg_count[s] = count;
   if (open_seg) {
-    open_seg[2 * s] = open_from > 0 ? open_from - 1 : -1;
-    open_seg[2 * s + 1] = open_from > 0 ? frame - 1 : -1;
+    open_seg[2 * s] = g.open_from > 0 ? g.open_from - 1 : -1;
+    open_seg[2 * s + 1] = g.open_from > 0 ? g.frame - 1 : -1;
+  }
+}
+
+// ---- Stream-VAD slot server (vadx_stream_serve_step) ----
+// Per slot and tick: an action (what happens to the slot's caches) and up to 2*T + 1 staged events.
+constexpr int kServeThreads = 128;
+enum : int8_t { kServeAdvance = 0, kServeHold = 1, kServeFinalize = 2 };
+
+// Zero samples [n, frame_len) of every slot fed a short chunk: a chunk shorter than one frame is zero-padded to
+// one frame (the reference's np.pad, Inference_FireRed_ONNX.py:790-792); later frames of a short chunk lie wholly
+// inside its n samples, and whatever lies past them only reaches frames the server discards.
+__global__ void __launch_bounds__(256) stream_serve_tail_kernel(int16_t* __restrict__ chunk, int64_t ld_chunk,
+                                                                const int32_t* __restrict__ n_samples,
+                                                                int64_t n_slots, int chunk_samples, int frame_len) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t s = i / frame_len;
+  const int k = (int)(i - s * frame_len);
+  if (s >= n_slots) return;
+  const int n = n_samples[s];
+  if (n > 0 && n < frame_len && k >= n && k < chunk_samples) chunk[s * ld_chunk + k] = 0;
+}
+
+// Thread per slot: validate the slot's control words, run the segmenter over this tick's frames, stage the events
+// slot-major in `staged` [S][2T+1] (kind, frame) and count them.  Each block writes its event total and its error
+// bits to block_info[2b], [2b+1]; stream_serve_emit_kernel turns those into offsets.  No atomics anywhere.
+__global__ void __launch_bounds__(kServeThreads) stream_serve_seg_kernel(
+    const float* __restrict__ probs, int64_t ld_probs, int n_frames_max, const int32_t* __restrict__ n_samples,
+    const uint8_t* __restrict__ last, int64_t n_slots, int chunk_samples, int frame_len, int frame_hop,
+    const vadx_stream_post_cfg cfg, int32_t* __restrict__ state, int32_t* __restrict__ frames_out,
+    int32_t* __restrict__ staged, int32_t* __restrict__ counts, int8_t* __restrict__ action,
+    int32_t* __restrict__ block_info) {
+  const int64_t s = (int64_t)blockIdx.x * kServeThreads + threadIdx.x;
+  int count = 0, err = 0;
+  if (s < n_slots) {
+    const int n = n_samples[s];
+    const bool fin = last[s] != 0;
+    err = (n < 0 || n > chunk_samples) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < chunk_samples && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+    int f = 0;
+    if (err || (n == 0 && !fin)) {
+      action[s] = kServeHold;                       // hold, or a rejected tick: the slot stays exactly as it was
+    } else {
+      const int ws = cfg.smooth_window < 1 ? 1 : cfg.smooth_window;
+      const int pad = cfg.pad_start_frame > ws ? cfg.pad_start_frame : ws;
+      int32_t* st = state + s * (int64_t)(kSpHeader + ws);
+      SpState g;
+      g.load(st, ws);
+      // frames of this chunk, cut at valid_frame_count(samples so far + n) (firered_vad.stream_frame_plan)
+      const int64_t total = ((int64_t)(uint32_t)st[10] | ((int64_t)st[11] << 32)) + n;
+      const int64_t valid = total < frame_len ? 0 : 1 + (total - frame_len) / frame_hop;
+      f = n == 0 ? 0 : (n < frame_len ? 1 : 1 + (n - frame_len) / frame_hop);
+      if (f > n_frames_max) f = n_frames_max;
+      if ((int64_t)f > valid - g.frame) f = (int)max((int64_t)0, valid - g.frame);
+      const int cap = 2 * n_frames_max + 1;
+      int2* ev = reinterpret_cast<int2*>(staged) + s * cap;
+      const float* p = probs + s * ld_probs;
+      for (int t = 0; t < f; ++t) {
+        int opened, begin, end;
+        sp_frame(g, __ldg(p + t), cfg, ws, pad, opened, begin, end);
+        if (opened > 0) ev[count++] = make_int2(VADX_SERVE_START, opened - 1);
+        if (begin > 0 && end > 0) ev[count++] = make_int2(VADX_SERVE_END, end - 1);
+      }
+      if (fin) {
+        if (g.open_from > 0) ev[count++] = make_int2(VADX_SERVE_END_OF_STREAM, g.frame - 1);
+        for (int i = 0; i < kSpHeader + ws; ++i) st[i] = 0;     // the next stream in this slot starts fresh
+        action[s] = kServeFinalize;
+      } else {
+        g.store(st, ws);
+        st[10] = (int32_t)(uint32_t)total;
+        st[11] = (int32_t)(total >> 32);
+        action[s] = kServeAdvance;
+      }
+    }
+    frames_out[s] = f;
+    counts[s] = count;
+  }
+  // block totals: warp sums, then the first warp adds the four
+  __shared__ int wsum[kServeThreads / 32], werr[kServeThreads / 32];
+  int c = count, e = err;
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    c += __shfl_xor_sync(0xffffffffu, c, off);
+    e |= __shfl_xor_sync(0xffffffffu, e, off);
+  }
+  if ((threadIdx.x & 31) == 0) { wsum[threadIdx.x >> 5] = c; werr[threadIdx.x >> 5] = e; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int tc = 0, te = 0;
+    for (int w = 0; w < kServeThreads / 32; ++w) { tc += wsum[w]; te |= werr[w]; }
+    block_info[2 * blockIdx.x] = tc;
+    block_info[2 * blockIdx.x + 1] = te;
+  }
+}
+
+// Blocks [0, n_seg_blocks): compact the staged events of their 128 slots to events [n][3] (slot, kind, frame) at
+// offset = events of all earlier blocks + events of earlier slots in the block; the last of them writes the header
+// {n_events, error bits}.  Every event and the header also go to the host mirror when one is given (pinned host memory,
+// written through unified addressing).  Blocks [n_seg_blocks, n_seg_blocks + S): slot blockIdx - n_seg_blocks applies
+// its action to the caches: hold copies its caches_in rows to caches_out, finalize zeroes its caches_out rows.
+__global__ void __launch_bounds__(kServeThreads) stream_serve_emit_kernel(
+    int64_t n_slots, int n_seg_blocks, int cap, const int32_t* __restrict__ staged, const int32_t* __restrict__ counts,
+    const int8_t* __restrict__ action, const int32_t* __restrict__ block_info, int32_t* __restrict__ events,
+    int32_t* __restrict__ header, int32_t* __restrict__ h_events, int32_t* __restrict__ h_header,
+    const float* __restrict__ caches_in, float* __restrict__ caches_out, int n_cache_blocks, int64_t cache_row) {
+  __shared__ int red[kServeThreads / 32][2];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if ((int)blockIdx.x >= n_seg_blocks) {
+    const int64_t s = blockIdx.x - n_seg_blocks;
+    const int8_t a = action[s];
+    if (a == kServeAdvance || !caches_out) return;
+    for (int r = 0; r < n_cache_blocks; ++r) {
+      const int64_t base = ((int64_t)r * n_slots + s) * cache_row;
+      if (a == kServeHold)
+        for (int64_t i = threadIdx.x; i < cache_row; i += kServeThreads) caches_out[base + i] = caches_in[base + i];
+      else
+        for (int64_t i = threadIdx.x; i < cache_row; i += kServeThreads) caches_out[base + i] = 0.0f;
+    }
+    return;
+  }
+  const int b = blockIdx.x;
+  // events and error bits of every earlier block (the last block also adds its own for the header)
+  int before = 0, err = 0;
+  const int upto = b == n_seg_blocks - 1 ? n_seg_blocks : b;
+  for (int i = threadIdx.x; i < upto; i += kServeThreads) {
+    if (i < b) before += block_info[2 * i];
+    err |= block_info[2 * i + 1];
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    before += __shfl_xor_sync(0xffffffffu, before, off);
+    err |= __shfl_xor_sync(0xffffffffu, err, off);
+  }
+  if (lane == 0) { red[warp][0] = before; red[warp][1] = err; }
+  __syncthreads();
+  before = 0; err = 0;
+  for (int w = 0; w < kServeThreads / 32; ++w) { before += red[w][0]; err |= red[w][1]; }
+  __syncthreads();
+  // exclusive scan of the slot counts within the block
+  const int64_t s = (int64_t)b * kServeThreads + threadIdx.x;
+  const int c = s < n_slots ? counts[s] : 0;
+  int incl = c;
+#pragma unroll
+  for (int off = 1; off < 32; off <<= 1) {
+    const int v = __shfl_up_sync(0xffffffffu, incl, off);
+    if (lane >= off) incl += v;
+  }
+  if (lane == 31) red[warp][0] = incl;
+  __syncthreads();
+  int at = before + incl - c;
+  for (int w = 0; w < warp; ++w) at += red[w][0];
+  if (c > 0) {
+    const int2* ev = reinterpret_cast<const int2*>(staged) + s * cap;
+    for (int j = 0; j < c; ++j) {
+      const int2 e = ev[j];
+      int32_t* o = events + 3 * (int64_t)(at + j);
+      o[0] = (int32_t)s; o[1] = e.x; o[2] = e.y;
+      if (h_events) {
+        int32_t* h = h_events + 3 * (int64_t)(at + j);
+        h[0] = (int32_t)s; h[1] = e.x; h[2] = e.y;
+      }
+    }
+  }
+  if (b == n_seg_blocks - 1 && threadIdx.x == kServeThreads - 1) {
+    int total = before;
+    for (int w = 0; w < kServeThreads / 32; ++w) total += red[w][0];
+    header[0] = total; header[1] = err;
+    if (h_header) { h_header[0] = total; h_header[1] = err; }
   }
 }
 
@@ -642,6 +832,80 @@ extern "C" int vadx_stream_postprocess(const float* d_probs, int64_t ld_probs, c
   stream_post_kernel<<<(unsigned)ceil_div(n_streams, 128), 128, 0, (cudaStream_t)stream>>>(
       d_probs, ld_probs, d_n_frames, n_streams, n_frames, *cfg, d_state, d_seg_count, d_segments, max_segments, d_open);
   return after_launch("vadx_stream_postprocess");
+}
+
+extern "C" int vadx_stream_serve_zero_tail(int16_t* d_chunk, int64_t ld_chunk, const int32_t* d_n_samples,
+                                           int64_t n_slots, int chunk_samples, int frame_len, void* stream) {
+  VADX_REQUIRE(d_chunk && d_n_samples, "vadx_stream_serve_zero_tail: null pointer");
+  VADX_REQUIRE(n_slots >= 0 && frame_len >= 1 && chunk_samples >= frame_len && ld_chunk >= chunk_samples,
+               "vadx_stream_serve_zero_tail: bad shape");
+  if (n_slots == 0) return VADX_OK;
+  stream_serve_tail_kernel<<<(unsigned)ceil_div(n_slots * frame_len, 256), 256, 0, (cudaStream_t)stream>>>(
+      d_chunk, ld_chunk, d_n_samples, n_slots, chunk_samples, frame_len);
+  return after_launch("vadx_stream_serve_zero_tail");
+}
+
+extern "C" int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, int n_frames, const int32_t* d_n_samples,
+                                      const uint8_t* d_last, int64_t n_slots, int chunk_samples, int frame_len,
+                                      int frame_hop, const vadx_stream_post_cfg* cfg, int32_t* d_state,
+                                      const float* d_caches_in, float* d_caches_out, int n_cache_blocks,
+                                      int64_t cache_row, int32_t* d_frames, int32_t* d_events, int32_t* d_header,
+                                      int32_t* h_events, int32_t* h_header, void* d_scratch, size_t scratch_bytes,
+                                      size_t* scratch_needed, void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && n_frames >= 1 && frame_len >= 1 && frame_hop >= 1 && chunk_samples >= frame_len,
+               "vadx_stream_serve_step: bad shape");
+  VADX_REQUIRE(1 + (chunk_samples - frame_len) / frame_hop <= n_frames,
+               "vadx_stream_serve_step: a full chunk gives %d frames, probs hold %d", 1 + (chunk_samples - frame_len) / frame_hop,
+               n_frames);
+  const int64_t cap = 2 * (int64_t)n_frames + 1;
+  const int64_t n_blocks = ceil_div(n_slots, kServeThreads);
+  const size_t o_counts = (size_t)round_up(n_slots * cap * 8, 256);
+  const size_t o_action = o_counts + (size_t)round_up(n_slots * 4, 256);
+  const size_t o_info = o_action + (size_t)round_up(n_slots, 256);
+  const size_t need = o_info + (size_t)round_up(n_blocks * 8, 256);
+  if (scratch_needed) *scratch_needed = need;
+  if (!d_scratch) return VADX_OK;                   // size query
+  VADX_REQUIRE(scratch_bytes >= need, "vadx_stream_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes, need);
+  VADX_REQUIRE(d_probs && d_n_samples && d_last && cfg && d_state && d_frames && d_events && d_header,
+               "vadx_stream_serve_step: null pointer");
+  VADX_REQUIRE(ld_probs >= n_frames, "vadx_stream_serve_step: ld_probs %lld < n_frames %d", (long long)ld_probs, n_frames);
+  VADX_REQUIRE(cfg->smooth_window <= kMaxSmooth, "vadx_stream_serve_step: smooth_window %d > %d", cfg->smooth_window,
+               kMaxSmooth);
+  VADX_REQUIRE((d_caches_in == nullptr) == (d_caches_out == nullptr) && (!d_caches_out || (n_cache_blocks >= 1 && cache_row >= 1)),
+               "vadx_stream_serve_step: caches_in and caches_out go together, with n_cache_blocks and cache_row >= 1");
+  VADX_REQUIRE(!d_caches_out || d_caches_in != d_caches_out, "vadx_stream_serve_step: caches_out must not alias caches_in");
+  VADX_REQUIRE((h_events == nullptr) == (h_header == nullptr), "vadx_stream_serve_step: h_events and h_header go together");
+  if (h_events) {
+    // the kernel writes the host mirror through unified addressing: it must be page-locked host memory whose device
+    // address is its host address.  Checked on eager calls; a capture replays the pointers an eager call checked.
+    cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
+    cudaError_t e = cudaStreamIsCapturing((cudaStream_t)stream, &cap_status);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaStreamIsCapturing");
+    if (cap_status == cudaStreamCaptureStatusNone) {
+      for (const void* h : {(const void*)h_events, (const void*)h_header}) {
+        cudaPointerAttributes at{};
+        e = cudaPointerGetAttributes(&at, h);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaPointerGetAttributes");
+        VADX_REQUIRE(at.type == cudaMemoryTypeHost && at.devicePointer == h,
+                     "vadx_stream_serve_step: the host mirror must be pinned host memory mapped at its own address");
+      }
+    }
+  }
+  StageTimer _timer(VADX_STAGE_POSTPROC, (cudaStream_t)stream, "stream_serve_seg_kernel", 4.0 * n_slots * n_frames);
+  char* sc = static_cast<char*>(d_scratch);
+  int32_t* staged = reinterpret_cast<int32_t*>(sc);
+  int32_t* counts = reinterpret_cast<int32_t*>(sc + o_counts);
+  int8_t* action = reinterpret_cast<int8_t*>(sc + o_action);
+  int32_t* info = reinterpret_cast<int32_t*>(sc + o_info);
+  stream_serve_seg_kernel<<<(unsigned)n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
+      d_probs, ld_probs, n_frames, d_n_samples, d_last, n_slots, chunk_samples, frame_len, frame_hop, *cfg, d_state,
+      d_frames, staged, counts, action, info);
+  VADX_TRY(after_launch("vadx_stream_serve_step"));
+  const int64_t grid = n_blocks + (d_caches_out ? n_slots : 0);
+  stream_serve_emit_kernel<<<(unsigned)grid, kServeThreads, 0, (cudaStream_t)stream>>>(
+      n_slots, (int)n_blocks, (int)cap, staged, counts, action, info, d_events, d_header, h_events, h_header, d_caches_in,
+      d_caches_out, n_cache_blocks, cache_row);
+  return after_launch("vadx_stream_serve_step");
 }
 
 extern "C" int vadx_postprocess_frames(const float* d_probs, int64_t ld_probs, const int32_t* d_n_frames,

@@ -265,9 +265,30 @@ def stream_frame_plan(lengths, chunk_samples: int = STREAM_CHUNK_SAMPLES):
 
 
 class _StreamGraphRunner:
-    """Two captured steps (caches a -> b and b -> a) over static buffers for one (streams, chunk) shape: a 160 ms
-    step is ~30 small launches, so eager execution is bound by host launch cost; replay costs two copies and
-    one graph launch."""
+    """Two captured tick bodies, body(0) (caches a -> b) and body(1) (b -> a), over static buffers: a 160 ms step is
+    ~30 small launches, so eager execution is bound by host launch cost; replay costs one graph launch."""
+
+    def __init__(self, body):
+        self.body = body
+        self.graphs = [None, None]
+
+    def step(self, k: int):
+        """runs body(k & 1)"""
+        import torch
+        i = k & 1
+        if self.graphs[i] is None:
+            self.body(i)                             # this step runs eagerly (constants, workspace) ...
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):                # ... and is recorded (not executed) for the later ones
+                self.body(i)
+            self.graphs[i] = g
+        else:
+            self.graphs[i].replay()
+
+
+class _LockStep:
+    """Static buffers of run_stream_vad_streams(graph=True) for one (streams, chunk) shape."""
 
     def __init__(self, session, S, chunk_samples, device, post):
         import torch
@@ -277,26 +298,15 @@ class _StreamGraphRunner:
         self.out = torch.empty((S, 1, T), dtype=torch.float32, device=device)
         self.n_frames = torch.zeros((S,), dtype=torch.int32, device=device)
         self.caches = [session.new_caches(S, device), session.new_caches(S, device)]
-        self.graphs = [None, None]
+        self.runner = _StreamGraphRunner(self._body)
+
+    def _body(self, i: int):
+        self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
+        self.post.feed(self.out[:, 0, :], self.n_frames)
 
     def step(self, k: int):
         """caches[k & 1] -> caches[1 - (k & 1)]"""
-        import torch
-        i = k & 1
-
-        def body():
-            self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
-            self.post.feed(self.out[:, 0, :], self.n_frames)
-
-        if self.graphs[i] is None:
-            body()                                   # this step runs eagerly (constants, workspace) ...
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):                # ... and is recorded (not executed) for the later ones
-                body()
-            self.graphs[i] = g
-        else:
-            self.graphs[i].replay()
+        self.runner.step(k)
 
 
 def run_stream_vad_streams(session: FireRedStreamSession, audio, lengths, chunk_samples: int = STREAM_CHUNK_SAMPLES,
@@ -319,7 +329,7 @@ def run_stream_vad_streams(session: FireRedStreamSession, audio, lengths, chunk_
         if r is None:
             p = PP.StreamVadPostprocessor(SMOOTH_WINDOW_SIZE, STREAM_VAD_THRESHOLD, PAD_START_FRAME, MIN_SPEECH_FRAME_STREAM,
                                           MAX_SPEECH_FRAME_STREAM, MIN_SILENCE_FRAME_STREAM, n_streams=S, device=audio.device)
-            r = runners[key] = _StreamGraphRunner(session, S, chunk_samples, audio.device, p)
+            r = runners[key] = _LockStep(session, S, chunk_samples, audio.device, p)
         r.post.reset()
         r.caches[0].zero_()
         T = session.frames(chunk_samples)
@@ -353,6 +363,107 @@ def run_stream_vad_streams(session: FireRedStreamSession, audio, lengths, chunk_
         probs[:, k, :].copy_(out[:, 0, :])
         a, b = b, a
     return probs.reshape(S, n_calls * T), post, a, plan
+
+
+class StreamServer:
+    """Live Stream-VAD serving: n_slots independent stream slots advance one tick per chunk of chunk_samples.  A stream
+    may start in any free slot on any tick.  Per tick and slot the caller gives the chunk (int16 [chunk_samples]), the
+    number of valid samples n and a `last` flag:
+
+        n > 0, last 0   feed a full chunk (n == chunk_samples)
+        n > 0, last 1   feed the stream's last chunk (may be short), then finalize and free the slot
+        n = 0, last 0   hold: the slot's caches and segmenter state are unchanged (idle slots, streams without audio)
+        n = 0, last 1   finalize and free the slot without new audio
+
+    Frames follow the reference loop (stream_frame_plan).  Samples past n never influence a result.  Each tick is one
+    model forward over all slots plus three small kernels (tail zeroing, segmenter, event compaction and cache
+    lifecycle), replayed as one CUDA graph per cache parity; it costs n_slots, not the number of live streams.  The
+    tick's result is a compact list of (slot, kind, frame) events: kind 0 = segment start, 1 = segment end
+    (min-silence or max-speech), 2 = end because the stream ended; frame counts from the stream's first frame.
+    Pairing a stream's starts and ends gives run_stream_vad(...).timestamps.
+
+    Inputs go through the static buffers `chunk`, `n_samples`, `last`: step() copies the arguments it is given into them
+    (non-blocking from pinned host memory), or a producer writes them and calls step() with no arguments."""
+
+    def __init__(self, session: FireRedStreamSession, n_slots: int, chunk_samples: int = STREAM_CHUNK_SAMPLES,
+                 smooth_window_size: int = SMOOTH_WINDOW_SIZE, speech_threshold: float = STREAM_VAD_THRESHOLD,
+                 pad_start_frame: int = PAD_START_FRAME, min_speech_frame: int = MIN_SPEECH_FRAME_STREAM,
+                 max_speech_frame: int = MAX_SPEECH_FRAME_STREAM, min_silence_frame: int = MIN_SILENCE_FRAME_STREAM,
+                 frames_per_second: int = 100, device=None, graph: bool = True):
+        import torch
+        if not isinstance(session, FireRedStreamSession):
+            raise ValueError("StreamServer needs a FireRedStreamSession (a streaming FireRed model)")
+        if getattr(session, "in_sample_rate", IN_SAMPLE_RATE) != IN_SAMPLE_RATE:
+            raise ValueError(f"StreamServer: the session must take {IN_SAMPLE_RATE} Hz audio")
+        if not 1 <= int(n_slots) <= FireRedSession.MAX_STREAMS_PER_CALL:
+            raise ValueError(f"StreamServer: n_slots must be in [1, {FireRedSession.MAX_STREAMS_PER_CALL}], got {n_slots}")
+        if int(chunk_samples) < WINDOW_LENGTH:
+            raise ValueError(f"StreamServer: chunk_samples must be at least one frame ({WINDOW_LENGTH}), got {chunk_samples}")
+        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        if dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        self.session, self.S, self.chunk_samples, self.device = session, int(n_slots), int(chunk_samples), dev
+        self.T = session.frames(self.chunk_samples)
+        self.chunk = torch.zeros((self.S, self.chunk_samples), dtype=torch.int16, device=dev)
+        self.n_samples = torch.zeros((self.S,), dtype=torch.int32, device=dev)
+        self.last = torch.zeros((self.S,), dtype=torch.uint8, device=dev)
+        self.out = torch.zeros((self.S, 1, self.T), dtype=torch.float32, device=dev)
+        self.caches = [session.new_caches(self.S, dev), session.new_caches(self.S, dev)]
+        with torch.cuda.device(dev):
+            self.seg = PP.StreamSlotSegmenter(smooth_window_size, speech_threshold, pad_start_frame, min_speech_frame,
+                                              max_speech_frame, min_silence_frame, self.S, self.T, self.chunk_samples,
+                                              WINDOW_LENGTH, HOP_LENGTH, dev, frames_per_second)
+        self._runner = _StreamGraphRunner(self._tick) if graph else None
+        self._k = 0
+
+    def _tick(self, i: int):
+        """the tick body on the static buffers, caches[i] -> caches[1 - i]; only libvadx launches"""
+        from . import lib
+        lib.check(lib.load().vadx_stream_serve_zero_tail(self.chunk.data_ptr(), self.chunk_samples,
+                                                         self.n_samples.data_ptr(), self.S, self.chunk_samples,
+                                                         WINDOW_LENGTH, lib.stream_ptr()))
+        self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
+        self.seg.enqueue(self.out[:, 0, :], self.n_samples, self.last, i, self.caches[i], self.caches[1 - i])
+
+    def _load(self, chunk, n_samples, last):
+        import torch
+        given = [a is not None for a in (chunk, n_samples, last)]
+        if any(given) and not all(given):
+            raise ValueError("StreamServer.step: pass chunk, n_samples and last together, or none of them")
+        if not all(given):
+            return
+        if not (torch.is_tensor(chunk) and chunk.dtype == torch.int16 and tuple(chunk.shape) == (self.S, self.chunk_samples)):
+            raise ValueError(f"StreamServer.step: chunk must be an int16 tensor [{self.S}, {self.chunk_samples}]")
+        PP._check_control(n_samples, last, self.S, "StreamServer.step")
+        for a in (chunk, n_samples, last):
+            if a.is_cuda and a.device != self.device:
+                raise ValueError(f"StreamServer.step: inputs must be on {self.device} or in host memory")
+        if not n_samples.is_cuda:        # host control words: checked here, before anything is copied
+            n = n_samples.numpy()
+            if n.min(initial=0) < 0 or n.max(initial=0) > self.chunk_samples:
+                raise ValueError(f"StreamServer.step: n_samples must be in [0, {self.chunk_samples}]")
+            if not last.is_cuda:
+                short = (n > 0) & (n < self.chunk_samples) & (last.view(torch.uint8).numpy() == 0)
+                if short.any():
+                    raise ValueError(f"StreamServer.step: slots {np.flatnonzero(short)[:8].tolist()} got a short chunk "
+                                     "that is not their stream's last")
+        self.chunk.copy_(chunk, non_blocking=True)
+        self.n_samples.copy_(n_samples, non_blocking=True)
+        self.last.copy_(last.view(torch.uint8), non_blocking=True)
+
+    def step(self, chunk=None, n_samples=None, last=None) -> PP.ServeTick:
+        """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, chunk_samples], n_samples int32
+        [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
+        for all three runs the tick on what the static buffers hold.  Returns the tick's handle (PP.ServeTick)."""
+        import torch
+        with torch.cuda.device(self.device):
+            self._load(chunk, n_samples, last)
+            if self._runner is not None:
+                self._runner.step(self._k)
+            else:
+                self._tick(self._k & 1)
+            self._k += 1
+            return self.seg.finish((self._k - 1) & 1, self.out[:, 0, :])
 
 
 def run_stream_vad(audio, session: FireRedStreamSession, chunk_samples: int = STREAM_CHUNK_SAMPLES) -> StreamVadResult:

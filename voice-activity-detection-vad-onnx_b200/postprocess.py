@@ -289,3 +289,150 @@ class StreamVadPostprocessor:
         self.feed(p.to(self.state.device, torch.float32).contiguous())
         ts = self.timestamps(before)
         return ts[0] if single else ts
+
+
+SERVE_START, SERVE_END, SERVE_END_OF_STREAM = 0, 1, 2      # event kinds of the slot server (include/vadx.h)
+SERVE_ERR_RANGE, SERVE_ERR_SHORT = 1, 2                    # error bits: n_samples out of range, short chunk not last
+
+
+class ServeTickError(ValueError):
+    """A tick in which the device rejected some slots' control words.  Those slots were held (left unchanged); every
+    other slot advanced, and its events are in `events` (as host_events / host_seconds would have returned them), so
+    a caller that catches this loses no segment.  `error` holds the VADX_SERVE_ERR_* bits."""
+
+    def __init__(self, msg, events, error):
+        super().__init__(msg)
+        self.events, self.error = events, error
+
+
+class ServeTick:
+    """One tick of the slot server.  Device side: `events` int32 [n_max, 3] (slot, kind, frame) of which the first
+    `n_events[0]` rows are this tick's, `error` (int32 [1], VADX_SERVE_ERR_* bits), `probs` fp32 [n_slots, T] and
+    `frames` int32 [n_slots] (the frames of `probs` each slot consumed).  probs and frames are valid until the next
+    tick; events, n_events and the host read-back until the tick after that."""
+
+    def __init__(self, owner, tick, parity, probs, frames, done):
+        self._owner, self._tick, self._i, self._done = owner, tick, parity, done
+        self.events, self.n_events, self.error = owner.events[parity], owner.header[parity][0:1], owner.header[parity][1:2]
+        self.probs, self.frames = probs, frames
+
+    def host_events(self):
+        """-> [(slot, kind, frame)] ordered by slot, then emission order.  Waits for the tick; raises ServeTickError
+        (a ValueError carrying the tick's events) if some slot's control words broke the contract on the device."""
+        if self._owner.ticks - self._tick > 2:
+            raise RuntimeError("ServeTick.host_events: two later ticks have reused this tick's buffers")
+        self._done.synchronize()
+        n, err = (int(v) for v in self._owner.h_header[self._i])
+        events = [tuple(e) for e in self._owner.h_events[self._i][:n].tolist()]
+        if err:
+            what = [m for b, m in ((SERVE_ERR_RANGE, "n_samples outside [0, chunk_samples]"),
+                                   (SERVE_ERR_SHORT, "a short chunk that is not the stream's last")) if err & b]
+            raise ServeTickError(f"stream server: rejected slot control words ({'; '.join(what)}); those slots were "
+                                 "held, the events of the others are in .events", events, err)
+        return events
+
+    def host_seconds(self):
+        """-> [(slot, kind, seconds)], seconds = frame * (1 / frames_per_second) as StreamVadPostprocessor.timestamps
+        forms.  A ServeTickError carries its events in seconds."""
+        inv = self._owner.inv_fps
+        try:
+            return [(s, k, int(f) * inv) for s, k, f in self.host_events()]
+        except ServeTickError as e:
+            e.events = [(s, k, int(f) * inv) for s, k, f in e.events]
+            raise
+
+    @property
+    def d2h_bytes(self) -> int:
+        """bytes the device sent to the host for this tick (header + events); read after host_events()"""
+        return 8 + 12 * int(self._owner.h_header[self._i][0])
+
+
+class StreamSlotSegmenter:
+    """The segmenter and slot lifecycle of the Stream-VAD slot server (vadx_stream_serve_step) for n_slots slots:
+    segmenter state (vadx_stream_post_state_words per slot, the layout StreamVadPostprocessor uses), scratch, and two
+    sets of event buffers (device and pinned host) used by alternate ticks.  `step` takes one tick's probabilities
+    fp32 [n_slots, n_frames] and control words; with caches it also holds / zeroes them.  Without a model it runs the
+    segmenter on given probabilities."""
+
+    def __init__(self, smooth_window_size, speech_threshold, pad_start_frame, min_speech_frame, max_speech_frame,
+                 min_silence_frame, n_slots: int, n_frames: int, chunk_samples: int, frame_len: int = 400,
+                 frame_hop: int = 160, device=None, frames_per_second: int = 100):
+        import torch
+        self.cfg = lib.StreamPostCfg(max(1, int(smooth_window_size)), float(np.float32(speech_threshold)),
+                                     int(pad_start_frame), int(min_speech_frame), int(max_speech_frame),
+                                     int(min_silence_frame))
+        self.S, self.T = int(n_slots), int(n_frames)
+        self.chunk_samples, self.frame_len, self.frame_hop = int(chunk_samples), int(frame_len), int(frame_hop)
+        self.inv_fps = 1.0 / frames_per_second
+        dev = device or torch.device("cuda", torch.cuda.current_device())
+        L = lib.load()
+        need = C.c_size_t()
+        lib.check(L.vadx_stream_serve_step(None, self.T, self.T, None, None, self.S, self.chunk_samples, self.frame_len,
+                                           self.frame_hop, C.byref(self.cfg), None, None, None, 0, 0, None, None, None,
+                                           None, None, None, 0, C.byref(need), None))
+        self.scratch = torch.empty((need.value,), dtype=torch.uint8, device=dev)
+        self.state = torch.zeros((self.S, L.vadx_stream_post_state_words(self.cfg.smooth_window)), dtype=torch.int32,
+                                 device=dev)
+        self.frames = torch.zeros((self.S,), dtype=torch.int32, device=dev)
+        n_max = self.S * (2 * self.T + 1)
+        self.events = [torch.zeros((n_max, 3), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.header = [torch.zeros((2,), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.h_events = [torch.zeros((n_max, 3), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.h_header = [torch.zeros((2,), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.ticks = 0
+
+    def reset(self):
+        """every slot idle (state zeroed); caches are the caller's"""
+        self.state.zero_()
+
+    def enqueue(self, probs, n_samples, last, parity: int, caches_in=None, caches_out=None, stream=None):
+        """Enqueue vadx_stream_serve_step for one tick (no checks beyond pointers: the server checks shapes once)."""
+        c = caches_in
+        lib.check(lib.load().vadx_stream_serve_step(
+            probs.data_ptr(), probs.stride(0), self.T, n_samples.data_ptr(), last.data_ptr(), self.S, self.chunk_samples,
+            self.frame_len, self.frame_hop, C.byref(self.cfg), self.state.data_ptr(), lib.ptr(c), lib.ptr(caches_out),
+            c.shape[0] if c is not None else 0, (c.shape[2] * c.shape[3]) if c is not None else 0, self.frames.data_ptr(),
+            self.events[parity].data_ptr(), self.header[parity].data_ptr(), self.h_events[parity].data_ptr(),
+            self.h_header[parity].data_ptr(), self.scratch.data_ptr(), self.scratch.numel(), None, lib.stream_ptr(stream)))
+
+    def step(self, probs, n_samples, last, caches_in=None, caches_out=None, stream=None) -> ServeTick:
+        """One tick on given CUDA tensors: probs fp32 [n_slots, >= n_frames] with contiguous rows, n_samples int32
+        [n_slots], last bool / uint8 [n_slots], caches fp32 [R, n_slots, P, Lb] (both or neither, distinct)."""
+        import torch
+        if not (torch.is_tensor(probs) and probs.is_cuda and probs.dtype == torch.float32 and probs.dim() == 2
+                and probs.shape[0] == self.S and probs.shape[1] >= self.T and probs.stride(1) == 1):
+            raise ValueError(f"StreamSlotSegmenter.step: probs must be CUDA fp32 [{self.S}, >= {self.T}] with contiguous rows")
+        _check_control(n_samples, last, self.S, "StreamSlotSegmenter.step", cuda=True)
+        if (caches_in is None) != (caches_out is None):
+            raise ValueError("StreamSlotSegmenter.step: caches_in and caches_out go together")
+        if caches_in is not None:
+            for c in (caches_in, caches_out):
+                if not (c.is_cuda and c.dtype == torch.float32 and c.dim() == 4 and c.shape[1] == self.S
+                        and c.is_contiguous() and c.shape == caches_in.shape):
+                    raise ValueError(f"StreamSlotSegmenter.step: caches must be contiguous CUDA fp32 [R, {self.S}, P, Lb]")
+            if caches_in.data_ptr() == caches_out.data_ptr():
+                raise ValueError("StreamSlotSegmenter.step: caches_out must be distinct from caches_in")
+        i = self.ticks & 1
+        self.enqueue(probs, n_samples, last.view(torch.uint8), i, caches_in, caches_out, stream)
+        return self.finish(i, probs, stream)
+
+    def finish(self, parity, probs, stream=None) -> ServeTick:
+        import torch
+        done = torch.cuda.Event()
+        done.record(stream)
+        t = ServeTick(self, self.ticks, parity, probs, self.frames, done)
+        self.ticks += 1
+        return t
+
+
+def _check_control(n_samples, last, S, who, cuda=None):
+    """dtype / shape of a tick's control arrays; cuda=True requires them on the device"""
+    import torch
+    if not (torch.is_tensor(n_samples) and n_samples.dtype == torch.int32 and tuple(n_samples.shape) == (S,)
+            and n_samples.is_contiguous()):
+        raise ValueError(f"{who}: n_samples must be a contiguous int32 tensor [{S}]")
+    if not (torch.is_tensor(last) and last.dtype in (torch.bool, torch.uint8) and tuple(last.shape) == (S,)
+            and last.is_contiguous()):
+        raise ValueError(f"{who}: last must be a contiguous bool or uint8 tensor [{S}]")
+    if cuda and not (n_samples.is_cuda and last.is_cuda):
+        raise ValueError(f"{who}: n_samples and last must be CUDA tensors")
