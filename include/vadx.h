@@ -502,6 +502,44 @@ int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, int n_frames,
                            int32_t* d_events, int32_t* d_header, int32_t* h_events, int32_t* h_header, void* d_scratch,
                            size_t scratch_bytes, size_t* scratch_needed, void* stream);
 
+/* Silero slot server: n_slots independent streams, one tick per W = windows_per_tick windows of 512 samples (16 kHz).
+ * Per tick and slot s the caller gives d_n_samples[s] in [0, W*512] and d_last[s] with the four actions of the
+ * Stream-VAD slot server above (feed a full chunk, feed a possibly short last chunk and finalize, hold, finalize
+ * without audio) and the same VADX_SERVE_ERR_* rules.  A slot consumes ceil(n / 512) windows; a short last window is
+ * zero-padded to 512 and counts as 512 samples, as the reference VADIterator counts a padded window.
+ *
+ * vadx_silero_serve_load runs BEFORE the model forward: it converts the int16 chunk d_chunk [n_slots][W*512]
+ * (contiguous) into columns [64, 64 + W*512) of the model input d_x [n_slots][64 + W*512] fp32 (both 16-byte
+ * aligned: the kernels move 16-byte vectors; a misaligned pointer is rejected), scaled by the
+ * reference's 0.000030517578 (exactly 2^-15 in float32) and zero from n on.  Columns 0..63 hold the slot's carried
+ * context and are not touched.  The forward reads d_x with input.row_stride = 64 + W*512 and input.n_windows = W.
+ *
+ * vadx_silero_serve_step runs AFTER the forward on its probabilities d_probs [W][ld_probs] (n_slots columns):
+ *   - runs the reference VADIterator (Silero/modeling_modified/utils_vad.py:494-585) over the slot's windows, comparing
+ *     each probability in double with `threshold` and `threshold - 0.15`, and a silence of (w - w_t) * 512 samples with
+ *     min_silence_samples; its state is d_state [n_slots][3] int32 (all zero = a fresh stream).  Writes the windows
+ *     consumed to d_windows [n_slots];
+ *   - rolls the context in d_x (may be NULL; 16-byte aligned): a fed slot's last 64 samples become columns 0..63, a finalized slot's
+ *     are zeroed, a held slot's are unchanged;
+ *   - applies the slot lifecycle to the LSTM state [2][n_slots][128] fp32 (d_state_in / d_state_out: both or neither,
+ *     distinct): a held slot's out rows <- its in rows, a finalized slot's out rows <- 0;
+ *   - writes the events to d_events [n][3] int32 (slot, kind, window) and d_header {n, error bits}, ordered by slot,
+ *     then emission order, and to the optional pinned host mirror h_events / h_header, as vadx_stream_serve_step does.
+ *     Windows count from the stream's first window, so a stream may run 2^31 windows (about 2.2 years).
+ *     VADX_SERVE_START: the iterator triggered on window w (its sample: max(0, w*512 - pad));
+ *     VADX_SERVE_END: the silence that ended the segment began on window w_t, the iterator's temp_end (its sample:
+ *     w_t*512 + pad); VADX_SERVE_END_OF_STREAM: the stream was finalized while triggered, the value is the windows
+ *     consumed.  d_events must hold n_slots * (W + 1) triples.
+ * d_scratch = NULL: only writes the scratch size to *scratch_needed and returns. */
+int vadx_silero_serve_load(const int16_t* d_chunk, const int32_t* d_n_samples, int64_t n_slots, int windows_per_tick,
+                           float* d_x, void* stream);
+int vadx_silero_serve_step(const float* d_probs, int64_t ld_probs, const int32_t* d_n_samples, const uint8_t* d_last,
+                           int64_t n_slots, int windows_per_tick, double threshold, double min_silence_samples,
+                           int32_t* d_state, float* d_x, const float* d_state_in, float* d_state_out,
+                           int32_t* d_windows, int32_t* d_events, int32_t* d_header, int32_t* h_events,
+                           int32_t* h_header, void* d_scratch, size_t scratch_bytes, size_t* scratch_needed,
+                           void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Model-level API: the replacement for InferenceSession(...).run(...)
  * ------------------------------------------------------------------------------------------ */

@@ -1,4 +1,5 @@
-"""FireRed Stream-VAD slot server (firered_vad.StreamServer) throughput on one GPU.
+"""Slot server throughput on one GPU: FireRed Stream-VAD (firered_vad.StreamServer, the default) or, with
+--family silero, Silero (silero_vad.StreamServer).
 
 For each slot count, at full occupancy and under churn (about 1 % of slots closing and joining per tick, 10 % held):
   device ms per tick      CUDA events around the tick's graph replay (inputs already in the static buffers)
@@ -6,11 +7,17 @@ For each slot count, at full occupancy and under churn (about 1 % of slots closi
   events, D2H bytes       per tick, from the host loop
   realtime streams        n_slots * 160 ms / device ms per tick
   lockstep ms per chunk   run_stream_vad_streams(graph=True) at the same S, alternating with the server in this process
+With --family silero, for each slot count and windows per tick (--windows, default 5 and 1) the same rows are
+measured, except: realtime streams = n_slots * W * 32 ms / device ms per tick, and instead of the lock-step chunk the
+bare forward of the same shape (SileroSession's engine over [n_slots][64 + W*512] rows, W windows, one CUDA graph),
+alternating with the server in this process.
 Prints one JSON line (card name and power limit read in the same run); --out also writes it to a file, --trace writes
 the torch.profiler launch list of a few server ticks.
 
   python tools/stream_server_bench.py --slots 4096,16384 --ticks 100 --out profiles/r03_stream_server.json \
       --trace profiles/r03_launches_stream_server.txt
+  python tools/stream_server_bench.py --family silero --slots 4096,16384 --out profiles/r04_silero_server.json \
+      --trace profiles/r04_launches_silero_server.txt
 """
 from __future__ import annotations
 
@@ -111,8 +118,100 @@ def bench_lockstep(session, audio, lengths, reps):
     return a.elapsed_time(b) / (reps * n_calls)
 
 
+class SileroForward:
+    """the bare forward of a Silero server tick: the session's engine over [S][64 + W*512] rows and W windows, state
+    a -> b, captured as one CUDA graph on buffers of its own"""
+
+    def __init__(self, session, S, W):
+        import torch
+        c = session.cfg
+        self.session, self.S, self.W = session, S, W
+        self.stride = c.context + W * c.window
+        g = torch.Generator(device="cuda").manual_seed(S + W)
+        self.x = (torch.rand((S, self.stride), generator=g, device="cuda") - 0.5) * 0.5
+        self.out = torch.empty((W, S, 1), dtype=torch.float32, device="cuda")
+        self.state = [torch.zeros((2, S, c.hidden), dtype=torch.float32, device="cuda") for _ in range(2)]
+        self._run()
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self._run()
+
+    def _run(self):
+        self.session.forward_windows(self.x, self.out, self.state[0], self.state[1], self.W, self.stride)
+
+    def time(self, reps):
+        import torch
+        for _ in range(5):
+            self.graph.replay()
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        for _ in range(reps):
+            self.graph.replay()
+        b.record()
+        torch.cuda.synchronize()
+        return a.elapsed_time(b) / reps
+
+
+def write_trace(path, server, traffic, title):
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for k in range(5):
+            server.step(*traffic.tick(k)).host_events()
+        torch.cuda.synchronize()
+    with open(path, "w") as f:
+        f.write(f"# {title}\n")
+        f.write(prof.key_averages().table(sort_by="cuda_time_total", row_limit=40))
+        names = [e.key for e in prof.key_averages()]
+        f.write("\nat:: kernels: %s\n" % ([n for n in names if "at::" in n] or "none"))
+
+
+def main_silero(a, info):
+    import torch
+    import vadx
+    from vadx import silero_vad as SV, weights as W
+    cfg = W.SileroConfig()
+    sess = vadx.SileroSession(W.silero_random_init(cfg, 0), cfg)
+    rows = []
+    for S in [int(v) for v in a.slots.split(",")]:
+        for Wt in [int(v) for v in a.windows.split(",")]:
+            C = Wt * cfg.window
+            fwd = SileroForward(sess, S, Wt)
+            for mode, churn, hold in (("full", 0.0, 0.0), ("churn", 0.01, 0.10)):
+                traffic = Traffic(S, C, churn, hold, seed=S + Wt + len(mode))
+                server = SV.StreamServer(sess, S, windows_per_tick=Wt)
+                res = {"dev": [], "host": [], "events": [], "d2h": [], "fwd": []}
+                for _ in range(a.rounds):
+                    d, h, e, b = bench_server(server, traffic, a.ticks, a.warmup)
+                    res["dev"].append(d), res["host"].append(h), res["events"].append(e), res["d2h"].append(b)
+                    res["fwd"].append(fwd.time(a.ticks))
+                dev = float(np.median(res["dev"]))
+                bare = float(np.median(res["fwd"]))
+                row = {"n_slots": S, "windows_per_tick": Wt, "traffic": mode, "device_ms_per_tick": round(dev, 4),
+                       "device_ms_per_tick_rounds": [round(v, 4) for v in res["dev"]],
+                       "host_ms_per_tick": round(float(np.median(res["host"])), 4),
+                       "events_per_tick": round(float(np.mean(res["events"])), 2),
+                       "d2h_bytes_per_tick": round(float(np.mean(res["d2h"])), 1),
+                       "realtime_streams": int(S * Wt * 32.0 / dev),
+                       "forward_ms": round(bare, 4), "forward_ms_rounds": [round(v, 4) for v in res["fwd"]],
+                       "tick_over_forward": round(dev / bare, 3)}
+                rows.append(row)
+                print(json.dumps(row), file=sys.stderr)
+                if a.trace and len(rows) == 1:
+                    write_trace(a.trace, server, traffic, f"silero StreamServer, {S} slots, W = {Wt}, 5 ticks, {info}")
+                del server
+            del fwd
+            torch.cuda.empty_cache()
+    return {"what": "silero StreamServer tick vs the bare forward of the same shape", "card": info,
+            "ticks": a.ticks, "rounds": a.rounds, "results": rows}
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
+    ap.add_argument("--family", choices=("firered", "silero"), default="firered")
+    ap.add_argument("--windows", default="5,1", help="silero: windows per tick to measure")
     ap.add_argument("--slots", default="4096,16384")
     ap.add_argument("--ticks", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
@@ -127,6 +226,14 @@ def main(argv=None):
         raise SystemExit("stream_server_bench: needs a CUDA device")
     torch.cuda.set_device(0)
     info = card()
+    if a.family == "silero":
+        out = main_silero(a, info)
+        line = json.dumps(out)
+        print(line)
+        if a.out:
+            with open(a.out, "w") as f:
+                f.write(line + "\n")
+        return
     cfg = W.FireRedConfig(N2=0, S2=0, streaming=True)
     sess = vadx.FireRedStreamSession(W.firered_random_init(cfg, 5), cfg)
     C = FV.STREAM_CHUNK_SAMPLES
@@ -158,17 +265,7 @@ def main(argv=None):
             rows.append(row)
             print(json.dumps(row), file=sys.stderr)
             if a.trace and len(rows) == 1:
-                from torch.profiler import ProfilerActivity, profile
-                torch.cuda.synchronize()
-                with profile(activities=[ProfilerActivity.CUDA]) as prof:
-                    for k in range(5):
-                        server.step(*traffic.tick(k)).host_events()
-                    torch.cuda.synchronize()
-                with open(a.trace, "w") as f:
-                    f.write(f"# StreamServer, {S} slots, 5 ticks, {info}\n")
-                    f.write(prof.key_averages().table(sort_by="cuda_time_total", row_limit=40))
-                    names = [e.key for e in prof.key_averages()]
-                    f.write("\nat:: kernels: %s\n" % ([n for n in names if "at::" in n] or "none"))
+                write_trace(a.trace, server, traffic, f"StreamServer, {S} slots, 5 ticks, {info}")
             del server
             torch.cuda.empty_cache()
     out = {"what": "firered StreamServer tick vs run_stream_vad_streams(graph=True) chunk", "card": info,

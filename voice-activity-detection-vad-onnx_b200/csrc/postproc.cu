@@ -662,6 +662,26 @@ __global__ void __launch_bounds__(256) stream_serve_tail_kernel(int16_t* __restr
   if (n > 0 && n < frame_len && k >= n && k < chunk_samples) chunk[s * ld_chunk + k] = 0;
 }
 
+// Block totals of a serve segmenter kernel: warp sums, then the first warp adds the four.  Every thread of the block
+// calls this (threads past n_slots with count = err = 0).
+__device__ __forceinline__ void serve_block_totals(int count, int err, int32_t* __restrict__ block_info) {
+  __shared__ int wsum[kServeThreads / 32], werr[kServeThreads / 32];
+  int c = count, e = err;
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    c += __shfl_xor_sync(0xffffffffu, c, off);
+    e |= __shfl_xor_sync(0xffffffffu, e, off);
+  }
+  if ((threadIdx.x & 31) == 0) { wsum[threadIdx.x >> 5] = c; werr[threadIdx.x >> 5] = e; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int tc = 0, te = 0;
+    for (int w = 0; w < kServeThreads / 32; ++w) { tc += wsum[w]; te |= werr[w]; }
+    block_info[2 * blockIdx.x] = tc;
+    block_info[2 * blockIdx.x + 1] = te;
+  }
+}
+
 // Thread per slot: validate the slot's control words, run the segmenter over this tick's frames, stage the events
 // slot-major in `staged` [S][2T+1] (kind, frame) and count them.  Each block writes its event total and its error
 // bits to block_info[2b], [2b+1]; stream_serve_emit_kernel turns those into offsets.  No atomics anywhere.
@@ -715,22 +735,7 @@ __global__ void __launch_bounds__(kServeThreads) stream_serve_seg_kernel(
     frames_out[s] = f;
     counts[s] = count;
   }
-  // block totals: warp sums, then the first warp adds the four
-  __shared__ int wsum[kServeThreads / 32], werr[kServeThreads / 32];
-  int c = count, e = err;
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) {
-    c += __shfl_xor_sync(0xffffffffu, c, off);
-    e |= __shfl_xor_sync(0xffffffffu, e, off);
-  }
-  if ((threadIdx.x & 31) == 0) { wsum[threadIdx.x >> 5] = c; werr[threadIdx.x >> 5] = e; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int tc = 0, te = 0;
-    for (int w = 0; w < kServeThreads / 32; ++w) { tc += wsum[w]; te |= werr[w]; }
-    block_info[2 * blockIdx.x] = tc;
-    block_info[2 * blockIdx.x + 1] = te;
-  }
+  serve_block_totals(count, err, block_info);
 }
 
 // Blocks [0, n_seg_blocks): compact the staged events of their 128 slots to events [n][3] (slot, kind, frame) at
@@ -809,6 +814,107 @@ __global__ void __launch_bounds__(kServeThreads) stream_serve_emit_kernel(
   }
 }
 
+// ---- Silero slot server (vadx_silero_serve_load, vadx_silero_serve_step) ----
+// A slot's model input row is [64 context | W*512 samples]; window w of the tick is columns [w*512, w*512 + 576).
+constexpr int kSileroWindow = 512, kSileroContext = 64, kSileroHidden = 128;
+constexpr int kSileroServeStateWords = 3;   // {windows so far, triggered, temp_end window + 1 (0 = none)}
+constexpr int kSileroMaxWindowsPerTick = 1 << 20;   // keeps W * 512 + 64 an int
+// the reference's int16 scale (Inference_Silero_VAD_ONNX.py:83); as float32 it is exactly 2^-15, so the product is exact
+constexpr float kSileroInt16Scale = 0.000030517578f;
+
+// Thread per 8 samples: int16 chunk [S][W*512] -> scaled fp32 in columns [64, 64 + W*512) of x, zero from n on.
+// The context columns 0..63 hold the slot's carried samples and are not touched.
+__global__ void __launch_bounds__(256) silero_serve_load_kernel(const int16_t* __restrict__ chunk,
+                                                                const int32_t* __restrict__ n_samples, int64_t n_slots,
+                                                                int chunk_samples, float* __restrict__ x) {
+  const int per_row = chunk_samples / 8;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t s = i / per_row;
+  if (s >= n_slots) return;
+  const int k0 = (int)(i - s * per_row) * 8;
+  const int n = n_samples[s];
+  const int4 raw = __ldg(reinterpret_cast<const int4*>(chunk + s * chunk_samples + k0));
+  const int16_t* v = reinterpret_cast<const int16_t*>(&raw);
+  float f[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) f[j] = k0 + j < n ? (float)v[j] * kSileroInt16Scale : 0.0f;
+  float4* o = reinterpret_cast<float4*>(x + s * (int64_t)(kSileroContext + chunk_samples) + kSileroContext + k0);
+  o[0] = make_float4(f[0], f[1], f[2], f[3]);
+  o[1] = make_float4(f[4], f[5], f[6], f[7]);
+}
+
+// Thread per slot: validate the control words (same rules and error bits as stream_serve_seg_kernel), run the
+// reference VADIterator (utils_vad.py:494-585) over the slot's ceil(n/512) windows of probs [W][ld_probs], comparing
+// in double as the reference compares Python floats, and stage at most W + 1 events (kind, window) in `staged`
+// [S][W+1].  Then the block rolls its slots' context in x: a fed slot's last 64 samples become columns 0..63, a
+// finalized slot's are zeroed, a held one's are left alone.
+__global__ void __launch_bounds__(kServeThreads) silero_serve_seg_kernel(
+    const float* __restrict__ probs, int64_t ld_probs, const int32_t* __restrict__ n_samples,
+    const uint8_t* __restrict__ last, int64_t n_slots, int W, double threshold, double min_silence_samples,
+    int32_t* __restrict__ state, float* __restrict__ x, int32_t* __restrict__ windows_out, int32_t* __restrict__ staged,
+    int32_t* __restrict__ counts, int8_t* __restrict__ action, int32_t* __restrict__ block_info) {
+  __shared__ int8_t s_act[kServeThreads];
+  const int64_t s = (int64_t)blockIdx.x * kServeThreads + threadIdx.x;
+  const int chunk_samples = W * kSileroWindow;
+  int count = 0, err = 0;
+  int8_t act = kServeHold;
+  if (s < n_slots) {
+    const int n = n_samples[s];
+    const bool fin = last[s] != 0;
+    err = (n < 0 || n > chunk_samples) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < chunk_samples && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+    int nw = 0;
+    if (!err && (n > 0 || fin)) {
+      int32_t* st = state + s * kSileroServeStateWords;
+      int cur = st[0], tend = st[2];
+      bool trig = st[1] != 0;
+      nw = (n + kSileroWindow - 1) / kSileroWindow;
+      int2* ev = reinterpret_cast<int2*>(staged) + s * (W + 1);
+      const double neg = threshold - 0.15;
+      for (int w = 0; w < nw; ++w) {
+        const double p = (double)__ldg(probs + w * ld_probs + s);
+        const int gw = cur + w;
+        if (p >= threshold) {
+          tend = 0;
+          if (!trig) { trig = true; ev[count++] = make_int2(VADX_SERVE_START, gw); }
+        } else if (trig && p < neg) {
+          if (tend == 0) tend = gw + 1;
+          // current_sample - temp_end = (gw - w_t) * 512 samples
+          if ((double)(gw - (tend - 1)) * kSileroWindow >= min_silence_samples) {
+            ev[count++] = make_int2(VADX_SERVE_END, tend - 1);
+            tend = 0;
+            trig = false;
+          }
+        }
+      }
+      cur += nw;
+      if (fin) {
+        if (trig) ev[count++] = make_int2(VADX_SERVE_END_OF_STREAM, cur);
+        st[0] = st[1] = st[2] = 0;                  // the next stream in this slot starts fresh
+        act = kServeFinalize;
+      } else {
+        st[0] = cur; st[1] = trig ? 1 : 0; st[2] = tend;
+        act = kServeAdvance;
+      }
+    }
+    action[s] = act;
+    windows_out[s] = nw;
+    counts[s] = count;
+  }
+  s_act[threadIdx.x] = act;
+  serve_block_totals(count, err, block_info);      // its barrier also publishes s_act
+  if (!x) return;
+  // 16 threads per row: columns 0..63 <- columns [W*512, W*512 + 64) (fed) or 0 (finalized), as float4s
+  const int64_t ld_x = kSileroContext + chunk_samples;
+  for (int i = threadIdx.x; i < kServeThreads * (kSileroContext / 4); i += kServeThreads) {
+    const int r = i / (kSileroContext / 4), q = i % (kSileroContext / 4);
+    const int64_t ss = (int64_t)blockIdx.x * kServeThreads + r;
+    const int8_t a = s_act[r];
+    if (ss >= n_slots || a == kServeHold) continue;
+    float4* row = reinterpret_cast<float4*>(x + ss * ld_x);
+    row[q] = a == kServeFinalize ? make_float4(0.0f, 0.0f, 0.0f, 0.0f) : row[chunk_samples / 4 + q];
+  }
+}
+
 }  // namespace vadx
 
 using namespace vadx;
@@ -845,6 +951,54 @@ extern "C" int vadx_stream_serve_zero_tail(int16_t* d_chunk, int64_t ld_chunk, c
   return after_launch("vadx_stream_serve_zero_tail");
 }
 
+namespace {
+// Scratch of a serve step: staged events [S][cap] int32 pairs, counts [S], actions [S], block totals [blocks][2].
+struct ServeScratch {
+  int64_t cap, n_blocks;
+  size_t o_counts, o_action, o_info, need;
+  ServeScratch(int64_t n_slots, int64_t cap_) : cap(cap_), n_blocks(ceil_div(n_slots, kServeThreads)) {
+    o_counts = (size_t)round_up(n_slots * cap * 8, 256);
+    o_action = o_counts + (size_t)round_up(n_slots * 4, 256);
+    o_info = o_action + (size_t)round_up(n_slots, 256);
+    need = o_info + (size_t)round_up(n_blocks * 8, 256);
+  }
+  int32_t* staged(void* p) const { return static_cast<int32_t*>(p); }
+  int32_t* counts(void* p) const { return reinterpret_cast<int32_t*>(static_cast<char*>(p) + o_counts); }
+  int8_t* action(void* p) const { return reinterpret_cast<int8_t*>(static_cast<char*>(p) + o_action); }
+  int32_t* info(void* p) const { return reinterpret_cast<int32_t*>(static_cast<char*>(p) + o_info); }
+};
+
+// The emit kernel writes the host mirror through unified addressing: it must be page-locked host memory whose device
+// address is its host address.  Checked on eager calls; a capture replays the pointers an eager call checked.
+int check_host_mirror(const int32_t* h_events, const int32_t* h_header, void* stream, const char* who) {
+  VADX_REQUIRE((h_events == nullptr) == (h_header == nullptr), "%s: h_events and h_header go together", who);
+  if (!h_events) return VADX_OK;
+  cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
+  cudaError_t e = cudaStreamIsCapturing((cudaStream_t)stream, &cap_status);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaStreamIsCapturing");
+  if (cap_status != cudaStreamCaptureStatusNone) return VADX_OK;
+  for (const void* h : {(const void*)h_events, (const void*)h_header}) {
+    cudaPointerAttributes at{};
+    e = cudaPointerGetAttributes(&at, h);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaPointerGetAttributes");
+    VADX_REQUIRE(at.type == cudaMemoryTypeHost && at.devicePointer == h,
+                 "%s: the host mirror must be pinned host memory mapped at its own address", who);
+  }
+  return VADX_OK;
+}
+
+// stream_serve_emit_kernel over a segmenter's staged events, plus one block per slot when there are caches
+int serve_emit(const ServeScratch& sl, int64_t n_slots, void* d_scratch, int32_t* d_events, int32_t* d_header,
+               int32_t* h_events, int32_t* h_header, const float* d_caches_in, float* d_caches_out, int n_cache_blocks,
+               int64_t cache_row, void* stream, const char* who) {
+  const int64_t grid = sl.n_blocks + (d_caches_out ? n_slots : 0);
+  stream_serve_emit_kernel<<<(unsigned)grid, kServeThreads, 0, (cudaStream_t)stream>>>(
+      n_slots, (int)sl.n_blocks, (int)sl.cap, sl.staged(d_scratch), sl.counts(d_scratch), sl.action(d_scratch),
+      sl.info(d_scratch), d_events, d_header, h_events, h_header, d_caches_in, d_caches_out, n_cache_blocks, cache_row);
+  return after_launch(who);
+}
+}  // namespace
+
 extern "C" int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, int n_frames, const int32_t* d_n_samples,
                                       const uint8_t* d_last, int64_t n_slots, int chunk_samples, int frame_len,
                                       int frame_hop, const vadx_stream_post_cfg* cfg, int32_t* d_state,
@@ -857,15 +1011,10 @@ extern "C" int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, in
   VADX_REQUIRE(1 + (chunk_samples - frame_len) / frame_hop <= n_frames,
                "vadx_stream_serve_step: a full chunk gives %d frames, probs hold %d", 1 + (chunk_samples - frame_len) / frame_hop,
                n_frames);
-  const int64_t cap = 2 * (int64_t)n_frames + 1;
-  const int64_t n_blocks = ceil_div(n_slots, kServeThreads);
-  const size_t o_counts = (size_t)round_up(n_slots * cap * 8, 256);
-  const size_t o_action = o_counts + (size_t)round_up(n_slots * 4, 256);
-  const size_t o_info = o_action + (size_t)round_up(n_slots, 256);
-  const size_t need = o_info + (size_t)round_up(n_blocks * 8, 256);
-  if (scratch_needed) *scratch_needed = need;
+  const ServeScratch sl(n_slots, 2 * (int64_t)n_frames + 1);
+  if (scratch_needed) *scratch_needed = sl.need;
   if (!d_scratch) return VADX_OK;                   // size query
-  VADX_REQUIRE(scratch_bytes >= need, "vadx_stream_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes, need);
+  VADX_REQUIRE(scratch_bytes >= sl.need, "vadx_stream_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes, sl.need);
   VADX_REQUIRE(d_probs && d_n_samples && d_last && cfg && d_state && d_frames && d_events && d_header,
                "vadx_stream_serve_step: null pointer");
   VADX_REQUIRE(ld_probs >= n_frames, "vadx_stream_serve_step: ld_probs %lld < n_frames %d", (long long)ld_probs, n_frames);
@@ -874,38 +1023,57 @@ extern "C" int vadx_stream_serve_step(const float* d_probs, int64_t ld_probs, in
   VADX_REQUIRE((d_caches_in == nullptr) == (d_caches_out == nullptr) && (!d_caches_out || (n_cache_blocks >= 1 && cache_row >= 1)),
                "vadx_stream_serve_step: caches_in and caches_out go together, with n_cache_blocks and cache_row >= 1");
   VADX_REQUIRE(!d_caches_out || d_caches_in != d_caches_out, "vadx_stream_serve_step: caches_out must not alias caches_in");
-  VADX_REQUIRE((h_events == nullptr) == (h_header == nullptr), "vadx_stream_serve_step: h_events and h_header go together");
-  if (h_events) {
-    // the kernel writes the host mirror through unified addressing: it must be page-locked host memory whose device
-    // address is its host address.  Checked on eager calls; a capture replays the pointers an eager call checked.
-    cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
-    cudaError_t e = cudaStreamIsCapturing((cudaStream_t)stream, &cap_status);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaStreamIsCapturing");
-    if (cap_status == cudaStreamCaptureStatusNone) {
-      for (const void* h : {(const void*)h_events, (const void*)h_header}) {
-        cudaPointerAttributes at{};
-        e = cudaPointerGetAttributes(&at, h);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaPointerGetAttributes");
-        VADX_REQUIRE(at.type == cudaMemoryTypeHost && at.devicePointer == h,
-                     "vadx_stream_serve_step: the host mirror must be pinned host memory mapped at its own address");
-      }
-    }
-  }
+  VADX_TRY(check_host_mirror(h_events, h_header, stream, "vadx_stream_serve_step"));
   StageTimer _timer(VADX_STAGE_POSTPROC, (cudaStream_t)stream, "stream_serve_seg_kernel", 4.0 * n_slots * n_frames);
-  char* sc = static_cast<char*>(d_scratch);
-  int32_t* staged = reinterpret_cast<int32_t*>(sc);
-  int32_t* counts = reinterpret_cast<int32_t*>(sc + o_counts);
-  int8_t* action = reinterpret_cast<int8_t*>(sc + o_action);
-  int32_t* info = reinterpret_cast<int32_t*>(sc + o_info);
-  stream_serve_seg_kernel<<<(unsigned)n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
+  stream_serve_seg_kernel<<<(unsigned)sl.n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
       d_probs, ld_probs, n_frames, d_n_samples, d_last, n_slots, chunk_samples, frame_len, frame_hop, *cfg, d_state,
-      d_frames, staged, counts, action, info);
+      d_frames, sl.staged(d_scratch), sl.counts(d_scratch), sl.action(d_scratch), sl.info(d_scratch));
   VADX_TRY(after_launch("vadx_stream_serve_step"));
-  const int64_t grid = n_blocks + (d_caches_out ? n_slots : 0);
-  stream_serve_emit_kernel<<<(unsigned)grid, kServeThreads, 0, (cudaStream_t)stream>>>(
-      n_slots, (int)n_blocks, (int)cap, staged, counts, action, info, d_events, d_header, h_events, h_header, d_caches_in,
-      d_caches_out, n_cache_blocks, cache_row);
-  return after_launch("vadx_stream_serve_step");
+  return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, d_caches_in, d_caches_out,
+                    n_cache_blocks, cache_row, stream, "vadx_stream_serve_step");
+}
+
+extern "C" int vadx_silero_serve_load(const int16_t* d_chunk, const int32_t* d_n_samples, int64_t n_slots,
+                                      int windows_per_tick, float* d_x, void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && windows_per_tick >= 1 && windows_per_tick <= kSileroMaxWindowsPerTick,
+               "vadx_silero_serve_load: bad shape");
+  VADX_REQUIRE(d_chunk && d_n_samples && d_x, "vadx_silero_serve_load: null pointer");
+  VADX_REQUIRE(aligned16(d_chunk) && aligned16(d_x), "vadx_silero_serve_load: d_chunk and d_x must be 16-byte aligned");
+  const int chunk_samples = windows_per_tick * kSileroWindow;
+  StageTimer _timer(VADX_STAGE_PREP, (cudaStream_t)stream, "silero_serve_load_kernel", 6.0 * n_slots * chunk_samples);
+  silero_serve_load_kernel<<<(unsigned)ceil_div(n_slots * (chunk_samples / 8), 256), 256, 0, (cudaStream_t)stream>>>(
+      d_chunk, d_n_samples, n_slots, chunk_samples, d_x);
+  return after_launch("vadx_silero_serve_load");
+}
+
+extern "C" int vadx_silero_serve_step(const float* d_probs, int64_t ld_probs, const int32_t* d_n_samples,
+                                      const uint8_t* d_last, int64_t n_slots, int windows_per_tick, double threshold,
+                                      double min_silence_samples, int32_t* d_state, float* d_x, const float* d_state_in,
+                                      float* d_state_out, int32_t* d_windows, int32_t* d_events, int32_t* d_header,
+                                      int32_t* h_events, int32_t* h_header, void* d_scratch, size_t scratch_bytes,
+                                      size_t* scratch_needed, void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && windows_per_tick >= 1 && windows_per_tick <= kSileroMaxWindowsPerTick,
+               "vadx_silero_serve_step: bad shape");
+  const ServeScratch sl(n_slots, (int64_t)windows_per_tick + 1);
+  if (scratch_needed) *scratch_needed = sl.need;
+  if (!d_scratch) return VADX_OK;                   // size query
+  VADX_REQUIRE(scratch_bytes >= sl.need, "vadx_silero_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes, sl.need);
+  VADX_REQUIRE(d_probs && d_n_samples && d_last && d_state && d_windows && d_events && d_header,
+               "vadx_silero_serve_step: null pointer");
+  VADX_REQUIRE(ld_probs >= n_slots, "vadx_silero_serve_step: ld_probs %lld < n_slots %lld", (long long)ld_probs,
+               (long long)n_slots);
+  VADX_REQUIRE(!d_x || aligned16(d_x), "vadx_silero_serve_step: d_x must be 16-byte aligned");
+  VADX_REQUIRE((d_state_in == nullptr) == (d_state_out == nullptr),
+               "vadx_silero_serve_step: state_in and state_out go together");
+  VADX_REQUIRE(!d_state_out || d_state_in != d_state_out, "vadx_silero_serve_step: state_out must not alias state_in");
+  VADX_TRY(check_host_mirror(h_events, h_header, stream, "vadx_silero_serve_step"));
+  StageTimer _timer(VADX_STAGE_POSTPROC, (cudaStream_t)stream, "silero_serve_seg_kernel", 4.0 * n_slots * windows_per_tick);
+  silero_serve_seg_kernel<<<(unsigned)sl.n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
+      d_probs, ld_probs, d_n_samples, d_last, n_slots, windows_per_tick, threshold, min_silence_samples, d_state, d_x,
+      d_windows, sl.staged(d_scratch), sl.counts(d_scratch), sl.action(d_scratch), sl.info(d_scratch));
+  VADX_TRY(after_launch("vadx_silero_serve_step"));
+  return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, d_state_in, d_state_out, 2,
+                    kSileroHidden, stream, "vadx_silero_serve_step");
 }
 
 extern "C" int vadx_postprocess_frames(const float* d_probs, int64_t ld_probs, const int32_t* d_n_frames,

@@ -425,39 +425,14 @@ class StreamServer:
         self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
         self.seg.enqueue(self.out[:, 0, :], self.n_samples, self.last, i, self.caches[i], self.caches[1 - i])
 
-    def _load(self, chunk, n_samples, last):
-        import torch
-        given = [a is not None for a in (chunk, n_samples, last)]
-        if any(given) and not all(given):
-            raise ValueError("StreamServer.step: pass chunk, n_samples and last together, or none of them")
-        if not all(given):
-            return
-        if not (torch.is_tensor(chunk) and chunk.dtype == torch.int16 and tuple(chunk.shape) == (self.S, self.chunk_samples)):
-            raise ValueError(f"StreamServer.step: chunk must be an int16 tensor [{self.S}, {self.chunk_samples}]")
-        PP._check_control(n_samples, last, self.S, "StreamServer.step")
-        for a in (chunk, n_samples, last):
-            if a.is_cuda and a.device != self.device:
-                raise ValueError(f"StreamServer.step: inputs must be on {self.device} or in host memory")
-        if not n_samples.is_cuda:        # host control words: checked here, before anything is copied
-            n = n_samples.numpy()
-            if n.min(initial=0) < 0 or n.max(initial=0) > self.chunk_samples:
-                raise ValueError(f"StreamServer.step: n_samples must be in [0, {self.chunk_samples}]")
-            if not last.is_cuda:
-                short = (n > 0) & (n < self.chunk_samples) & (last.view(torch.uint8).numpy() == 0)
-                if short.any():
-                    raise ValueError(f"StreamServer.step: slots {np.flatnonzero(short)[:8].tolist()} got a short chunk "
-                                     "that is not their stream's last")
-        self.chunk.copy_(chunk, non_blocking=True)
-        self.n_samples.copy_(n_samples, non_blocking=True)
-        self.last.copy_(last.view(torch.uint8), non_blocking=True)
-
     def step(self, chunk=None, n_samples=None, last=None) -> PP.ServeTick:
         """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, chunk_samples], n_samples int32
         [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
         for all three runs the tick on what the static buffers hold.  Returns the tick's handle (PP.ServeTick)."""
         import torch
         with torch.cuda.device(self.device):
-            self._load(chunk, n_samples, last)
+            PP.load_tick_inputs("StreamServer.step", chunk, n_samples, last, self.chunk, self.n_samples, self.last,
+                                self.device)
             if self._runner is not None:
                 self._runner.step(self._k)
             else:

@@ -115,6 +115,9 @@ SIGNATURES = {
     "vadx_stream_serve_zero_tail": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _i32, _vp]),
     "vadx_stream_serve_step": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _i64, _i32, _i32, _i32, C.POINTER(StreamPostCfg), _vp,
                                          _vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
+    "vadx_silero_serve_load": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
+    "vadx_silero_serve_step": (C.c_int, [_vp, _i64, _vp, _vp, _i64, _i32, C.c_double, C.c_double, _vp, _vp, _vp, _vp, _vp,
+                                         _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
     "vadx_create": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), _i32, C.POINTER(_vp)]),
     "vadx_destroy": (None, [_vp]),
     "vadx_set_tensor": (C.c_int, [_vp, C.c_char_p, _vp, _i32, C.POINTER(_i64), _i32]),

@@ -425,6 +425,136 @@ class StreamSlotSegmenter:
         return t
 
 
+class SileroServeTick(ServeTick):
+    """One tick of the Silero slot server (SileroSlotSegmenter).  As ServeTick, but `events` hold (slot, kind, window),
+    `frames` the windows each slot consumed and `probs` is fp32 [n_slots, W] (a view of the forward's [W][n_slots]
+    output).  host_samples / host_seconds convert windows to what the reference VADIterator returns."""
+
+    def _value(self, kind, w):
+        """the reference's float arithmetic (utils_vad.py:566-585): current_sample = (w + 1) * 512 after window w"""
+        o = self._owner
+        if kind == SERVE_START:
+            return max(0, (w + 1) * o.window - o.speech_pad_samples - o.window)
+        if kind == SERVE_END:
+            return (w + 1) * o.window + o.speech_pad_samples - o.window
+        return w * o.window                          # end of stream: the samples consumed
+
+    def _converted(self, conv):
+        try:
+            return [(s, k, conv(self._value(k, int(w)))) for s, k, w in self.host_events()]
+        except ServeTickError as e:
+            e.events = [(s, k, conv(self._value(k, int(w)))) for s, k, w in e.events]
+            raise
+
+    def host_samples(self):
+        """-> [(slot, kind, sample)] as VADIterator(...)(window) returns them; an end-of-stream event gives the samples
+        consumed.  A ServeTickError carries its events in samples."""
+        return self._converted(int)
+
+    def host_seconds(self, time_resolution: int = 1):
+        """-> [(slot, kind, seconds)] as VADIterator(...)(window, return_seconds=True, time_resolution) returns them"""
+        sr = self._owner.sampling_rate
+        return self._converted(lambda v: round(v / sr, time_resolution))
+
+
+class SileroSlotSegmenter:
+    """The VADIterator machine and slot lifecycle of the Silero slot server (vadx_silero_serve_step) for n_slots slots
+    and W windows per tick: iterator state (3 int32 words per slot), scratch, and two sets of event buffers (device and
+    pinned host) used by alternate ticks.  `step` runs it on given probabilities fp32 [W, n_slots], without a model.
+    The defaults are the reference VADIterator constructor's."""
+
+    STATE_WORDS = 3
+    window = 512
+    sampling_rate = 16000
+
+    def __init__(self, threshold: float = 0.5, min_silence_duration_ms: int = 100, speech_pad_ms: int = 30,
+                 n_slots: int = 1, windows_per_tick: int = 5, device=None):
+        import torch
+        self.threshold = float(threshold)
+        self.min_silence_samples = self.sampling_rate * min_silence_duration_ms / 1000
+        self.speech_pad_samples = self.sampling_rate * speech_pad_ms / 1000
+        self.S, self.W = int(n_slots), int(windows_per_tick)
+        dev = device or torch.device("cuda", torch.cuda.current_device())
+        need = C.c_size_t()
+        lib.check(lib.load().vadx_silero_serve_step(None, self.S, None, None, self.S, self.W, self.threshold,
+                                                    self.min_silence_samples, None, None, None, None, None, None, None,
+                                                    None, None, None, 0, C.byref(need), None))
+        self.scratch = torch.empty((need.value,), dtype=torch.uint8, device=dev)
+        self.state = torch.zeros((self.S, self.STATE_WORDS), dtype=torch.int32, device=dev)
+        self.frames = torch.zeros((self.S,), dtype=torch.int32, device=dev)
+        n_max = self.S * (self.W + 1)
+        self.events = [torch.zeros((n_max, 3), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.header = [torch.zeros((2,), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.h_events = [torch.zeros((n_max, 3), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.h_header = [torch.zeros((2,), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.ticks = 0
+
+    def reset(self):
+        """every slot idle (state zeroed); the model input and LSTM state are the caller's"""
+        self.state.zero_()
+
+    def enqueue(self, probs, n_samples, last, parity: int, x=None, state_in=None, state_out=None, stream=None):
+        """Enqueue vadx_silero_serve_step for one tick (no checks beyond pointers: the server checks shapes once)."""
+        lib.check(lib.load().vadx_silero_serve_step(
+            probs.data_ptr(), probs.stride(0), n_samples.data_ptr(), last.data_ptr(), self.S, self.W, self.threshold,
+            self.min_silence_samples, self.state.data_ptr(), lib.ptr(x), lib.ptr(state_in), lib.ptr(state_out),
+            self.frames.data_ptr(), self.events[parity].data_ptr(), self.header[parity].data_ptr(),
+            self.h_events[parity].data_ptr(), self.h_header[parity].data_ptr(), self.scratch.data_ptr(),
+            self.scratch.numel(), None, lib.stream_ptr(stream)))
+
+    def step(self, probs, n_samples, last, stream=None) -> SileroServeTick:
+        """One tick on given CUDA tensors: probs fp32 [W, n_slots] with contiguous rows, n_samples int32 [n_slots]
+        (in [0, W*512]), last bool / uint8 [n_slots]."""
+        import torch
+        if not (torch.is_tensor(probs) and probs.is_cuda and probs.dtype == torch.float32 and probs.dim() == 2
+                and tuple(probs.shape) == (self.W, self.S) and probs.stride(1) == 1):
+            raise ValueError(f"SileroSlotSegmenter.step: probs must be CUDA fp32 [{self.W}, {self.S}] with contiguous rows")
+        _check_control(n_samples, last, self.S, "SileroSlotSegmenter.step", cuda=True)
+        i = self.ticks & 1
+        self.enqueue(probs, n_samples, last.view(torch.uint8), i, stream=stream)
+        return self.finish(i, probs, stream)
+
+    def finish(self, parity, probs, stream=None) -> SileroServeTick:
+        """probs: the tick's [W, n_slots] probabilities"""
+        import torch
+        done = torch.cuda.Event()
+        done.record(stream)
+        t = SileroServeTick(self, self.ticks, parity, probs.t(), self.frames, done)
+        self.ticks += 1
+        return t
+
+
+def load_tick_inputs(who, chunk, n_samples, last, dst_chunk, dst_n_samples, dst_last, device):
+    """A slot server's step(chunk, n_samples, last): checks the arguments against the static buffers and copies them in
+    (non-blocking from pinned host memory).  Host control words are checked here, before anything is copied; control
+    words already on the device are checked by the serve kernel.  None for all three leaves the buffers as they are."""
+    import torch
+    given = [a is not None for a in (chunk, n_samples, last)]
+    if any(given) and not all(given):
+        raise ValueError(f"{who}: pass chunk, n_samples and last together, or none of them")
+    if not all(given):
+        return
+    S, L = dst_chunk.shape
+    if not (torch.is_tensor(chunk) and chunk.dtype == torch.int16 and tuple(chunk.shape) == (S, L)):
+        raise ValueError(f"{who}: chunk must be an int16 tensor [{S}, {L}]")
+    _check_control(n_samples, last, S, who)
+    for a in (chunk, n_samples, last):
+        if a.is_cuda and a.device != device:
+            raise ValueError(f"{who}: inputs must be on {device} or in host memory")
+    if not n_samples.is_cuda:
+        n = n_samples.numpy()
+        if n.min(initial=0) < 0 or n.max(initial=0) > L:
+            raise ValueError(f"{who}: n_samples must be in [0, {L}]")
+        if not last.is_cuda:
+            short = (n > 0) & (n < L) & (last.view(torch.uint8).numpy() == 0)
+            if short.any():
+                raise ValueError(f"{who}: slots {np.flatnonzero(short)[:8].tolist()} got a short chunk "
+                                 "that is not their stream's last")
+    dst_chunk.copy_(chunk, non_blocking=True)
+    dst_n_samples.copy_(n_samples, non_blocking=True)
+    dst_last.copy_(last.view(torch.uint8), non_blocking=True)
+
+
 def _check_control(n_samples, last, S, who, cuda=None):
     """dtype / shape of a tick's control arrays; cuda=True requires them on the device"""
     import torch

@@ -718,6 +718,22 @@ class SileroSession:
         self._final_state = state.clone()
         return probs[:, :, 0].transpose(0, 1).contiguous()
 
+    def forward_windows(self, x, out, state_in, state_out, n_windows: int, row_stride: int, stream=None):
+        """One forward over n_windows consecutive 512-sample windows of S streams, read in place: x CUDA fp32 rows
+        row_stride floats apart, window w of row s at columns [w*512, w*512 + 576) (64 context samples, then the
+        window); out fp32 [n_windows][S][1]; state_in -> state_out fp32 [2][S][128], distinct.  It only enqueues
+        library launches, so a CUDA graph can capture it: the engine scalars it sets are read on the host when the
+        launches are enqueued, and input.n_windows is back at 1 on return."""
+        c = self.cfg
+        if row_stride != self._row_stride:
+            self._e.set_scalar("input.row_stride", float(row_stride))
+            self._row_stride = row_stride
+        self._e.set_scalar("input.n_windows", float(n_windows))
+        try:
+            self._e.forward([x], [out], [state_in, state_out], state_in.shape[1], c.window + c.context, stream)
+        finally:
+            self._e.set_scalar("input.n_windows", 1.0)
+
     def speech_probs(self, audio, stream=None):
         """audio: CUDA fp32 [S, n] (already scaled by 1/32768) -> probs CUDA fp32 [S, ceil(n/512)].
         One graph step per 32 ms window for all S streams; the context is not copied: every window
@@ -733,24 +749,16 @@ class SileroSession:
         probs = torch.empty((n_win, S, 1), dtype=torch.float32, device=audio.device)
         state = torch.zeros((2, S, c.hidden), dtype=torch.float32, device=audio.device)
         stride = padded.shape[1]
-        if stride != self._row_stride:
-            self._e.set_scalar("input.row_stride", float(stride))
-            self._row_stride = stride
-        n_in = c.window + c.context
         nxt = torch.empty_like(state)
         # blocks of windows per call: the state-free part of the graph (STFT, encoder, input half of the gates)
         # runs once over streams x windows rows, only the recurrence runs per window (input.n_windows)
         block = max(1, min(n_win, self.MAX_ROWS_PER_CALL // max(S, 1)))
         t = 0
-        try:
-            while t < n_win:
-                wb = min(block, n_win - t)
-                self._e.set_scalar("input.n_windows", float(wb))
-                self._e.forward([padded[:, t * c.window:]], [probs[t:t + wb]], [state, nxt], S, n_in, stream)
-                state, nxt = nxt, state
-                t += wb
-        finally:
-            self._e.set_scalar("input.n_windows", 1.0)
+        while t < n_win:
+            wb = min(block, n_win - t)
+            self.forward_windows(padded[:, t * c.window:], probs[t:t + wb], state, nxt, wb, stride, stream)
+            state, nxt = nxt, state
+            t += wb
         self._final_state = state
         return probs[:, :, 0].transpose(0, 1).contiguous()
 

@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import audio_io, lib, postprocess as PP, weights as W
-from .firered_vad import VadResult
+from .firered_vad import VadResult, _StreamGraphRunner
 from .session import SileroSession
 
 use_fp16 = False
@@ -179,6 +179,87 @@ class VADIterator:
                 self.temp_end, self.triggered = 0, False
                 return {"end": self._fmt(end, return_seconds, time_resolution)}
         return None
+
+
+class StreamServer:
+    """Live Silero serving with VADIterator events: n_slots independent stream slots advance one tick of
+    windows_per_tick (W) 512-sample windows at a time (W = 5: 160 ms, W = 1: VADIterator's 32 ms cadence).  A stream
+    may start in any free slot on any tick.  Per tick and slot the caller gives the chunk (int16 [W*512]), the number of
+    valid samples n and a `last` flag:
+
+        n > 0, last 0   feed a full chunk (n == W*512)
+        n > 0, last 1   feed the stream's last chunk (may be short), then finalize and free the slot
+        n = 0, last 0   hold: LSTM state, context and iterator state are unchanged
+        n = 0, last 1   finalize and free the slot without new audio
+
+    A slot consumes ceil(n/512) windows; a short last window is zero-padded to 512, as get_speech_timestamps pads it.
+    Samples past n never influence a result.  Each tick is the int16 load, one forward of the session over all slots
+    and W windows, the iterator and the event compaction, replayed as one CUDA graph per LSTM-state parity.  Its result
+    (PP.SileroServeTick) is a compact list of (slot, kind, window) events: kind 0 = start (the window the iterator
+    triggered on), 1 = end (the window the silence began on, VADIterator's temp_end), 2 = the stream ended while
+    triggered (the windows consumed; the reference would leave that segment open).  host_samples() / host_seconds()
+    give exactly what VADIterator returns.  Windows count from the stream's first window, so a stream may run 2^31
+    windows (about 2.2 years).
+
+    The defaults are the reference VADIterator constructor's.  Inputs go through the static buffers `chunk`,
+    `n_samples`, `last`: step() copies the arguments it is given into them (non-blocking from pinned host memory), or a
+    producer writes them and calls step() with no arguments.  The session stays usable between ticks."""
+
+    def __init__(self, session: SileroSession, n_slots: int, windows_per_tick: int = 5, threshold: float = 0.5,
+                 min_silence_duration_ms: int = 100, speech_pad_ms: int = 30, device=None, graph: bool = True):
+        import torch
+        if not isinstance(session, SileroSession):
+            raise ValueError("StreamServer needs a SileroSession")
+        c = session.cfg
+        if (c.window, c.context, c.hidden) != (512, 64, 128):
+            raise ValueError("StreamServer: the session must be the 16 kHz model (512-sample windows, 64-sample "
+                             "context, 128 LSTM units)")
+        S, W = int(n_slots), int(windows_per_tick)
+        if S < 1:
+            raise ValueError(f"StreamServer: n_slots must be at least 1, got {n_slots}")
+        if W < 1:
+            raise ValueError(f"StreamServer: windows_per_tick must be at least 1, got {windows_per_tick}")
+        if S * W > SileroSession.MAX_ROWS_PER_CALL:
+            raise ValueError(f"StreamServer: n_slots * windows_per_tick must be at most {SileroSession.MAX_ROWS_PER_CALL}, "
+                             f"got {S * W}")
+        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        if dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        self.session, self.S, self.W, self.device = session, S, W, dev
+        self.chunk_samples = W * c.window
+        self.row_stride = c.context + self.chunk_samples
+        self.chunk = torch.zeros((S, self.chunk_samples), dtype=torch.int16, device=dev)
+        self.n_samples = torch.zeros((S,), dtype=torch.int32, device=dev)
+        self.last = torch.zeros((S,), dtype=torch.uint8, device=dev)
+        self.x = torch.zeros((S, self.row_stride), dtype=torch.float32, device=dev)     # [context | chunk] per slot
+        self.out = torch.zeros((W, S, 1), dtype=torch.float32, device=dev)
+        self.state = [torch.zeros((2, S, c.hidden), dtype=torch.float32, device=dev) for _ in range(2)]
+        with torch.cuda.device(dev):
+            self.seg = PP.SileroSlotSegmenter(threshold, min_silence_duration_ms, speech_pad_ms, S, W, dev)
+        self._runner = _StreamGraphRunner(self._tick) if graph else None
+        self._k = 0
+
+    def _tick(self, i: int):
+        """the tick body on the static buffers; only libvadx launches"""
+        lib.check(lib.load().vadx_silero_serve_load(self.chunk.data_ptr(), self.n_samples.data_ptr(), self.S, self.W,
+                                                    self.x.data_ptr(), lib.stream_ptr()))
+        self.session.forward_windows(self.x, self.out, self.state[i], self.state[1 - i], self.W, self.row_stride)
+        self.seg.enqueue(self.out[:, :, 0], self.n_samples, self.last, i, self.x, self.state[i], self.state[1 - i])
+
+    def step(self, chunk=None, n_samples=None, last=None) -> PP.SileroServeTick:
+        """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, W*512], n_samples int32
+        [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
+        for all three runs the tick on what the static buffers hold.  Returns the tick's handle (PP.SileroServeTick)."""
+        import torch
+        with torch.cuda.device(self.device):
+            PP.load_tick_inputs("StreamServer.step", chunk, n_samples, last, self.chunk, self.n_samples, self.last,
+                                self.device)
+            if self._runner is not None:
+                self._runner.step(self._k)
+            else:
+                self._tick(self._k & 1)
+            self._k += 1
+            return self.seg.finish((self._k - 1) & 1, self.out[:, :, 0])
 
 
 def run_vad(audio, model: SileroSession, save_timestamps_second: str | None = None,
