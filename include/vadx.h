@@ -540,6 +540,57 @@ int vadx_silero_serve_step(const float* d_probs, int64_t ld_probs, const int32_t
                            int32_t* h_header, void* d_scratch, size_t scratch_bytes, size_t* scratch_needed,
                            void* stream);
 
+/* FSMN slot server: n_slots independent FSMN-VAD streams, one reference window of chunk_len samples per tick.  Windows
+ * follow the reference (FSMN/Inference_FSMN_VAD_ONNX.py:79-99): window k of a stream covers samples
+ * [k*stride, k*stride + chunk_len), stride = chunk_len - (look_backward + 1) * 160 (both multiples of 8).  Per tick and slot
+ * s the caller gives d_n_samples[s] and d_last[s] with the four actions of the slot servers above (feed a full chunk, feed
+ * a possibly short last chunk and finalize, hold, finalize without audio) and the same VADX_SERVE_ERR_* rules, where a
+ * full chunk is min(stride, chunk_len - received) until the slot holds chunk_len samples and stride from then on
+ * (VADX_SERVE_ERR_RANGE: n outside [0, full]).  The tick that completes a slot's first chunk_len samples runs its first
+ * window, every later fed tick one more; a stream that ends earlier gets one window, zero-padded, as does a short last
+ * chunk.  Finalize without audio flushes the look-ahead of the latest window (its last look_backward score flags are in
+ * the state).  The state is d_state [n_slots][vadx_fsmn_serve_state_words(look_backward)] int32, all zero = a fresh slot.
+ *
+ * vadx_fsmn_serve_load runs BEFORE the forward: it writes the int16 chunk d_chunk [n_slots][stride] into the slot's row of
+ * the window buffer d_window [n_slots][chunk_len] (the forward's input; both 16-byte aligned: the kernel moves 16-byte
+ * vectors, a misaligned pointer is rejected): before the first window at the samples received so far, afterwards after
+ * shifting the row left by stride; zeros from n on; a held slot's row is not touched.  It also writes each slot's
+ * background level (the gate's noise_average_dB input) to d_noise_avg [n_slots].
+ *
+ * vadx_fsmn_serve_step runs AFTER the forward on its score flags d_score [n_slots][ld_score] (n_frames columns, 0 / 1) and
+ * noisy_dB [n_slots]:
+ *   - runs the look-ahead hysteresis (lookahead_hysteresis, mode 0) over each window's flags, writes the decisions of the
+ *     tick to d_decisions [n_slots], and updates the level as the reference does (if noisy_dB > 0: level =
+ *     0.5 * ((level + noisy_dB) + snr_threshold), fp32);
+ *   - turns the decisions into the reference's final timestamps, process_timestamps(runs_to_timestamps(...), fusion,
+ *     min_duration) (:102-141), in Python doubles, emitting each event as soon as it is certain: VADX_SERVE_START a (time
+ *     a*d), VADX_SERVE_END b (the run closed by silence decision b, time b*d + d), VADX_SERVE_END_OF_STREAM n (the
+ *     segment was open at finalize after n decisions, time n*d), d = frame_duration.  Decisions count from the stream's
+ *     first window as int32, so a stream may run 2^31 decisions (about 248 days at 100 per second);
+ *   - applies the slot lifecycle to the caches [n_cache_blocks][n_slots][cache_row] fp32 as vadx_stream_serve_step does
+ *     (a slot that ran no window holds them) and writes d_events [n][3] (slot, kind, decision) / d_header and the optional
+ *     pinned host mirror.  d_events must hold n_slots * (2 * n_frames + 2) triples.
+ * d_scratch = NULL: only writes the scratch size to *scratch_needed and returns. */
+typedef struct {
+  double speaking_score;
+  double silence_score;
+  double frame_duration;        /* seconds per decision: 160 / 16000 */
+  double fusion_threshold;      /* seconds */
+  double min_speech_duration;   /* seconds */
+  float snr_threshold;          /* snr_threshold_dB * 0.1 */
+  float noise_init;             /* the initial background level */
+} vadx_fsmn_serve_cfg;
+int vadx_fsmn_serve_state_words(int look_backward);
+int vadx_fsmn_serve_load(const int16_t* d_chunk, const int32_t* d_n_samples, const uint8_t* d_last,
+                         const int32_t* d_state, int64_t n_slots, int chunk_len, int stride, int look_backward,
+                         float noise_init, int16_t* d_window, float* d_noise_avg, void* stream);
+int vadx_fsmn_serve_step(const uint8_t* d_score, int64_t ld_score, const float* d_noisy_dB, int n_frames,
+                         const int32_t* d_n_samples, const uint8_t* d_last, int64_t n_slots, int chunk_len, int stride,
+                         int look_backward, const vadx_fsmn_serve_cfg* cfg, int32_t* d_state, const float* d_caches_in,
+                         float* d_caches_out, int n_cache_blocks, int64_t cache_row, int32_t* d_decisions,
+                         int32_t* d_events, int32_t* d_header, int32_t* h_events, int32_t* h_header, void* d_scratch,
+                         size_t scratch_bytes, size_t* scratch_needed, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Model-level API: the replacement for InferenceSession(...).run(...)
  * ------------------------------------------------------------------------------------------ */

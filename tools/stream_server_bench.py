@@ -11,6 +11,10 @@ With --family silero, for each slot count and windows per tick (--windows, defau
 measured, except: realtime streams = n_slots * W * 32 ms / device ms per tick, and instead of the lock-step chunk the
 bare forward of the same shape (SileroSession's engine over [n_slots][64 + W*512] rows, W windows, one CUDA graph),
 alternating with the server in this process.
+With --family fsmn (fsmn_vad.StreamServer), for each slot count and window length (--chunk-lens, default 16000 and
+7520, look-backward 0.3 s), the same rows with ticks of one reference window (stride = L - 31 * 160 samples), plus the
+bare forward of the same [n_slots][L] shape as one CUDA graph and the lock-step run_streams(graph=True) time per window,
+both alternating with the server in this process; realtime streams = n_slots * stride / 16000 / tick.
 Prints one JSON line (card name and power limit read in the same run); --out also writes it to a file, --trace writes
 the torch.profiler launch list of a few server ticks.
 
@@ -18,6 +22,8 @@ the torch.profiler launch list of a few server ticks.
       --trace profiles/r03_launches_stream_server.txt
   python tools/stream_server_bench.py --family silero --slots 4096,16384 --out profiles/r04_silero_server.json \
       --trace profiles/r04_launches_silero_server.txt
+  python tools/stream_server_bench.py --family fsmn --slots 4096,16384 --out profiles/r05_fsmn_server.json \
+      --trace profiles/r05_launches_fsmn_server.txt
 """
 from __future__ import annotations
 
@@ -208,9 +214,136 @@ def main_silero(a, info):
             "ticks": a.ticks, "rounds": a.rounds, "results": rows}
 
 
+class FsmnTraffic:
+    """Seeded control words for the FSMN server, simulated tick by tick because a full chunk depends on the samples a
+    slot holds (server.full_chunk): every slot feeds full chunks; under churn about `churn` of the slots close per tick
+    (a short last chunk, possibly empty) and a new stream starts there on the next one, and `hold` of the others hold.
+    tick() ignores its argument and hands out the next tick, so the control words stay consistent with the device."""
+
+    def __init__(self, S, L, stride, churn, hold, seed, n_ticks, n_pool=2):
+        import torch
+        rs = np.random.RandomState(seed)
+        audio = rs.randint(-3000, 3000, size=(S, stride)).astype(np.int16)
+        t = np.arange(stride)[None, :]
+        audio += (8000 * np.sin(t / rs.uniform(3, 30, size=(S, 1))) * (rs.rand(S, 1) < 0.5)).astype(np.int16)
+        self.chunks = [torch.from_numpy(np.roll(audio, 97 * i, axis=0)).pin_memory() for i in range(n_pool)]
+        self.ctrl = []
+        rec = np.zeros(S, np.int64)
+        for _ in range(n_ticks):
+            full = np.where(rec < L, np.minimum(stride, L - rec), stride)
+            n = full.astype(np.int32)
+            last = np.zeros(S, np.uint8)
+            if churn > 0:
+                close = rs.rand(S) < churn
+                n[close] = (rs.rand(S) * (full + 1)).astype(np.int32)[close]
+                last[close] = 1
+                n[(rs.rand(S) < hold) & ~close] = 0
+            rec += n
+            rec[last != 0] = 0
+            self.ctrl.append((torch.from_numpy(n).pin_memory(), torch.from_numpy(last).pin_memory()))
+        self.k = 0
+
+    def tick(self, _k):
+        n, last = self.ctrl[self.k]
+        self.k += 1
+        return self.chunks[self.k % len(self.chunks)], n, last
+
+
+class FsmnForward:
+    """the bare forward of an FSMN server tick: FsmnSession.run_batch over [S][L] rows into static outputs, caches
+    a -> b, captured as one CUDA graph on buffers of its own"""
+
+    def __init__(self, session, S):
+        import torch
+        L, T = session.chunk_len, session.T
+        self.session = session
+        g = torch.Generator(device="cuda").manual_seed(S + L)
+        self.x = torch.randint(-8000, 8000, (S, L), generator=g, device="cuda", dtype=torch.int16)
+        self.noise = torch.full((S,), 4.0, device="cuda")
+        self.score = torch.empty((S, T), dtype=torch.uint8, device="cuda")
+        self.noisy = torch.empty((S,), dtype=torch.float32, device="cuda")
+        self.caches = [torch.zeros((session.cfg.fsmn_layers, S) + session.cache_shape, device="cuda") for _ in range(2)]
+        self._run()
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self._run()
+
+    def _run(self):
+        self.session.run_batch(self.x, self.caches[0].unbind(0), self.noise, out=(self.score, self.noisy, None, None),
+                               caches_out=self.caches[1].unbind(0))
+
+    time = SileroForward.time
+
+
+def bench_fsmn_lockstep(session, aligned, stride, lb_s, reps):
+    """run_streams(graph=True) over recordings of a few windows: ms per window"""
+    import torch
+    from vadx import fsmn_vad as FSV
+    n_windows = (aligned.shape[1] - session.chunk_len) // stride + 1
+    FSV.run_streams(session, aligned, stride, lb_s, graph=True)
+    torch.cuda.synchronize()
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    for _ in range(reps):
+        FSV.run_streams(session, aligned, stride, lb_s, graph=True)
+    b.record()
+    torch.cuda.synchronize()
+    return a.elapsed_time(b) / (reps * n_windows)
+
+
+def main_fsmn(a, info):
+    import torch
+    import vadx
+    from vadx import fsmn_vad as FSV, weights as W
+    cfg = W.FsmnConfig()
+    wts = W.fsmn_random_init(cfg, 0)
+    lb_s = FSV.LOOK_BACKWARD
+    rows = []
+    for L in [int(v) for v in a.chunk_lens.split(",")]:
+        sess = vadx.FsmnSession(wts, cfg, chunk_len=L)
+        stride = L - (FSV.look_backward_frames(lb_s) + 1) * FSV.OUTPUT_FRAME_LENGTH
+        for S in [int(v) for v in a.slots.split(",")]:
+            fwd = FsmnForward(sess, S)
+            lock = torch.from_numpy(np.random.RandomState(S).randint(-8000, 8000, size=(S, L + 3 * stride))
+                                    .astype(np.int16)).cuda()
+            for mode, churn, hold in (("full", 0.0, 0.0), ("churn", 0.01, 0.10)):
+                n_ticks = a.rounds * (a.warmup + 2 * a.ticks) + (5 if a.trace and not rows else 0)
+                traffic = FsmnTraffic(S, L, stride, churn, hold, S + L + len(mode), n_ticks)
+                server = FSV.StreamServer(sess, S, look_backward_s=lb_s)
+                res = {"dev": [], "host": [], "events": [], "d2h": [], "fwd": [], "lock": []}
+                for _ in range(a.rounds):
+                    d, h, e, b = bench_server(server, traffic, a.ticks, a.warmup)
+                    res["dev"].append(d), res["host"].append(h), res["events"].append(e), res["d2h"].append(b)
+                    res["fwd"].append(fwd.time(a.ticks))
+                    res["lock"].append(bench_fsmn_lockstep(sess, lock, stride, lb_s, 2))
+                dev = float(np.median(res["dev"]))
+                bare = float(np.median(res["fwd"]))
+                row = {"chunk_len": L, "stride": stride, "n_slots": S, "traffic": mode, "device_ms_per_tick": round(dev, 4),
+                       "device_ms_per_tick_rounds": [round(v, 4) for v in res["dev"]],
+                       "host_ms_per_tick": round(float(np.median(res["host"])), 4),
+                       "events_per_tick": round(float(np.mean(res["events"])), 2),
+                       "d2h_bytes_per_tick": round(float(np.mean(res["d2h"])), 1),
+                       "realtime_streams": int(S * stride / 16000 / (dev / 1e3)),
+                       "forward_ms": round(bare, 4), "forward_ms_rounds": [round(v, 4) for v in res["fwd"]],
+                       "tick_over_forward": round(dev / bare, 3),
+                       "lockstep_ms_per_window": round(float(np.median(res["lock"])), 4)}
+                rows.append(row)
+                print(json.dumps(row), file=sys.stderr)
+                if a.trace and len(rows) == 1:
+                    write_trace(a.trace, server, traffic, f"fsmn StreamServer, L = {L}, {S} slots, 5 ticks, {info}")
+                del server, traffic
+                torch.cuda.empty_cache()
+            del fwd, lock
+            torch.cuda.empty_cache()
+    return {"what": "fsmn StreamServer tick vs the bare forward of the same shape and the lock-step window", "card": info,
+            "look_backward_s": lb_s, "ticks": a.ticks, "rounds": a.rounds, "results": rows}
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
-    ap.add_argument("--family", choices=("firered", "silero"), default="firered")
+    ap.add_argument("--family", choices=("firered", "silero", "fsmn"), default="firered")
+    ap.add_argument("--chunk-lens", default="16000,7520", help="fsmn: window lengths to measure")
     ap.add_argument("--windows", default="5,1", help="silero: windows per tick to measure")
     ap.add_argument("--slots", default="4096,16384")
     ap.add_argument("--ticks", type=int, default=200)
@@ -226,8 +359,8 @@ def main(argv=None):
         raise SystemExit("stream_server_bench: needs a CUDA device")
     torch.cuda.set_device(0)
     info = card()
-    if a.family == "silero":
-        out = main_silero(a, info)
+    if a.family in ("silero", "fsmn"):
+        out = main_silero(a, info) if a.family == "silero" else main_fsmn(a, info)
         line = json.dumps(out)
         print(line)
         if a.out:

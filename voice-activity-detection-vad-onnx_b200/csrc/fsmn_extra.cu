@@ -1,7 +1,7 @@
 // fsmn_extra.cu -- the FunASR-FSMN specific stages: LFR + CMVN (a4), softmax class-0 head (a8),
 // frame-energy gate (a9), look-ahead hysteresis with on-device stream state (a13) and run-length
 // extraction (a14).
-#include "common.cuh"
+#include "hysteresis.cuh"
 
 namespace vadx {
 
@@ -124,51 +124,8 @@ __global__ void __launch_bounds__(128) fsmn_gate_kernel(const float* __restrict_
   if (threadIdx.x == 0) noisy_dB[s] = s_sum[0] / (float)s_cnt[0];  // 0/0 = NaN like torch.mean of nothing
 }
 
-// a13: look-ahead hysteresis, one stream per lane, state carried on the device between chunks.
-// mode 0 (FSMN): `in` is uint8 flags; a frame votes "speech" when flag != 0 and "silence" when
-//                flag != 1 (FSMN/Inference_FSMN_VAD_ONNX.py:188-215).
-// mode 1 (DFSMN): `in` is fp32 probabilities; a frame votes with p >= SPEAKING_SCORE / p <= SILENCE_SCORE, the same two
-//                scores the vote RATIO is then tested against (DFSMN/near_and_far_end_audio/Inference_DFSMN_VAD_ONNX.py:
-//                231-273).  The per-frame test compares a numpy float32 with a Python float: under NEP 50 (numpy >= 2) the
-//                Python float is the weak operand, so the comparison happens in float32; the ratio test is Python floats.
-// one chunk of the machine for one stream: appends T - look_backward decisions (all T when is_final) to out[n...]
-__device__ __forceinline__ void hysteresis_chunk(const uint8_t* fl, const float* pr, int mode, int T, int look_backward,
-                                                 double speaking_score, double silence_score, int is_final, bool& silence, int& n,
-                                                 uint8_t* out, int64_t ld_saved) {
-  const float speak_f = (float)speaking_score, sil_f = (float)silence_score;
-  auto speech_vote = [&](int i) { return mode == 0 ? fl[i] != 0 : pr[i] >= speak_f; };
-  auto silence_vote = [&](int i) { return mode == 0 ? fl[i] != 1 : pr[i] <= sil_f; };
-  const int lb = look_backward != 0 ? look_backward : 1;
-  const double inv_d = 1.0 / (double)lb;
-  const int range = T - look_backward;
-  for (int i = 0; i < range; ++i) {
-    if (silence) {
-      if (speech_vote(i)) {
-        int votes = 1;
-        for (int j = 1; j < lb; ++j) votes += speech_vote(i + j) ? 1 : 0;
-        silence = !((double)votes * inv_d >= speaking_score);
-      }
-    } else {
-      if (silence_vote(i)) {
-        int votes = 1;
-        for (int j = 1; j < lb; ++j) votes += silence_vote(i + j) ? 1 : 0;
-        silence = !((double)votes * inv_d <= silence_score);
-      } else {
-        silence = false;
-      }
-    }
-    if (n < ld_saved) out[n] = silence ? 1 : 0;
-    ++n;
-  }
-  if (is_final) {
-    for (int i = range; i < T; ++i) {
-      silence = silence ? !speech_vote(i) : silence_vote(i);
-      if (n < ld_saved) out[n] = silence ? 1 : 0;
-      ++n;
-    }
-  }
-}
-
+// a13: look-ahead hysteresis (hysteresis.cuh), one stream per lane, state carried on the device between chunks; the
+// decisions are appended to saved[n...].
 __global__ void __launch_bounds__(128) lookahead_hysteresis_kernel(const void* __restrict__ in, int mode, int64_t ld_in,
                                                                    int64_t n_streams, int T, int look_backward,
                                                                    double speaking_score, double silence_score,
@@ -181,8 +138,12 @@ __global__ void __launch_bounds__(128) lookahead_hysteresis_kernel(const void* _
   if (s >= n_streams) return;
   bool silence = silence_state[s] != 0;
   int n = n_saved[s];
+  uint8_t* out = saved + s * ld_saved;
   hysteresis_chunk(static_cast<const uint8_t*>(in) + s * ld_in, static_cast<const float*>(in) + s * ld_in, mode, T, look_backward,
-                   speaking_score, silence_score, is_final, silence, n, saved + s * ld_saved, ld_saved);
+                   speaking_score, silence_score, is_final, silence, [&](bool sil) {
+                     if (n < ld_saved) out[n] = sil ? 1 : 0;
+                     ++n;
+                   });
   silence_state[s] = silence ? 1 : 0;
   n_saved[s] = n;
   if (noise_avg && noisy_dB) {
@@ -238,8 +199,11 @@ __global__ void __launch_bounds__(128) fsmn_gate_hysteresis_windows_kernel(
       const float nd = s_sum[0] / (float)s_cnt[0];      // 0/0 = NaN like torch.mean of nothing
       if (noisy_out) noisy_out[s * W + w] = nd;
       if (noise_in_out) noise_in_out[s * W + w] = noise;
-      hysteresis_chunk(s_flags, nullptr, 0, T, look_backward, speaking_score, silence_score, w == W - 1, silence, n,
-                       saved + s * ld_saved, ld_saved);
+      uint8_t* out = saved + s * ld_saved;
+      hysteresis_chunk(s_flags, nullptr, 0, T, look_backward, speaking_score, silence_score, w == W - 1, silence, [&](bool sil) {
+        if (n < ld_saved) out[n] = sil ? 1 : 0;
+        ++n;
+      });
       if (nd > 0.0f) s_noise = 0.5f * ((noise + nd) + snr);
     }
     __syncthreads();

@@ -5,7 +5,7 @@
 // decisions at ties.  Every arithmetic step below reproduces one numpy float32 operation of
 // FireRedVAD/Inference_FireRed_ONNX.py:181-304 (MarbleNet copy:
 // NVIDIA_*/Inference_NVIDIA_MarbleNet_VAD_ONNX.py:160-353).
-#include "common.cuh"
+#include "hysteresis.cuh"
 
 namespace vadx {
 
@@ -915,6 +915,207 @@ __global__ void __launch_bounds__(kServeThreads) silero_serve_seg_kernel(
   }
 }
 
+
+// ---- FSMN slot server (vadx_fsmn_serve_load, vadx_fsmn_serve_step) ----
+// State words per slot: 0 samples received before the first window (chunk_len from the first window on), 1 the machine
+// is out of silence (0 = silence, the reference's initial state), 2 decisions so far, 3 background level bits XOR the
+// initial level's bits (0 = the initial level), 4 first decision of the open run + 1 (0 = none), 5 segment state
+// (kFsmnSeg*), 6 closing decision of the pending segment's last run, 7 spare (0), 8.. the last look_backward score
+// flags of the latest window, one bit each.  All zero is a fresh slot.
+constexpr int kFsmnServeHeader = 8;
+constexpr int kFsmnMaxChunk = 1 << 24;
+enum : int { kFsmnSegNone = 0, kFsmnSegOpen = 1, kFsmnSegPending = 2 };
+enum : int { kFsmnHold = 0, kFsmnFill = 1, kFsmnWindow = 2, kFsmnFlush = 3 };
+
+__host__ __device__ __forceinline__ int fsmn_serve_words(int look_backward) { return kFsmnServeHeader + (look_backward + 31) / 32; }
+
+// What a slot does this tick, from its control words and the samples it holds.  Until a slot has `chunk_len` samples a
+// full chunk is min(stride, chunk_len - received), so no stream is carried past its first window; from then on it is
+// `stride`.  kFsmnFill: samples only; kFsmnWindow: one window (the first one once chunk_len samples are in, or a
+// zero-padded one at a short stream's end); kFsmnFlush: finalize without new audio after the last window (or a stream
+// that never got a sample).  Load and step decide alike.
+__device__ __forceinline__ int fsmn_serve_plan(int n, bool fin, int received, int chunk_len, int stride, int& err) {
+  const int full = received < chunk_len ? min(stride, chunk_len - received) : stride;
+  err = (n < 0 || n > full) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < full && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+  if (err || (n == 0 && !fin)) return kFsmnHold;
+  if (received < chunk_len) {
+    if (received + n < chunk_len && !fin) return kFsmnFill;
+    return received + n > 0 ? kFsmnWindow : kFsmnFlush;   // a stream that ends before its first window gets a padded one
+  }
+  return n > 0 ? kFsmnWindow : kFsmnFlush;
+}
+
+__device__ __forceinline__ int4 fsmn_chunk_vec(const int16_t* src, int k, int n) {
+  if (k + 8 <= n) return __ldg(reinterpret_cast<const int4*>(src + k));
+  int4 v = make_int4(0, 0, 0, 0);
+  int16_t* e = reinterpret_cast<int16_t*>(&v);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) e[j] = k + j < n ? src[k + j] : (int16_t)0;
+  return v;
+}
+
+// CTA per slot: the tick's samples into the slot's window row [chunk_len] (the forward's input), 8 samples per thread
+// and vector, zeros from n on.  Before the first window the chunk lands at `received` and zeros fill the rest of the row.
+// From then on the row moves left by `stride` and the chunk fills its last `stride` samples: the shift overlaps itself
+// whenever chunk_len - stride > stride, so it runs in strips of 8 * blockDim samples, all reads of a strip before a
+// barrier and all its writes after it (a strip's writes lie below every later strip's reads).  A held slot's row is not
+// touched.  Thread 0 also writes the slot's background level, the forward's gate input.
+__global__ void __launch_bounds__(256) fsmn_serve_load_kernel(const int16_t* __restrict__ chunk,
+                                                             const int32_t* __restrict__ n_samples,
+                                                             const uint8_t* __restrict__ last,
+                                                             const int32_t* __restrict__ state, int words, int chunk_len,
+                                                             int stride, float noise_init, int16_t* __restrict__ window,
+                                                             float* __restrict__ noise_avg) {
+  const int64_t s = blockIdx.x;
+  const int32_t* st = state + s * words;
+  const int received = st[0], n = n_samples[s];
+  if (threadIdx.x == 0) noise_avg[s] = __int_as_float(st[3] ^ __float_as_int(noise_init));
+  int err;
+  const int plan = fsmn_serve_plan(n, last[s] != 0, received, chunk_len, stride, err);
+  if (plan == kFsmnHold || plan == kFsmnFlush) return;
+  int16_t* row = window + s * chunk_len;
+  const int16_t* src = chunk + s * stride;
+  if (received < chunk_len) {
+    for (int k = received + 8 * threadIdx.x; k < chunk_len; k += 8 * blockDim.x)
+      *reinterpret_cast<int4*>(row + k) = fsmn_chunk_vec(src, k - received, n);
+    return;
+  }
+  const int keep = chunk_len - stride;
+  for (int base = 0; base < chunk_len; base += 8 * blockDim.x) {
+    const int k = base + 8 * threadIdx.x;
+    int4 v = make_int4(0, 0, 0, 0);
+    if (k < keep) v = *reinterpret_cast<const int4*>(row + k + stride);
+    else if (k < chunk_len) v = fsmn_chunk_vec(src, k - keep, n);
+    __syncthreads();
+    if (k < chunk_len) *reinterpret_cast<int4*>(row + k) = v;
+  }
+}
+
+// The reference's final timestamps, online.  Offline they are process_timestamps(runs_to_timestamps(saved, d), fusion,
+// min_dur) (FSMN/Inference_FSMN_VAD_ONNX.py:102-141): a run of non-silence decisions a..b-1 is (a*d, b*d + d), one still
+// open at the end (a*d, n*d); runs shorter than min_dur go, then neighbours with start - previous end <= fusion fuse (the
+// second fusion pass never fuses again).  Here every double is formed as Python forms it (no contraction into FMAs), and
+// an event leaves as soon as it is certain:
+//   - an open run is kept once m*d - a*d >= min_dur (m decisions so far): every end it can still get is >= m*d;
+//   - a pending segment's end is final once the earliest start a later kept run can have (the open run's, else m) lies
+//     more than `fusion` after it.
+struct FsmnTimestamps {
+  int m, run_a, seg, seg_b;      // run_a < 0: no open run; seg_b: the closing decision of the pending segment's last run
+  double d, fusion, min_dur;
+  int2* ev;
+  int count;
+
+  __device__ __forceinline__ double at(int i) const { return __dmul_rn((double)i, d); }
+  __device__ __forceinline__ double end_at(int b) const { return __dadd_rn(at(b), d); }
+  __device__ __forceinline__ void push(int kind, int v) { ev[count++] = make_int2(kind, v); }
+  // the run starting at a is kept: it fuses into the pending segment or ends it and opens the next
+  __device__ __forceinline__ void kept(int a) {
+    if (seg == kFsmnSegPending) {
+      if (__dsub_rn(at(a), end_at(seg_b)) <= fusion) { seg = kFsmnSegOpen; return; }
+      push(VADX_SERVE_END, seg_b);
+    }
+    push(VADX_SERVE_START, a);
+    seg = kFsmnSegOpen;
+  }
+  __device__ __forceinline__ void decide(bool silence) {
+    const int i = m++;
+    if (!silence) {
+      if (run_a < 0) run_a = i;
+      if (seg != kFsmnSegOpen && __dsub_rn(at(m), at(run_a)) >= min_dur) kept(run_a);
+    } else if (run_a >= 0) {
+      if (seg == kFsmnSegOpen || __dsub_rn(end_at(i), at(run_a)) >= min_dur) {
+        if (seg != kFsmnSegOpen) kept(run_a);
+        seg = kFsmnSegPending;
+        seg_b = i;
+      }
+      run_a = -1;
+    }
+    if (seg == kFsmnSegPending && __dsub_rn(at(run_a >= 0 ? run_a : m), end_at(seg_b)) > fusion) {
+      push(VADX_SERVE_END, seg_b);
+      seg = kFsmnSegNone;
+    }
+  }
+  __device__ __forceinline__ void finish() {
+    if (run_a >= 0 && (seg == kFsmnSegOpen || __dsub_rn(at(m), at(run_a)) >= min_dur)) {
+      if (seg != kFsmnSegOpen) kept(run_a);
+      push(VADX_SERVE_END_OF_STREAM, m);
+    } else if (seg == kFsmnSegPending) {
+      push(VADX_SERVE_END, seg_b);
+    }
+  }
+};
+
+// Thread per slot, after the forward: validate the control words (fsmn_serve_plan), run the look-ahead hysteresis over
+// the slot's score row [T] feeding every decision to the timestamp machine, update the background level, and stage at
+// most 2T + 2 events (kind, decision) in `staged` [S][2T+2]: a tick hands D <= T decisions to the machine, at most one
+// START per decision (a run that is only kept at finalize has its last decision in this tick, which started nothing,
+// unless D = 0), and every END / END_OF_STREAM closes a segment started in this tick or the one open before it; so
+// events <= 2D + 1 <= 2T + 1 for D >= 1, and 3 <= 2T + 2 for D = 0.
+__global__ void __launch_bounds__(kServeThreads) fsmn_serve_seg_kernel(
+    const uint8_t* __restrict__ score, int64_t ld_score, const float* __restrict__ noisy_dB, int T,
+    const int32_t* __restrict__ n_samples, const uint8_t* __restrict__ last, int64_t n_slots, int chunk_len, int stride,
+    int look_backward, const vadx_fsmn_serve_cfg cfg, int32_t* __restrict__ state, int32_t* __restrict__ decisions_out,
+    int32_t* __restrict__ staged, int32_t* __restrict__ counts, int8_t* __restrict__ action, int32_t* __restrict__ block_info) {
+  const int64_t s = (int64_t)blockIdx.x * kServeThreads + threadIdx.x;
+  int count = 0, err = 0;
+  if (s < n_slots) {
+    const int words = fsmn_serve_words(look_backward);
+    int32_t* st = state + s * words;
+    const int n = n_samples[s];
+    const bool fin = last[s] != 0;
+    const int plan = fsmn_serve_plan(n, fin, st[0], chunk_len, stride, err);
+    int8_t act = kServeHold;                         // no window ran: the caches stay as they were
+    int D = 0;
+    if (plan == kFsmnFill) {
+      st[0] += n;
+    } else if (plan != kFsmnHold) {
+      const int32_t init_bits = __float_as_int(cfg.noise_init);
+      bool silence = st[1] == 0;
+      FsmnTimestamps ts{st[2], st[4] - 1, st[5], st[6], cfg.frame_duration, cfg.fusion_threshold, cfg.min_speech_duration,
+                        reinterpret_cast<int2*>(staged) + s * (2 * (int64_t)T + 2), 0};
+      const int m0 = ts.m;
+      if (plan == kFsmnWindow) {
+        const uint8_t* fl = score + s * ld_score;
+        hysteresis_chunk(fl, nullptr, 0, T, look_backward, cfg.speaking_score, cfg.silence_score, fin, silence,
+                         [&](bool sil) { ts.decide(sil); });
+        const float nd = noisy_dB[s];
+        if (nd > 0.0f) {
+          const float level = __int_as_float(st[3] ^ init_bits);
+          st[3] = __float_as_int(0.5f * ((level + nd) + cfg.snr_threshold)) ^ init_bits;
+        }
+        for (int w = 0; w < (look_backward + 31) / 32; ++w) {
+          uint32_t bits = 0;
+          for (int j = 0; j < 32 && 32 * w + j < look_backward; ++j)
+            bits |= (fl[T - look_backward + 32 * w + j] != 0 ? 1u : 0u) << j;
+          st[kFsmnServeHeader + w] = (int32_t)bits;
+        }
+        st[0] = chunk_len;
+      } else if (st[0] == chunk_len) {               // finalize without audio: the flush of the latest window
+        for (int j = 0; j < look_backward; ++j) {
+          const bool speech = ((uint32_t)st[kFsmnServeHeader + j / 32] >> (j & 31)) & 1u;
+          silence = hysteresis_tail(silence, speech, !speech);
+          ts.decide(silence);
+        }
+      }
+      D = ts.m - m0;
+      if (fin) {
+        ts.finish();
+        for (int i = 0; i < words; ++i) st[i] = 0;   // the next stream in this slot starts fresh
+        act = kServeFinalize;
+      } else {
+        st[1] = silence ? 0 : 1;
+        st[2] = ts.m; st[4] = ts.run_a + 1; st[5] = ts.seg; st[6] = ts.seg_b;
+        act = kServeAdvance;
+      }
+      count = ts.count;
+    }
+    action[s] = act;
+    decisions_out[s] = D;
+    counts[s] = count;
+  }
+  serve_block_totals(count, err, block_info);
+}
+
 }  // namespace vadx
 
 using namespace vadx;
@@ -1074,6 +1275,53 @@ extern "C" int vadx_silero_serve_step(const float* d_probs, int64_t ld_probs, co
   VADX_TRY(after_launch("vadx_silero_serve_step"));
   return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, d_state_in, d_state_out, 2,
                     kSileroHidden, stream, "vadx_silero_serve_step");
+}
+
+extern "C" int vadx_fsmn_serve_state_words(int look_backward) { return fsmn_serve_words(look_backward < 0 ? 0 : look_backward); }
+
+extern "C" int vadx_fsmn_serve_load(const int16_t* d_chunk, const int32_t* d_n_samples, const uint8_t* d_last,
+                                    const int32_t* d_state, int64_t n_slots, int chunk_len, int stride, int look_backward,
+                                    float noise_init, int16_t* d_window, float* d_noise_avg, void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && stride >= 1 && stride < chunk_len && chunk_len <= kFsmnMaxChunk && chunk_len % 8 == 0 &&
+                   stride % 8 == 0 && look_backward >= 0,
+               "vadx_fsmn_serve_load: bad shape");
+  VADX_REQUIRE(d_chunk && d_n_samples && d_last && d_state && d_window && d_noise_avg, "vadx_fsmn_serve_load: null pointer");
+  VADX_REQUIRE(aligned16(d_chunk) && aligned16(d_window), "vadx_fsmn_serve_load: d_chunk and d_window must be 16-byte aligned");
+  StageTimer _timer(VADX_STAGE_PREP, (cudaStream_t)stream, "fsmn_serve_load_kernel", 2.0 * n_slots * (stride + 2.0 * chunk_len));
+  fsmn_serve_load_kernel<<<(unsigned)n_slots, 256, 0, (cudaStream_t)stream>>>(
+      d_chunk, d_n_samples, d_last, d_state, fsmn_serve_words(look_backward), chunk_len, stride, noise_init,
+      d_window, d_noise_avg);
+  return after_launch("vadx_fsmn_serve_load");
+}
+
+extern "C" int vadx_fsmn_serve_step(const uint8_t* d_score, int64_t ld_score, const float* d_noisy_dB, int n_frames,
+                                    const int32_t* d_n_samples, const uint8_t* d_last, int64_t n_slots, int chunk_len,
+                                    int stride, int look_backward, const vadx_fsmn_serve_cfg* cfg, int32_t* d_state,
+                                    const float* d_caches_in, float* d_caches_out, int n_cache_blocks, int64_t cache_row,
+                                    int32_t* d_decisions, int32_t* d_events, int32_t* d_header, int32_t* h_events,
+                                    int32_t* h_header, void* d_scratch, size_t scratch_bytes, size_t* scratch_needed,
+                                    void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && n_frames >= 1 && stride >= 1 && stride < chunk_len && chunk_len <= kFsmnMaxChunk &&
+                   look_backward >= 0 && look_backward < n_frames,
+               "vadx_fsmn_serve_step: bad shape");
+  const ServeScratch sl(n_slots, 2 * (int64_t)n_frames + 2);
+  if (scratch_needed) *scratch_needed = sl.need;
+  if (!d_scratch) return VADX_OK;                   // size query
+  VADX_REQUIRE(scratch_bytes >= sl.need, "vadx_fsmn_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes, sl.need);
+  VADX_REQUIRE(d_score && d_noisy_dB && d_n_samples && d_last && cfg && d_state && d_decisions && d_events && d_header,
+               "vadx_fsmn_serve_step: null pointer");
+  VADX_REQUIRE(ld_score >= n_frames, "vadx_fsmn_serve_step: ld_score %lld < n_frames %d", (long long)ld_score, n_frames);
+  VADX_REQUIRE((d_caches_in == nullptr) == (d_caches_out == nullptr) && (!d_caches_out || (n_cache_blocks >= 1 && cache_row >= 1)),
+               "vadx_fsmn_serve_step: caches_in and caches_out go together, with n_cache_blocks and cache_row >= 1");
+  VADX_REQUIRE(!d_caches_out || d_caches_in != d_caches_out, "vadx_fsmn_serve_step: caches_out must not alias caches_in");
+  VADX_TRY(check_host_mirror(h_events, h_header, stream, "vadx_fsmn_serve_step"));
+  StageTimer _timer(VADX_STAGE_POSTPROC, (cudaStream_t)stream, "fsmn_serve_seg_kernel", 1.0 * n_slots * n_frames);
+  fsmn_serve_seg_kernel<<<(unsigned)sl.n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
+      d_score, ld_score, d_noisy_dB, n_frames, d_n_samples, d_last, n_slots, chunk_len, stride, look_backward, *cfg, d_state,
+      d_decisions, sl.staged(d_scratch), sl.counts(d_scratch), sl.action(d_scratch), sl.info(d_scratch));
+  VADX_TRY(after_launch("vadx_fsmn_serve_step"));
+  return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, d_caches_in, d_caches_out,
+                    n_cache_blocks, cache_row, stream, "vadx_fsmn_serve_step");
 }
 
 extern "C" int vadx_postprocess_frames(const float* d_probs, int64_t ld_probs, const int32_t* d_n_frames,

@@ -31,6 +31,12 @@ class StreamPostCfg(C.Structure):
                 ("min_speech_frame", C.c_int32), ("max_speech_frame", C.c_int32), ("min_silence_frame", C.c_int32)]
 
 
+class FsmnServeCfg(C.Structure):
+    _fields_ = [("speaking_score", C.c_double), ("silence_score", C.c_double), ("frame_duration", C.c_double),
+                ("fusion_threshold", C.c_double), ("min_speech_duration", C.c_double), ("snr_threshold", C.c_float),
+                ("noise_init", C.c_float)]
+
+
 _i64, _i32, _f32, _vp, _sz = C.c_int64, C.c_int, C.c_float, C.c_void_p, C.c_size_t
 
 # name -> (restype, argtypes); must list every symbol include/vadx.h declares (tests check this)
@@ -118,6 +124,10 @@ SIGNATURES = {
     "vadx_silero_serve_load": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "vadx_silero_serve_step": (C.c_int, [_vp, _i64, _vp, _vp, _i64, _i32, C.c_double, C.c_double, _vp, _vp, _vp, _vp, _vp,
                                          _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
+    "vadx_fsmn_serve_state_words": (C.c_int, [_i32]),
+    "vadx_fsmn_serve_load": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _f32, _vp, _vp, _vp]),
+    "vadx_fsmn_serve_step": (C.c_int, [_vp, _i64, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, C.POINTER(FsmnServeCfg), _vp,
+                                       _vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
     "vadx_create": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), _i32, C.POINTER(_vp)]),
     "vadx_destroy": (None, [_vp]),
     "vadx_set_tensor": (C.c_int, [_vp, C.c_char_p, _vp, _i32, C.POINTER(_i64), _i32]),

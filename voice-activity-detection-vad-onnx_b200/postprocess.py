@@ -311,6 +311,8 @@ class ServeTick:
     `frames` int32 [n_slots] (the frames of `probs` each slot consumed).  probs and frames are valid until the next
     tick; events, n_events and the host read-back until the tick after that."""
 
+    RANGE_TEXT = "n_samples outside [0, chunk_samples]"
+
     def __init__(self, owner, tick, parity, probs, frames, done):
         self._owner, self._tick, self._i, self._done = owner, tick, parity, done
         self.events, self.n_events, self.error = owner.events[parity], owner.header[parity][0:1], owner.header[parity][1:2]
@@ -325,7 +327,7 @@ class ServeTick:
         n, err = (int(v) for v in self._owner.h_header[self._i])
         events = [tuple(e) for e in self._owner.h_events[self._i][:n].tolist()]
         if err:
-            what = [m for b, m in ((SERVE_ERR_RANGE, "n_samples outside [0, chunk_samples]"),
+            what = [m for b, m in ((SERVE_ERR_RANGE, self.RANGE_TEXT),
                                    (SERVE_ERR_SHORT, "a short chunk that is not the stream's last")) if err & b]
             raise ServeTickError(f"stream server: rejected slot control words ({'; '.join(what)}); those slots were "
                                  "held, the events of the others are in .events", events, err)
@@ -524,10 +526,119 @@ class SileroSlotSegmenter:
         return t
 
 
-def load_tick_inputs(who, chunk, n_samples, last, dst_chunk, dst_n_samples, dst_last, device):
+class FsmnServeTick(ServeTick):
+    """One tick of the FSMN slot server (FsmnSlotSegmenter).  As ServeTick, but `events` hold (slot, kind, decision),
+    `frames` the decisions each slot made this tick and `probs` is the tick's score flags uint8 [n_slots, T].
+    host_seconds / host_indices give the reference's final timestamps (process_timestamps after runs_to_timestamps)."""
+
+    RANGE_TEXT = "n_samples outside [0, full_chunk(received)]"
+
+    def _converted(self, conv):
+        d = self._owner.frame_duration
+
+        def sec(kind, i):
+            """the reference's doubles (FSMN/Inference_FSMN_VAD_ONNX.py:124-141)"""
+            return i * d if kind == SERVE_START else (i * d + d if kind == SERVE_END else i * d)
+        try:
+            return [(s, k, conv(sec(k, int(i)))) for s, k, i in self.host_events()]
+        except ServeTickError as e:
+            e.events = [(s, k, conv(sec(k, int(i)))) for s, k, i in e.events]
+            raise
+
+    def host_seconds(self):
+        """-> [(slot, kind, seconds)]: START a*d, END b*d + d, END_OF_STREAM n*d, d = 160 / 16000.  Pairing one stream's
+        starts and ends gives its process_timestamps(runs_to_timestamps(...)) list.  A ServeTickError carries its events
+        in seconds."""
+        return self._converted(float)
+
+    def host_indices(self):
+        """-> [(slot, kind, sample)], int(seconds * 16000) as the reference's indices file writes them"""
+        sr = self._owner.sampling_rate
+        return self._converted(lambda v: int(v * sr))
+
+
+class FsmnSlotSegmenter:
+    """The look-ahead hysteresis, background level, timestamp machine and slot lifecycle of the FSMN slot server
+    (vadx_fsmn_serve_step) for n_slots slots: state (vadx_fsmn_serve_state_words int32 per slot), scratch, and two sets
+    of event buffers (device and pinned host) used by alternate ticks.  `step` runs it on given score flags uint8
+    [n_slots, T] (0 / 1, as the gate writes them) and noisy_dB fp32 [n_slots], without a model; a slot only consumes
+    them on ticks that run a window (see fsmn_vad.StreamServer).  Seconds per decision: 160 / 16000."""
+
+    sampling_rate = 16000
+    frame_duration = 160 / 16000
+
+    def __init__(self, n_slots: int, n_frames: int, chunk_len: int, look_backward: int, speaking_score: float = 0.5,
+                 silence_score: float = 0.5, snr_threshold: float = 1.0, noise_init: float = 4.0,
+                 fusion_threshold: float = 0.3, min_speech_duration: float = 0.2, device=None):
+        import torch
+        self.S, self.T, self.L, self.lb = int(n_slots), int(n_frames), int(chunk_len), int(look_backward)
+        self.stride = self.L - (self.lb + 1) * 160
+        self.cfg = lib.FsmnServeCfg(float(speaking_score), float(silence_score), self.frame_duration,
+                                    float(fusion_threshold), float(min_speech_duration), float(snr_threshold),
+                                    float(np.float32(noise_init)))
+        dev = device or torch.device("cuda", torch.cuda.current_device())
+        L = lib.load()
+        need = C.c_size_t()
+        lib.check(L.vadx_fsmn_serve_step(None, self.T, None, self.T, None, None, self.S, self.L, self.stride, self.lb,
+                                         C.byref(self.cfg), None, None, None, 0, 0, None, None, None, None, None, None, 0,
+                                         C.byref(need), None))
+        self.scratch = torch.empty((need.value,), dtype=torch.uint8, device=dev)
+        self.state = torch.zeros((self.S, L.vadx_fsmn_serve_state_words(self.lb)), dtype=torch.int32, device=dev)
+        self.frames = torch.zeros((self.S,), dtype=torch.int32, device=dev)
+        n_max = self.S * (2 * self.T + 2)
+        self.events = [torch.zeros((n_max, 3), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.header = [torch.zeros((2,), dtype=torch.int32, device=dev) for _ in range(2)]
+        self.h_events = [torch.zeros((n_max, 3), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.h_header = [torch.zeros((2,), dtype=torch.int32).pin_memory() for _ in range(2)]
+        self.ticks = 0
+
+    def full_chunk(self, received: int) -> int:
+        """samples of a full chunk for a stream that has sent `received` samples so far"""
+        return min(self.stride, self.L - received) if received < self.L else self.stride
+
+    def reset(self):
+        """every slot idle (state zeroed); the window buffer and caches are the caller's"""
+        self.state.zero_()
+
+    def enqueue(self, score, noisy_dB, n_samples, last, parity: int, caches_in=None, caches_out=None, stream=None):
+        """Enqueue vadx_fsmn_serve_step for one tick (no checks beyond pointers: the server checks shapes once)."""
+        c = caches_in
+        lib.check(lib.load().vadx_fsmn_serve_step(
+            score.data_ptr(), score.stride(0), noisy_dB.data_ptr(), self.T, n_samples.data_ptr(), last.data_ptr(), self.S,
+            self.L, self.stride, self.lb, C.byref(self.cfg), self.state.data_ptr(), lib.ptr(c), lib.ptr(caches_out),
+            c.shape[0] if c is not None else 0, (c.shape[2] * c.shape[3]) if c is not None else 0, self.frames.data_ptr(),
+            self.events[parity].data_ptr(), self.header[parity].data_ptr(), self.h_events[parity].data_ptr(),
+            self.h_header[parity].data_ptr(), self.scratch.data_ptr(), self.scratch.numel(), None, lib.stream_ptr(stream)))
+
+    def step(self, score, noisy_dB, n_samples, last, stream=None) -> FsmnServeTick:
+        """One tick on given CUDA tensors: score uint8 [n_slots, >= T] with contiguous rows, noisy_dB fp32 [n_slots],
+        n_samples int32 [n_slots], last bool / uint8 [n_slots]."""
+        import torch
+        if not (torch.is_tensor(score) and score.is_cuda and score.dtype == torch.uint8 and score.dim() == 2
+                and score.shape[0] == self.S and score.shape[1] >= self.T and score.stride(1) == 1):
+            raise ValueError(f"FsmnSlotSegmenter.step: score must be CUDA uint8 [{self.S}, >= {self.T}] with contiguous rows")
+        if not (torch.is_tensor(noisy_dB) and noisy_dB.is_cuda and noisy_dB.dtype == torch.float32
+                and tuple(noisy_dB.shape) == (self.S,) and noisy_dB.is_contiguous()):
+            raise ValueError(f"FsmnSlotSegmenter.step: noisy_dB must be a contiguous CUDA fp32 tensor [{self.S}]")
+        _check_control(n_samples, last, self.S, "FsmnSlotSegmenter.step", cuda=True)
+        i = self.ticks & 1
+        self.enqueue(score, noisy_dB, n_samples, last.view(torch.uint8), i, stream=stream)
+        return self.finish(i, score, stream)
+
+    def finish(self, parity, score, stream=None) -> FsmnServeTick:
+        import torch
+        done = torch.cuda.Event()
+        done.record(stream)
+        t = FsmnServeTick(self, self.ticks, parity, score, self.frames, done)
+        self.ticks += 1
+        return t
+
+
+def load_tick_inputs(who, chunk, n_samples, last, dst_chunk, dst_n_samples, dst_last, device, check_short: bool = True):
     """A slot server's step(chunk, n_samples, last): checks the arguments against the static buffers and copies them in
     (non-blocking from pinned host memory).  Host control words are checked here, before anything is copied; control
-    words already on the device are checked by the serve kernel.  None for all three leaves the buffers as they are."""
+    words already on the device are checked by the serve kernel.  None for all three leaves the buffers as they are.
+    check_short=False leaves the short-chunk rule to the device (a server whose full chunk depends on the slot's state)."""
     import torch
     given = [a is not None for a in (chunk, n_samples, last)]
     if any(given) and not all(given):
@@ -545,7 +656,7 @@ def load_tick_inputs(who, chunk, n_samples, last, dst_chunk, dst_n_samples, dst_
         n = n_samples.numpy()
         if n.min(initial=0) < 0 or n.max(initial=0) > L:
             raise ValueError(f"{who}: n_samples must be in [0, {L}]")
-        if not last.is_cuda:
+        if check_short and not last.is_cuda:
             short = (n > 0) & (n < L) & (last.view(torch.uint8).numpy() == 0)
             if short.any():
                 raise ValueError(f"{who}: slots {np.flatnonzero(short)[:8].tolist()} got a short chunk "

@@ -344,9 +344,12 @@ class FsmnSession:
         return [torch.zeros((n_streams,) + self.cache_shape, dtype=torch.float32, device=device)
                 for _ in range(self.cfg.fsmn_layers)]
 
-    def run_batch(self, audio, caches, noise_average_dB, one_minus_speech_threshold: float = 1.0, stream=None):
+    def run_batch(self, audio, caches, noise_average_dB, one_minus_speech_threshold: float = 1.0, stream=None, out=None,
+                  caches_out=None):
         """audio cuda int16 [S, L]; caches: list of cuda fp32 [S,128,19]; noise_average_dB cuda fp32 [S].
-        -> (score u8 [S,T], new_caches, noisy_dB [S], p_silence [S,T], power_dB [S,T]); asynchronous."""
+        -> (score u8 [S,T], new_caches, noisy_dB [S], p_silence [S,T], power_dB [S,T]); asynchronous.
+        out = (score, noisy_dB, p_silence, power_dB) and caches_out (a list like caches, distinct from it) are static
+        outputs to write instead of new tensors; p_silence and power_dB may be None there (not returned then)."""
         import torch
         if not (torch.is_tensor(audio) and audio.is_cuda and audio.dtype == torch.int16 and audio.dim() == 2
                 and audio.is_contiguous()):
@@ -365,11 +368,27 @@ class FsmnSession:
             self._e.set_scalar("one_minus_speech_threshold", self._thr)
         self._leave_window_mode()
         dev = audio.device
-        score = torch.empty((S, self.T), dtype=torch.uint8, device=dev)
-        noisy = torch.empty((S,), dtype=torch.float32, device=dev)
-        p_sil = torch.empty((S, self.T), dtype=torch.float32, device=dev)
-        power = torch.empty((S, self.T), dtype=torch.float32, device=dev)
-        new = [torch.empty_like(c) for c in caches]
+        if out is None:
+            score = torch.empty((S, self.T), dtype=torch.uint8, device=dev)
+            noisy = torch.empty((S,), dtype=torch.float32, device=dev)
+            p_sil = torch.empty((S, self.T), dtype=torch.float32, device=dev)
+            power = torch.empty((S, self.T), dtype=torch.float32, device=dev)
+        else:
+            score, noisy, p_sil, power = out
+            want = ((torch.uint8, (S, self.T)), (torch.float32, (S,)), (torch.float32, (S, self.T)), (torch.float32, (S, self.T)))
+            for i, (t, (dt, shape)) in enumerate(zip(out, want)):
+                if (t is None and i < 2) or (t is not None and not (t.is_cuda and t.dtype == dt and tuple(t.shape) == shape
+                                                                     and t.is_contiguous())):
+                    raise ValueError("run_batch: out must be contiguous CUDA (score u8 [S,T], noisy_dB fp32 [S], "
+                                     "p_silence fp32 [S,T] or None, power_dB fp32 [S,T] or None)")
+        if caches_out is None:
+            new = [torch.empty_like(c) for c in caches]
+        else:
+            new = list(caches_out)
+            if len(new) != n or any(tuple(c.shape) != tuple(ci.shape) or c.dtype != torch.float32 or not c.is_cuda
+                                    or not c.is_contiguous() or c.data_ptr() == ci.data_ptr() for c, ci in zip(new, caches)):
+                raise ValueError(f"run_batch: caches_out must be {n} contiguous CUDA fp32 caches of the caches' shape, "
+                                 "distinct from them")
         self._e.forward([audio, noise_average_dB], [score, noisy, p_sil, power], list(caches) + new, S, L, stream)
         return score, new, noisy, p_sil, power
 
