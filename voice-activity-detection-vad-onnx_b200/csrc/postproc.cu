@@ -648,6 +648,12 @@ __global__ void __launch_bounds__(128) stream_post_kernel(const float* __restric
 constexpr int kServeThreads = 128;
 enum : int8_t { kServeAdvance = 0, kServeHold = 1, kServeFinalize = 2 };
 
+// The control-word rule of every slot server: n outside [0, full] is out of range, and a chunk shorter than full must
+// be the stream's last.  Returns the slot's VADX_SERVE_ERR_* bits (0: the words are valid).
+__device__ __forceinline__ int serve_control_error(int n, bool fin, int full) {
+  return (n < 0 || n > full) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < full && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+}
+
 // Zero samples [n, frame_len) of every slot fed a short chunk: a chunk shorter than one frame is zero-padded to
 // one frame (the reference's np.pad, Inference_FireRed_ONNX.py:790-792); later frames of a short chunk lie wholly
 // inside its n samples, and whatever lies past them only reaches frames the server discards.
@@ -696,7 +702,7 @@ __global__ void __launch_bounds__(kServeThreads) stream_serve_seg_kernel(
   if (s < n_slots) {
     const int n = n_samples[s];
     const bool fin = last[s] != 0;
-    err = (n < 0 || n > chunk_samples) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < chunk_samples && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+    err = serve_control_error(n, fin, chunk_samples);
     int f = 0;
     if (err || (n == 0 && !fin)) {
       action[s] = kServeHold;                       // hold, or a rejected tick: the slot stays exactly as it was
@@ -861,7 +867,7 @@ __global__ void __launch_bounds__(kServeThreads) silero_serve_seg_kernel(
   if (s < n_slots) {
     const int n = n_samples[s];
     const bool fin = last[s] != 0;
-    err = (n < 0 || n > chunk_samples) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < chunk_samples && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+    err = serve_control_error(n, fin, chunk_samples);
     int nw = 0;
     if (!err && (n > 0 || fin)) {
       int32_t* st = state + s * kSileroServeStateWords;
@@ -936,7 +942,7 @@ __host__ __device__ __forceinline__ int fsmn_serve_words(int look_backward) { re
 // that never got a sample).  Load and step decide alike.
 __device__ __forceinline__ int fsmn_serve_plan(int n, bool fin, int received, int chunk_len, int stride, int& err) {
   const int full = received < chunk_len ? min(stride, chunk_len - received) : stride;
-  err = (n < 0 || n > full) ? VADX_SERVE_ERR_RANGE : (n > 0 && n < full && !fin) ? VADX_SERVE_ERR_SHORT : 0;
+  err = serve_control_error(n, fin, full);
   if (err || (n == 0 && !fin)) return kFsmnHold;
   if (received < chunk_len) {
     if (received + n < chunk_len && !fin) return kFsmnFill;

@@ -11,7 +11,7 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from . import audio_io, postprocess as PP, weights as W
+from . import audio_io, postprocess as PP, serve, weights as W
 from .session import FireRedSession, FireRedStreamSession
 
 IN_SAMPLE_RATE = 16000
@@ -264,29 +264,6 @@ def stream_frame_plan(lengths, chunk_samples: int = STREAM_CHUNK_SAMPLES):
     return np.clip(np.minimum(f, valid[None, :] - before), 0, None).astype(np.int32)
 
 
-class _StreamGraphRunner:
-    """Two captured tick bodies, body(0) (caches a -> b) and body(1) (b -> a), over static buffers: a 160 ms step is
-    ~30 small launches, so eager execution is bound by host launch cost; replay costs one graph launch."""
-
-    def __init__(self, body):
-        self.body = body
-        self.graphs = [None, None]
-
-    def step(self, k: int):
-        """runs body(k & 1)"""
-        import torch
-        i = k & 1
-        if self.graphs[i] is None:
-            self.body(i)                             # this step runs eagerly (constants, workspace) ...
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):                # ... and is recorded (not executed) for the later ones
-                self.body(i)
-            self.graphs[i] = g
-        else:
-            self.graphs[i].replay()
-
-
 class _LockStep:
     """Static buffers of run_stream_vad_streams(graph=True) for one (streams, chunk) shape."""
 
@@ -298,7 +275,7 @@ class _LockStep:
         self.out = torch.empty((S, 1, T), dtype=torch.float32, device=device)
         self.n_frames = torch.zeros((S,), dtype=torch.int32, device=device)
         self.caches = [session.new_caches(S, device), session.new_caches(S, device)]
-        self.runner = _StreamGraphRunner(self._body)
+        self.runner = serve._StreamGraphRunner(self._body)
 
     def _body(self, i: int):
         self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
@@ -365,7 +342,7 @@ def run_stream_vad_streams(session: FireRedStreamSession, audio, lengths, chunk_
     return probs.reshape(S, n_calls * T), post, a, plan
 
 
-class StreamServer:
+class StreamServer(serve.SlotServer):
     """Live Stream-VAD serving: n_slots independent stream slots advance one tick per chunk of chunk_samples.  A stream
     may start in any free slot on any tick.  Per tick and slot the caller gives the chunk (int16 [chunk_samples]), the
     number of valid samples n and a `last` flag:
@@ -399,22 +376,15 @@ class StreamServer:
             raise ValueError(f"StreamServer: n_slots must be in [1, {FireRedSession.MAX_STREAMS_PER_CALL}], got {n_slots}")
         if int(chunk_samples) < WINDOW_LENGTH:
             raise ValueError(f"StreamServer: chunk_samples must be at least one frame ({WINDOW_LENGTH}), got {chunk_samples}")
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        if dev.index is None:
-            dev = torch.device("cuda", torch.cuda.current_device())
-        self.session, self.S, self.chunk_samples, self.device = session, int(n_slots), int(chunk_samples), dev
+        self.session, self.chunk_samples = session, int(chunk_samples)
+        super().__init__(n_slots, self.chunk_samples, device, graph)
         self.T = session.frames(self.chunk_samples)
-        self.chunk = torch.zeros((self.S, self.chunk_samples), dtype=torch.int16, device=dev)
-        self.n_samples = torch.zeros((self.S,), dtype=torch.int32, device=dev)
-        self.last = torch.zeros((self.S,), dtype=torch.uint8, device=dev)
-        self.out = torch.zeros((self.S, 1, self.T), dtype=torch.float32, device=dev)
-        self.caches = [session.new_caches(self.S, dev), session.new_caches(self.S, dev)]
-        with torch.cuda.device(dev):
-            self.seg = PP.StreamSlotSegmenter(smooth_window_size, speech_threshold, pad_start_frame, min_speech_frame,
-                                              max_speech_frame, min_silence_frame, self.S, self.T, self.chunk_samples,
-                                              WINDOW_LENGTH, HOP_LENGTH, dev, frames_per_second)
-        self._runner = _StreamGraphRunner(self._tick) if graph else None
-        self._k = 0
+        self.out = torch.zeros((self.S, 1, self.T), dtype=torch.float32, device=self.device)
+        self.caches = [session.new_caches(self.S, self.device), session.new_caches(self.S, self.device)]
+        with torch.cuda.device(self.device):
+            self.seg = serve.StreamSlotSegmenter(smooth_window_size, speech_threshold, pad_start_frame, min_speech_frame,
+                                                 max_speech_frame, min_silence_frame, self.S, self.T, self.chunk_samples,
+                                                 WINDOW_LENGTH, HOP_LENGTH, self.device, frames_per_second)
 
     def _tick(self, i: int):
         """the tick body on the static buffers, caches[i] -> caches[1 - i]; only libvadx launches"""
@@ -425,20 +395,8 @@ class StreamServer:
         self.session.run_batch(self.chunk, self.caches[i], out=self.out, caches_out=self.caches[1 - i])
         self.seg.enqueue(self.out[:, 0, :], self.n_samples, self.last, i, self.caches[i], self.caches[1 - i])
 
-    def step(self, chunk=None, n_samples=None, last=None) -> PP.ServeTick:
-        """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, chunk_samples], n_samples int32
-        [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
-        for all three runs the tick on what the static buffers hold.  Returns the tick's handle (PP.ServeTick)."""
-        import torch
-        with torch.cuda.device(self.device):
-            PP.load_tick_inputs("StreamServer.step", chunk, n_samples, last, self.chunk, self.n_samples, self.last,
-                                self.device)
-            if self._runner is not None:
-                self._runner.step(self._k)
-            else:
-                self._tick(self._k & 1)
-            self._k += 1
-            return self.seg.finish((self._k - 1) & 1, self.out[:, 0, :])
+    def _tick_probs(self):
+        return self.out[:, 0, :]
 
 
 def run_stream_vad(audio, session: FireRedStreamSession, chunk_samples: int = STREAM_CHUNK_SAMPLES) -> StreamVadResult:

@@ -13,8 +13,7 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from . import audio_io, lib, postprocess as PP, weights as W
-from .firered_vad import _StreamGraphRunner
+from . import audio_io, lib, postprocess as PP, serve, weights as W
 from .session import FsmnSession
 
 SAMPLE_RATE = 16000
@@ -171,7 +170,7 @@ def _run_streams_graph(session, aligned, stride, look_backward_s, thr, snr_thres
     return r.state
 
 
-class StreamServer:
+class StreamServer(serve.SlotServer):
     """Live FSMN-VAD serving with the reference's final timestamps as events: n_slots independent stream slots advance
     one reference window per tick.  A stream may start in any free slot on any tick.  Windows follow the reference
     (audio_io.align_overlapping): window k covers samples [k*stride, k*stride + L), L = session.chunk_len,
@@ -189,14 +188,17 @@ class StreamServer:
     raw int16: the reference's whole-file peak normalisation is not causal, so the offline twin is
     run_vad(..., normalize=False).  Each tick is the window load, one forward of the session over [n_slots][L], the
     look-ahead hysteresis, the level update, the timestamp machine and the event compaction, replayed as one CUDA graph
-    per cache parity.  Its result (PP.FsmnServeTick) is a compact list of (slot, kind, decision) events, each emitted as
+    per cache parity.  Its result (serve.FsmnServeTick) is a compact list of (slot, kind, decision) events, each emitted as
     soon as it is certain: kind 0 = a segment starts, 1 = it ends (closed by silence decision b), 2 = it was open when
     the stream ended.  host_seconds() / host_indices() give exactly the reference's final timestamps (minimum duration
     and fusion applied).  Decisions count from the stream's first window, so a stream may run 2^31 of them.
 
     The defaults are the module constants, which are the reference's.  Inputs go through the static buffers `chunk`,
     `n_samples`, `last`: step() copies the arguments it is given into them (non-blocking from pinned host memory), or a
-    producer writes them and calls step() with no arguments.  The session stays usable between ticks."""
+    producer writes them and calls step() with no arguments.  Whether a chunk is full depends on the slot's samples so
+    far, so the device checks that rule.  The session stays usable between ticks."""
+
+    check_short = False
 
     def __init__(self, session: FsmnSession, n_slots: int, look_backward_s: float = LOOK_BACKWARD,
                  one_minus_speech_threshold: float = ONE_MINUS_SPEECH_THRESHOLD, snr_threshold_db: float = SNR_THRESHOLD,
@@ -215,15 +217,11 @@ class StreamServer:
             raise ValueError(f"StreamServer: a {L}-sample window is too short for a look-backward of {lb} frames")
         if L % 8:
             raise ValueError(f"StreamServer: the session's chunk_len {L} must be a multiple of 8")
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        if dev.index is None:
-            dev = torch.device("cuda", torch.cuda.current_device())
-        self.session, self.S, self.L, self.T, self.lb, self.stride, self.device = session, S, L, T, lb, stride, dev
+        self.session, self.L, self.T, self.lb, self.stride = session, L, T, lb, stride
+        super().__init__(S, stride, device, graph)
+        dev = self.device
         self.thr = float(one_minus_speech_threshold)
         self.noise_init = float(np.float32(noise_init_db + snr_threshold_db) * np.float32(0.1))
-        self.chunk = torch.zeros((S, stride), dtype=torch.int16, device=dev)
-        self.n_samples = torch.zeros((S,), dtype=torch.int32, device=dev)
-        self.last = torch.zeros((S,), dtype=torch.uint8, device=dev)
         self.window = torch.zeros((S, L), dtype=torch.int16, device=dev)      # the forward's input, one row per slot
         self.noise_avg = torch.zeros((S,), dtype=torch.float32, device=dev)  # the gate's level, written by the load
         self.score = torch.zeros((S, T), dtype=torch.uint8, device=dev)
@@ -231,10 +229,8 @@ class StreamServer:
         self.caches = [torch.zeros((session.cfg.fsmn_layers, S) + session.cache_shape, dtype=torch.float32, device=dev)
                        for _ in range(2)]
         with torch.cuda.device(dev):
-            self.seg = PP.FsmnSlotSegmenter(S, T, L, lb, speaking_score, silence_score, snr_threshold_db * 0.1,
-                                            self.noise_init, fusion_threshold, min_speech_duration, dev)
-        self._runner = _StreamGraphRunner(self._tick) if graph else None
-        self._k = 0
+            self.seg = serve.FsmnSlotSegmenter(S, T, L, lb, speaking_score, silence_score, snr_threshold_db * 0.1,
+                                               self.noise_init, fusion_threshold, min_speech_duration, dev)
 
     def full_chunk(self, received: int) -> int:
         """samples of a full chunk for a stream that has sent `received` samples so far"""
@@ -250,21 +246,8 @@ class StreamServer:
                                out=(self.score, self.noisy, None, None), caches_out=self.caches[1 - i].unbind(0))
         self.seg.enqueue(self.score, self.noisy, self.n_samples, self.last, i, self.caches[i], self.caches[1 - i])
 
-    def step(self, chunk=None, n_samples=None, last=None) -> PP.FsmnServeTick:
-        """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, stride], n_samples int32
-        [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
-        for all three runs the tick on what the static buffers hold.  Whether a chunk is full depends on the slot's
-        samples so far, so the device checks that rule.  Returns the tick's handle (PP.FsmnServeTick)."""
-        import torch
-        with torch.cuda.device(self.device):
-            PP.load_tick_inputs("StreamServer.step", chunk, n_samples, last, self.chunk, self.n_samples, self.last,
-                                self.device, check_short=False)
-            if self._runner is not None:
-                self._runner.step(self._k)
-            else:
-                self._tick(self._k & 1)
-            self._k += 1
-            return self.seg.finish((self._k - 1) & 1, self.score)
+    def _tick_probs(self):
+        return self.score
 
 
 def run_vad(audio, session: FsmnSession, look_backward_s: float = LOOK_BACKWARD, rng=None,

@@ -12,8 +12,8 @@ import ctypes as C
 
 import numpy as np
 
-from . import audio_io, lib, postprocess as PP, weights as W
-from .firered_vad import VadResult, _StreamGraphRunner
+from . import audio_io, lib, postprocess as PP, serve, weights as W
+from .firered_vad import VadResult
 from .session import SileroSession
 
 use_fp16 = False
@@ -181,7 +181,7 @@ class VADIterator:
         return None
 
 
-class StreamServer:
+class StreamServer(serve.SlotServer):
     """Live Silero serving with VADIterator events: n_slots independent stream slots advance one tick of
     windows_per_tick (W) 512-sample windows at a time (W = 5: 160 ms, W = 1: VADIterator's 32 ms cadence).  A stream
     may start in any free slot on any tick.  Per tick and slot the caller gives the chunk (int16 [W*512]), the number of
@@ -195,7 +195,7 @@ class StreamServer:
     A slot consumes ceil(n/512) windows; a short last window is zero-padded to 512, as get_speech_timestamps pads it.
     Samples past n never influence a result.  Each tick is the int16 load, one forward of the session over all slots
     and W windows, the iterator and the event compaction, replayed as one CUDA graph per LSTM-state parity.  Its result
-    (PP.SileroServeTick) is a compact list of (slot, kind, window) events: kind 0 = start (the window the iterator
+    (serve.SileroServeTick) is a compact list of (slot, kind, window) events: kind 0 = start (the window the iterator
     triggered on), 1 = end (the window the silence began on, VADIterator's temp_end), 2 = the stream ended while
     triggered (the windows consumed; the reference would leave that segment open).  host_samples() / host_seconds()
     give exactly what VADIterator returns.  Windows count from the stream's first window, so a stream may run 2^31
@@ -222,22 +222,14 @@ class StreamServer:
         if S * W > SileroSession.MAX_ROWS_PER_CALL:
             raise ValueError(f"StreamServer: n_slots * windows_per_tick must be at most {SileroSession.MAX_ROWS_PER_CALL}, "
                              f"got {S * W}")
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        if dev.index is None:
-            dev = torch.device("cuda", torch.cuda.current_device())
-        self.session, self.S, self.W, self.device = session, S, W, dev
-        self.chunk_samples = W * c.window
+        self.session, self.W, self.chunk_samples = session, W, W * c.window
+        super().__init__(S, self.chunk_samples, device, graph)
         self.row_stride = c.context + self.chunk_samples
-        self.chunk = torch.zeros((S, self.chunk_samples), dtype=torch.int16, device=dev)
-        self.n_samples = torch.zeros((S,), dtype=torch.int32, device=dev)
-        self.last = torch.zeros((S,), dtype=torch.uint8, device=dev)
-        self.x = torch.zeros((S, self.row_stride), dtype=torch.float32, device=dev)     # [context | chunk] per slot
-        self.out = torch.zeros((W, S, 1), dtype=torch.float32, device=dev)
-        self.state = [torch.zeros((2, S, c.hidden), dtype=torch.float32, device=dev) for _ in range(2)]
-        with torch.cuda.device(dev):
-            self.seg = PP.SileroSlotSegmenter(threshold, min_silence_duration_ms, speech_pad_ms, S, W, dev)
-        self._runner = _StreamGraphRunner(self._tick) if graph else None
-        self._k = 0
+        self.x = torch.zeros((S, self.row_stride), dtype=torch.float32, device=self.device)  # [context | chunk] per slot
+        self.out = torch.zeros((W, S, 1), dtype=torch.float32, device=self.device)
+        self.state = [torch.zeros((2, S, c.hidden), dtype=torch.float32, device=self.device) for _ in range(2)]
+        with torch.cuda.device(self.device):
+            self.seg = serve.SileroSlotSegmenter(threshold, min_silence_duration_ms, speech_pad_ms, S, W, self.device)
 
     def _tick(self, i: int):
         """the tick body on the static buffers; only libvadx launches"""
@@ -246,20 +238,8 @@ class StreamServer:
         self.session.forward_windows(self.x, self.out, self.state[i], self.state[1 - i], self.W, self.row_stride)
         self.seg.enqueue(self.out[:, :, 0], self.n_samples, self.last, i, self.x, self.state[i], self.state[1 - i])
 
-    def step(self, chunk=None, n_samples=None, last=None) -> PP.SileroServeTick:
-        """Enqueue one tick on the current stream (asynchronous).  chunk int16 [n_slots, W*512], n_samples int32
-        [n_slots], last bool / uint8 [n_slots]: CUDA tensors, or host tensors (pinned for a non-blocking copy); None
-        for all three runs the tick on what the static buffers hold.  Returns the tick's handle (PP.SileroServeTick)."""
-        import torch
-        with torch.cuda.device(self.device):
-            PP.load_tick_inputs("StreamServer.step", chunk, n_samples, last, self.chunk, self.n_samples, self.last,
-                                self.device)
-            if self._runner is not None:
-                self._runner.step(self._k)
-            else:
-                self._tick(self._k & 1)
-            self._k += 1
-            return self.seg.finish((self._k - 1) & 1, self.out[:, :, 0])
+    def _tick_probs(self):
+        return self.out[:, :, 0].t()
 
 
 def run_vad(audio, model: SileroSession, save_timestamps_second: str | None = None,
