@@ -591,6 +591,38 @@ int vadx_fsmn_serve_step(const uint8_t* d_score, int64_t ld_score, const float* 
                          int32_t* d_events, int32_t* d_header, int32_t* h_events, int32_t* h_header, void* d_scratch,
                          size_t scratch_bytes, size_t* scratch_needed, void* stream);
 
+/* MarbleNet slot server: n_slots independent MarbleNet Frame-VAD streams, one static-axis window of window_samples = L
+ * samples per tick (the reference's non-overlapping windows, audio_io.align_non_overlapping), of which the model's first
+ * n_frames = F = T' - 1 frames count (signal_len).  Per tick and slot s the caller gives d_n_samples[s] in [0, L] and
+ * d_last[s] with the four actions of the slot servers above and the same VADX_SERVE_ERR_* rules (a full chunk is L).
+ * A fed tick consumes F frames; a short last chunk is zero-padded to L by vadx_stream_serve_zero_tail (frame_len = L)
+ * before the forward.  The model keeps no state across windows, so there are no caches.
+ *
+ * vadx_marblenet_serve_step runs AFTER the forward on its active-class probabilities d_probs [n_slots][ld_probs]:
+ *   - runs the reference's VadPostprocessor (the passes of vadx_postprocess_frames: smoothing, the four-state machine,
+ *     the rising-edge extension by the smoothing window, the gap merge, the dilation, the max-speech split at the first
+ *     arg-min of the raw probabilities) online, one thread per slot.  A frame's decision before the split is final
+ *     D = D2 + D3 + D4 + D5 frames after it, D2 = max(min_speech, 1) (0 when min_speech <= 0 and min_silence <= 0),
+ *     D3 = ws (when ws > 1), D4 = max(merge - 1, 0), D5 = max(extend, 0): at most max(min_speech, 1) + ws + merge +
+ *     extend, 15 frames at MarbleNet's defaults.  Finalize flushes what is still in flight as the whole-track passes
+ *     treat a track's end.  The state is d_state [n_slots][vadx_marblenet_serve_state_words(cfg)] int32, all zero = a
+ *     fresh slot; D is at most 65536.  Writes the frames consumed to d_frames [n_slots];
+ *   - writes the events to d_events [n][3] int32 (slot, kind, value) / d_header {n, error bits} and the optional pinned
+ *     host mirror, as vadx_stream_serve_step does: VADX_SERVE_START a (a final segment starts at frame a, time
+ *     float32(a) * frame_shift), VADX_SERVE_END b (it ends before frame b, max-speech cuts included),
+ *     VADX_SERVE_END_OF_STREAM (the last segment was open at finalize): the value is the bit pattern of the reference's
+ *     float32 end, n * frame_shift after n frames, replaced by samples / 16000 when that is smaller (compared in double,
+ *     then rounded to float32; samples is a 64-bit count in the state).  Frames count from the stream's first window as
+ *     int32, so a stream may run 2^31 frames.  A tick stages at most 2 (F + D) + 2 events per slot; d_events must hold
+ *     n_slots * (2 * (n_frames + D) + 2) triples.
+ * d_scratch = NULL: only writes the scratch size to *scratch_needed and returns. */
+int vadx_marblenet_serve_state_words(const vadx_post_cfg* cfg);
+int vadx_marblenet_serve_step(const float* d_probs, int64_t ld_probs, int n_frames, const int32_t* d_n_samples,
+                              const uint8_t* d_last, int64_t n_slots, int window_samples, const vadx_post_cfg* cfg,
+                              float frame_shift, int32_t* d_state, int32_t* d_frames, int32_t* d_events,
+                              int32_t* d_header, int32_t* h_events, int32_t* h_header, void* d_scratch,
+                              size_t scratch_bytes, size_t* scratch_needed, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Model-level API: the replacement for InferenceSession(...).run(...)
  * ------------------------------------------------------------------------------------------ */

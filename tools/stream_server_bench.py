@@ -1,5 +1,5 @@
 """Slot server throughput on one GPU: FireRed Stream-VAD (firered_vad.StreamServer, the default) or, with
---family silero, Silero (silero_vad.StreamServer).
+--family silero / fsmn / marblenet, that family's StreamServer.
 
 For each slot count, at full occupancy and under churn (about 1 % of slots closing and joining per tick, 10 % held):
   device ms per tick      CUDA events around the tick's graph replay (inputs already in the static buffers)
@@ -15,6 +15,10 @@ With --family fsmn (fsmn_vad.StreamServer), for each slot count and window lengt
 7520, look-backward 0.3 s), the same rows with ticks of one reference window (stride = L - 31 * 160 samples), plus the
 bare forward of the same [n_slots][L] shape as one CUDA graph and the lock-step run_streams(graph=True) time per window,
 both alternating with the server in this process; realtime streams = n_slots * stride / 16000 / tick.
+With --family marblenet (marblenet_vad.StreamServer), for each slot count and window (--window-samples, default 16000
+and 32000), the same rows with ticks of one static-axis window and traffic drawn from synth-enveloped chunks, plus the
+bare forward (MarbleNetSession.run_batch over the same [n_slots][L] into a static output, one CUDA graph), alternating
+with the server in this process; realtime streams = n_slots * L / 16000 / tick.
 Prints one JSON line (card name and power limit read in the same run); --out also writes it to a file, --trace writes
 the torch.profiler launch list of a few server ticks.
 
@@ -24,6 +28,8 @@ the torch.profiler launch list of a few server ticks.
       --trace profiles/r04_launches_silero_server.txt
   python tools/stream_server_bench.py --family fsmn --slots 4096,16384 --out profiles/r05_fsmn_server.json \
       --trace profiles/r05_launches_fsmn_server.txt
+  python tools/stream_server_bench.py --family marblenet --slots 4096,16384 --window-samples 16000,32000 \
+      --out profiles/r06_marblenet_server.json --trace profiles/r06_launches_marblenet_server.txt
 """
 from __future__ import annotations
 
@@ -340,11 +346,85 @@ def main_fsmn(a, info):
             "look_backward_s": lb_s, "ticks": a.ticks, "rounds": a.rounds, "results": rows}
 
 
+class MarbleNetTraffic(Traffic):
+    """Traffic whose chunks are drawn from a pool of synth-enveloped windows (speech-like bursts and pauses), so that
+    segments keep opening and closing after warm-up"""
+
+    def __init__(self, S, C, churn, hold, seed, n_pool=2):
+        import torch
+        from vadx import synth
+        super().__init__(S, C, churn, hold, seed, n_pool=0)
+        self.chunks = [torch.from_numpy(synth.synth_streams(S, C, seed=seed + i)).pin_memory() for i in range(n_pool)]
+
+
+class MarbleNetForward:
+    """the bare forward of a MarbleNet server tick: MarbleNetSession.run_batch over [S][L] rows into a static output,
+    captured as one CUDA graph on buffers of its own"""
+
+    def __init__(self, session, S, L):
+        import torch
+        g = torch.Generator(device="cuda").manual_seed(S + L)
+        self.session = session
+        self.x = torch.randint(-8000, 8000, (S, L), generator=g, device="cuda", dtype=torch.int16)
+        self.out = torch.empty((2, S, session.frames(L)), dtype=torch.float32, device="cuda")
+        self._run()
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self._run()
+
+    def _run(self):
+        self.session.run_batch(self.x, out=self.out)
+
+    time = SileroForward.time
+
+
+def main_marblenet(a, info):
+    import torch
+    import vadx
+    from vadx import marblenet_vad as MV, weights as W
+    cfg = W.MarbleNetConfig()
+    sess = vadx.MarbleNetSession(W.marblenet_random_init(cfg, 0), cfg)
+    rows = []
+    for L in [int(v) for v in a.window_samples.split(",")]:
+        for S in [int(v) for v in a.slots.split(",")]:
+            fwd = MarbleNetForward(sess, S, L)
+            for mode, churn, hold in (("full", 0.0, 0.0), ("churn", 0.01, 0.10)):
+                traffic = MarbleNetTraffic(S, L, churn, hold, seed=S + L + len(mode))
+                server = MV.StreamServer(sess, S, window_samples=L)
+                res = {"dev": [], "host": [], "events": [], "d2h": [], "fwd": []}
+                for _ in range(a.rounds):
+                    d, h, e, b = bench_server(server, traffic, a.ticks, a.warmup)
+                    res["dev"].append(d), res["host"].append(h), res["events"].append(e), res["d2h"].append(b)
+                    res["fwd"].append(fwd.time(a.ticks))
+                dev = float(np.median(res["dev"]))
+                bare = float(np.median(res["fwd"]))
+                row = {"window_samples": L, "frames_per_tick": server.F, "n_slots": S, "traffic": mode,
+                       "device_ms_per_tick": round(dev, 4), "device_ms_per_tick_rounds": [round(v, 4) for v in res["dev"]],
+                       "host_ms_per_tick": round(float(np.median(res["host"])), 4),
+                       "events_per_tick": round(float(np.mean(res["events"])), 2),
+                       "d2h_bytes_per_tick": round(float(np.mean(res["d2h"])), 1),
+                       "realtime_streams": int(S * L / 16000 / (dev / 1e3)),
+                       "forward_ms": round(bare, 4), "forward_ms_rounds": [round(v, 4) for v in res["fwd"]],
+                       "tick_over_forward": round(dev / bare, 3)}
+                rows.append(row)
+                print(json.dumps(row), file=sys.stderr)
+                if a.trace and len(rows) == 1:
+                    write_trace(a.trace, server, traffic, f"marblenet StreamServer, L = {L}, {S} slots, 5 ticks, {info}")
+                del server, traffic
+                torch.cuda.empty_cache()
+            del fwd
+            torch.cuda.empty_cache()
+    return {"what": "marblenet StreamServer tick vs the bare forward of the same shape", "card": info,
+            "ticks": a.ticks, "rounds": a.rounds, "results": rows}
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
-    ap.add_argument("--family", choices=("firered", "silero", "fsmn"), default="firered")
+    ap.add_argument("--family", choices=("firered", "silero", "fsmn", "marblenet"), default="firered")
     ap.add_argument("--chunk-lens", default="16000,7520", help="fsmn: window lengths to measure")
     ap.add_argument("--windows", default="5,1", help="silero: windows per tick to measure")
+    ap.add_argument("--window-samples", default="16000,32000", help="marblenet: samples per tick (window) to measure")
     ap.add_argument("--slots", default="4096,16384")
     ap.add_argument("--ticks", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=20)
@@ -359,8 +439,8 @@ def main(argv=None):
         raise SystemExit("stream_server_bench: needs a CUDA device")
     torch.cuda.set_device(0)
     info = card()
-    if a.family in ("silero", "fsmn"):
-        out = main_silero(a, info) if a.family == "silero" else main_fsmn(a, info)
+    if a.family in ("silero", "fsmn", "marblenet"):
+        out = {"silero": main_silero, "fsmn": main_fsmn, "marblenet": main_marblenet}[a.family](a, info)
         line = json.dumps(out)
         print(line)
         if a.out:

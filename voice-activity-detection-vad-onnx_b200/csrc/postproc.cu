@@ -1122,6 +1122,241 @@ __global__ void __launch_bounds__(kServeThreads) fsmn_serve_seg_kernel(
   serve_block_totals(count, err, block_info);
 }
 
+// ---- MarbleNet slot server (vadx_marblenet_serve_step) ----
+// The reference's VadPostprocessor (oracle/postproc.frame_decisions + segments_from_decisions, the passes of
+// postprocess_frames_runs_kernel) online: each whole-track pass only reaches a bounded number of frames back, so it
+// becomes a stage with a fixed delay that hands final decisions, in frame order, to the next one:
+//   2. the four-state machine back-fills at most D2 = max(min_speech, 1) frames (0 in the plain-threshold case);
+//   3. a rising edge at t sets [t - ws, t) (D3 = ws when ws > 1);
+//   4. a gap [g, t) is filled when t - g < merge, so t <= g + merge - 1 (D4 = max(merge - 1, 0));
+//   5. dilation by extend is "a 1 in [f - extend, f + extend]" (D5 = max(extend, 0), no ring: the latest 1 suffices);
+//   6. the max-speech split runs on the final decisions with a running first-minimum of the raw probabilities.
+// A frame's pre-split decision is final D = D2 + D3 + D4 + D5 frames after it (16 at MarbleNet's defaults; D <= K =
+// max(min_speech, 1) + ws + merge + extend).  Stages 2-4 keep their provisional decisions in bit rings of D_i + 1 bits
+// (a back-fill never reaches past the ring), the split reads the raw probabilities from a ring of D + 1 floats.
+// State words per slot: 0 frames consumed, 1..2 samples consumed (int64, low word first), 3 running sum (float bits),
+// 4 machine state, 5 t_sp, 6 t_si, 7 previous stage-3 input, 8 previous stage-4 input, 9 gap start + 1 (0 = none),
+// 10 latest stage-5 speech frame + 1 (0 = none), 11 in a run, 12 piece start, 13 piece START emitted, 14 running
+// minimum (float bits), 15 its frame, then the running-sum ring [ws] (ws > 1), the probability ring [D + 1] and the
+// bit rings of stages 2, 3, 4.  All zero = a fresh slot.
+constexpr int kMnHeader = 16;
+constexpr int kMnMaxDelay = 1 << 16;       // keeps a slot's state words and staged events well inside int
+
+struct MnLayout {
+  int ws, D2, D3, D4, D5, D, o_cs, o_p, o_r2, o_r3, o_r4, words;
+  __host__ __device__ explicit MnLayout(const vadx_post_cfg& c) {
+    ws = c.smooth_window < 1 ? 1 : c.smooth_window;
+    D2 = (c.min_speech_frame <= 0 && c.min_silence_frame <= 0) ? 0 : (c.min_speech_frame > 1 ? c.min_speech_frame : 1);
+    D3 = ws > 1 ? ws : 0;
+    D4 = c.merge_silence_frame > 1 ? c.merge_silence_frame - 1 : 0;
+    D5 = c.extend_speech_frame > 0 ? c.extend_speech_frame : 0;
+    D = D2 + D3 + D4 + D5;
+    o_cs = kMnHeader;
+    o_p = o_cs + (ws > 1 ? ws : 0);
+    o_r2 = o_p + D + 1;
+    o_r3 = o_r2 + (D2 + 32) / 32;
+    o_r4 = o_r3 + (D3 + 32) / 32;
+    words = o_r4 + (D4 + 32) / 32;
+  }
+};
+
+struct MnSeg {
+  const MnLayout lay;
+  int32_t* st;
+  int max_sf, half, min_sp, min_si, merge, extend;
+  int t, mode, t_sp, t_si, prev3, prev4, gap, l1, in_run, pos, started, best_i;
+  float run, best;
+  int2* ev;
+  int count;
+
+  __device__ __forceinline__ bool bit(int off, int size, int f) const {
+    const int i = f % size;
+    return ((uint32_t)st[off + (i >> 5)] >> (i & 31)) & 1u;
+  }
+  __device__ __forceinline__ void set_bit(int off, int size, int f, bool v) {
+    const int i = f % size;
+    const uint32_t m = 1u << (i & 31), w = (uint32_t)st[off + (i >> 5)];
+    st[off + (i >> 5)] = (int32_t)(v ? (w | m) : (w & ~m));
+  }
+  __device__ __forceinline__ void push(int kind, int v) { ev[count++] = make_int2(kind, v); }
+  __device__ __forceinline__ void reset_min() { best = INFINITY; best_i = 0; }
+
+  // 6: the max-speech split on final decisions, in frame order.  A START leaves once its frame can no longer be cut:
+  // at once for max_speech >= 2 (a cut lies at least half >= 1 past the piece start), with the piece's END for 1.
+  __device__ __forceinline__ void in6(int f, bool d) {
+    const bool defer = max_sf == 1;
+    if (d) {
+      if (!in_run) {
+        in_run = 1; pos = f; started = 0; reset_min();
+        if (!defer) { push(VADX_SERVE_START, f); started = 1; }
+      } else if (max_sf >= 1 && f == pos + max_sf) {   // frame pos + max is speech: cut at the first arg-min
+        const int cut = best_i;
+        if (cut > pos) {
+          if (!started) push(VADX_SERVE_START, pos);
+          push(VADX_SERVE_END, cut);
+        }
+        pos = cut + 1; started = 0; reset_min();           // the next window starts at cut + 1 + half >= f
+        if (!defer) { push(VADX_SERVE_START, pos); started = 1; }
+      }
+      if (max_sf >= 1 && f >= pos + half) {
+        const float p = __int_as_float(st[lay.o_p + f % (lay.D + 1)]);
+        if (p < best) { best = p; best_i = f; }
+      }
+    } else if (in_run) {
+      if (!started) push(VADX_SERVE_START, pos);
+      push(VADX_SERVE_END, f);
+      in_run = 0;
+    }
+  }
+  // 5: dilation by extend
+  __device__ __forceinline__ bool dilated(int f) const { return l1 > 0 && l1 - 1 >= f - extend; }
+  __device__ __forceinline__ void in5(int i, bool b) {
+    if (lay.D5 == 0) { in6(i, b); return; }
+    if (b) l1 = i + 1;
+    if (i - lay.D5 >= 0) in6(i - lay.D5, dilated(i - lay.D5));
+  }
+  // 4: gaps shorter than merge are filled
+  __device__ __forceinline__ void in4(int i, bool b) {
+    if (lay.D4 == 0) { in5(i, b); return; }
+    const int R = lay.D4 + 1;
+    set_bit(lay.o_r4, R, i, b);
+    if (i >= 1) {
+      if (prev4 && !b && gap == 0) {
+        gap = i + 1;
+      } else if (!prev4 && b && gap > 0) {
+        if (i - (gap - 1) < merge)
+          for (int g = gap - 1; g < i; ++g) set_bit(lay.o_r4, R, g, true);
+        gap = 0;
+      }
+    }
+    prev4 = b;
+    if (i - lay.D4 >= 0) in5(i - lay.D4, bit(lay.o_r4, R, i - lay.D4));
+  }
+  // 3: rising edges move left by ws
+  __device__ __forceinline__ void in3(int i, bool b) {
+    if (lay.D3 == 0) { in4(i, b); return; }
+    const int R = lay.D3 + 1;
+    set_bit(lay.o_r3, R, i, b);
+    if (i >= 1 && b && !prev3)
+      for (int g = i - lay.ws < 0 ? 0 : i - lay.ws; g < i; ++g) set_bit(lay.o_r3, R, g, true);
+    prev3 = b;
+    if (i - lay.D3 >= 0) in4(i - lay.D3, bit(lay.o_r3, R, i - lay.D3));
+  }
+  // 1 + 2: smoothing with postprocess_frames_runs_kernel's rounding, then the four-state machine.  The mean of the
+  // stream's first ws - 1 frames divides by u + 1; its flag comes in as early_hot (see early_flags).
+  __device__ __forceinline__ void frame(float p, bool early_hot) {
+    const int u = t++;
+    st[lay.o_p + u % (lay.D + 1)] = __float_as_int(p);
+    bool hot = p >= __int_as_float(thr_bits);
+    if (lay.ws > 1) {
+      const int k = lay.o_cs + u % lay.ws;
+      const float old = __int_as_float(st[k]);           // the running sum ws frames back (0 before the stream)
+      run = __fadd_rn(run, p);
+      hot = u < lay.ws - 1 ? early_hot
+                           : __fmul_rn(__fsub_rn(run, old), (float)(1.0 / (double)lay.ws)) >= __int_as_float(thr_bits);
+      st[k] = __float_as_int(run);
+    }
+    if (lay.D2 == 0) { in3(u, hot); return; }
+    const int R = lay.D2 + 1;
+    if (mode == 0) {
+      if (hot) { mode = 1; t_sp = u; }
+    } else if (mode == 1) {
+      if (!hot) {
+        mode = 0;
+      } else if (u - t_sp >= min_sp) {
+        mode = 2;
+        for (int g = t_sp; g < u; ++g) set_bit(lay.o_r2, R, g, true);   // u - t_sp == D2
+      }
+    } else if (mode == 2) {
+      if (!hot) { mode = 3; t_si = u; }
+    } else {
+      if (hot) mode = 2;
+      else if (u - t_si >= min_si) mode = 0;
+    }
+    set_bit(lay.o_r2, R, u, mode >= 2);
+    if (u - lay.D2 >= 0) in3(u - lay.D2, bit(lay.o_r2, R, u - lay.D2));
+  }
+  // finalize: every stage flushes its delay line in order (a MAYBE_SP stretch stays silence, an open gap is not
+  // merged, dilation runs to n), then a run reaching n ends the stream
+  __device__ __forceinline__ void finish(float frame_shift, int64_t samples) {
+    const int n = t;
+    if (lay.D2) for (int o = n - lay.D2 < 0 ? 0 : n - lay.D2; o < n; ++o) in3(o, bit(lay.o_r2, lay.D2 + 1, o));
+    if (lay.D3) for (int o = n - lay.D3 < 0 ? 0 : n - lay.D3; o < n; ++o) in4(o, bit(lay.o_r3, lay.D3 + 1, o));
+    if (lay.D4) for (int o = n - lay.D4 < 0 ? 0 : n - lay.D4; o < n; ++o) in5(o, bit(lay.o_r4, lay.D4 + 1, o));
+    if (lay.D5) for (int o = n - lay.D5 < 0 ? 0 : n - lay.D5; o < n; ++o) in6(o, dilated(o));
+    if (in_run) {
+      if (!started) push(VADX_SERVE_START, pos);
+      // PP.segments_to_seconds: n * fs in float32, replaced by the recording's duration when that is smaller
+      const float e = __fmul_rn(__int2float_rn(n), frame_shift);
+      const double dur = __ddiv_rn((double)samples, 16000.0);
+      push(VADX_SERVE_END_OF_STREAM, __float_as_int(dur < (double)e ? __double2float_rn(dur) : e));
+    }
+  }
+  int32_t thr_bits;
+};
+
+// Thread per slot, after the forward: validate the slot's control words, run the online post-processor over the F
+// frames of a fed tick (none on a hold or a finalize without audio), and stage the events (kind, value) in `staged`
+// [S][2 (F + D) + 2].  The split stage receives at most F + D frames in a tick (F new ones, and D more when finalize
+// flushes the delay lines); each of them emits at most one START (a run opens, a piece starts after a cut, or a deferred
+// START leaves with its END) and one END (a cut or a run's end), and finalize adds at most a deferred START and the
+// END_OF_STREAM.
+__global__ void __launch_bounds__(kServeThreads) marblenet_serve_seg_kernel(
+    const float* __restrict__ probs, int64_t ld_probs, int F, const int32_t* __restrict__ n_samples,
+    const uint8_t* __restrict__ last, int64_t n_slots, int window_samples, const vadx_post_cfg cfg, float frame_shift,
+    int32_t* __restrict__ state, int32_t* __restrict__ frames_out, int32_t* __restrict__ staged,
+    int32_t* __restrict__ counts, int8_t* __restrict__ action, int32_t* __restrict__ block_info) {
+  const int64_t s = (int64_t)blockIdx.x * kServeThreads + threadIdx.x;
+  int count = 0, err = 0;
+  if (s < n_slots) {
+    const int n = n_samples[s];
+    const bool fin = last[s] != 0;
+    err = serve_control_error(n, fin, window_samples);
+    int f = 0;
+    if (err || (n == 0 && !fin)) {
+      action[s] = kServeHold;                       // hold, or a rejected tick: the slot stays exactly as it was
+    } else {
+      const MnLayout lay(cfg);
+      int32_t* st = state + s * (int64_t)lay.words;
+      const int64_t cap = 2 * ((int64_t)F + lay.D) + 2;
+      MnSeg g{lay, st, cfg.max_speech_frame, cfg.max_speech_frame >> 1, cfg.min_speech_frame, cfg.min_silence_frame,
+              cfg.merge_silence_frame, cfg.extend_speech_frame, st[0], st[4], st[5], st[6], st[7], st[8], st[9], st[10],
+              st[11], st[12], st[13], st[15], __int_as_float(st[3]), __int_as_float(st[14]),
+              reinterpret_cast<int2*>(staged) + s * cap, 0, __float_as_int(cfg.threshold)};
+      const int64_t samples = ((int64_t)(uint32_t)st[1] | ((int64_t)st[2] << 32)) + n;
+      if (n > 0) {
+        f = F;
+        const float* p = probs + s * ld_probs;
+        // flags of the frames u < ws - 1 (at most 63: ws <= kMaxSmooth), in a loop of their own so that the division's
+        // slow-path call does not make the main loop spill
+        uint64_t early = 0;
+        const int n_early = min(F, lay.ws - 1 - g.t);
+        float r = g.run;
+        for (int k = 0; k < n_early; ++k) {
+          r = __fadd_rn(r, __ldg(p + k));
+          if (__fdiv_rn(r, (float)(g.t + k + 1)) >= cfg.threshold) early |= 1ull << k;
+        }
+        for (int k = 0; k < F; ++k) g.frame(__ldg(p + k), k < n_early && ((early >> k) & 1));
+      }
+      if (fin) {
+        g.finish(frame_shift, samples);
+        for (int i = 0; i < lay.words; ++i) st[i] = 0;   // the next stream in this slot starts fresh
+        action[s] = kServeFinalize;
+      } else {
+        st[0] = g.t; st[1] = (int32_t)(uint32_t)samples; st[2] = (int32_t)(samples >> 32);
+        st[3] = __float_as_int(g.run); st[4] = g.mode; st[5] = g.t_sp; st[6] = g.t_si; st[7] = g.prev3; st[8] = g.prev4;
+        st[9] = g.gap; st[10] = g.l1; st[11] = g.in_run; st[12] = g.pos; st[13] = g.started;
+        st[14] = __float_as_int(g.best); st[15] = g.best_i;
+        action[s] = kServeAdvance;
+      }
+      count = g.count;
+    }
+    frames_out[s] = f;
+    counts[s] = count;
+  }
+  serve_block_totals(count, err, block_info);
+}
+
 }  // namespace vadx
 
 using namespace vadx;
@@ -1328,6 +1563,43 @@ extern "C" int vadx_fsmn_serve_step(const uint8_t* d_score, int64_t ld_score, co
   VADX_TRY(after_launch("vadx_fsmn_serve_step"));
   return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, d_caches_in, d_caches_out,
                     n_cache_blocks, cache_row, stream, "vadx_fsmn_serve_step");
+}
+
+extern "C" int vadx_marblenet_serve_state_words(const vadx_post_cfg* cfg) {
+  VADX_REQUIRE(cfg, "vadx_marblenet_serve_state_words: null pointer");
+  VADX_REQUIRE(MnLayout(*cfg).D <= kMnMaxDelay, "vadx_marblenet_serve_state_words: a decision delay of %d frames > %d",
+               MnLayout(*cfg).D, kMnMaxDelay);
+  return MnLayout(*cfg).words;
+}
+
+extern "C" int vadx_marblenet_serve_step(const float* d_probs, int64_t ld_probs, int n_frames, const int32_t* d_n_samples,
+                                         const uint8_t* d_last, int64_t n_slots, int window_samples,
+                                         const vadx_post_cfg* cfg, float frame_shift, int32_t* d_state, int32_t* d_frames,
+                                         int32_t* d_events, int32_t* d_header, int32_t* h_events, int32_t* h_header,
+                                         void* d_scratch, size_t scratch_bytes, size_t* scratch_needed, void* stream) {
+  VADX_REQUIRE(n_slots >= 1 && n_frames >= 1 && window_samples >= 1, "vadx_marblenet_serve_step: bad shape");
+  VADX_REQUIRE(cfg, "vadx_marblenet_serve_step: null pointer");
+  const MnLayout lay(*cfg);
+  VADX_REQUIRE(lay.D <= kMnMaxDelay, "vadx_marblenet_serve_step: a decision delay of %d frames > %d", lay.D, kMnMaxDelay);
+  VADX_REQUIRE(cfg->smooth_window <= kMaxSmooth, "vadx_marblenet_serve_step: smooth_window %d > %d", cfg->smooth_window,
+               kMaxSmooth);
+  const ServeScratch sl(n_slots, 2 * ((int64_t)n_frames + lay.D) + 2);
+  if (scratch_needed) *scratch_needed = sl.need;
+  if (!d_scratch) return VADX_OK;                   // size query
+  VADX_REQUIRE(scratch_bytes >= sl.need, "vadx_marblenet_serve_step: scratch of %zu bytes, %zu needed", scratch_bytes,
+               sl.need);
+  VADX_REQUIRE(d_probs && d_n_samples && d_last && d_state && d_frames && d_events && d_header,
+               "vadx_marblenet_serve_step: null pointer");
+  VADX_REQUIRE(ld_probs >= n_frames, "vadx_marblenet_serve_step: ld_probs %lld < n_frames %d", (long long)ld_probs,
+               n_frames);
+  VADX_TRY(check_host_mirror(h_events, h_header, stream, "vadx_marblenet_serve_step"));
+  StageTimer _timer(VADX_STAGE_POSTPROC, (cudaStream_t)stream, "marblenet_serve_seg_kernel", 4.0 * n_slots * n_frames);
+  marblenet_serve_seg_kernel<<<(unsigned)sl.n_blocks, kServeThreads, 0, (cudaStream_t)stream>>>(
+      d_probs, ld_probs, n_frames, d_n_samples, d_last, n_slots, window_samples, *cfg, frame_shift, d_state, d_frames,
+      sl.staged(d_scratch), sl.counts(d_scratch), sl.action(d_scratch), sl.info(d_scratch));
+  VADX_TRY(after_launch("vadx_marblenet_serve_step"));
+  return serve_emit(sl, n_slots, d_scratch, d_events, d_header, h_events, h_header, nullptr, nullptr, 0, 0, stream,
+                    "vadx_marblenet_serve_step");
 }
 
 extern "C" int vadx_postprocess_frames(const float* d_probs, int64_t ld_probs, const int32_t* d_n_frames,

@@ -128,6 +128,9 @@ SIGNATURES = {
     "vadx_fsmn_serve_load": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _f32, _vp, _vp, _vp]),
     "vadx_fsmn_serve_step": (C.c_int, [_vp, _i64, _vp, _i32, _vp, _vp, _i64, _i32, _i32, _i32, C.POINTER(FsmnServeCfg), _vp,
                                        _vp, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
+    "vadx_marblenet_serve_state_words": (C.c_int, [C.POINTER(PostCfg)]),
+    "vadx_marblenet_serve_step": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _i64, _i32, C.POINTER(PostCfg), _f32, _vp, _vp,
+                                            _vp, _vp, _vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]),
     "vadx_create": (C.c_int, [C.c_char_p, C.POINTER(C.c_int32), _i32, C.POINTER(_vp)]),
     "vadx_destroy": (None, [_vp]),
     "vadx_set_tensor": (C.c_int, [_vp, C.c_char_p, _vp, _i32, C.POINTER(_i64), _i32]),

@@ -5,7 +5,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from . import audio_io, postprocess as PP, weights as W
+from . import audio_io, lib, postprocess as PP, serve, weights as W
 from .firered_vad import VadResult
 from .session import MarbleNetSession
 
@@ -58,6 +58,69 @@ def run_vad_windows(session: MarbleNetSession, windows, post: PP.FramePostConfig
     probs = scores[1, :, :n].reshape(S, n_win * n)
     dec, cnt, seg = PP.postprocess_frames(probs, post, None, stream=stream)
     return probs, dec, cnt, seg
+
+
+class StreamServer(serve.SlotServer):
+    """Live MarbleNet Frame-VAD serving with the reference's timestamps as events: n_slots independent stream slots
+    advance one static-axis window of L = window_samples samples per tick, the reference's non-overlapping windows
+    (audio_io.align_non_overlapping), of which the first F = session.frames(L) - 1 frames count (signal_len).  At
+    L = 16000 a tick is 1 s of 50 frames.  A stream may start in any free slot on any tick.  Per tick and slot the caller
+    gives the chunk (int16 [L]), the number of valid samples n and a `last` flag:
+
+        n > 0, last 0   feed a full chunk (n == L)
+        n > 0, last 1   feed the stream's last chunk (may be short), then finalize and free the slot
+        n = 0, last 0   hold: the slot is unchanged
+        n = 0, last 1   finalize and free the slot without new audio
+
+    A short last chunk is zero-padded to L (the reference pads with RMS-matched noise from the unseeded global numpy
+    generator), so the offline twin is run_vad(..., input_audio_length=L) with zero noise.  Audio is raw int16:
+    normalise_audio is off by default in the reference and is not causal.  Each tick is the tail zeroing, one forward of
+    the session over [n_slots][L] and the online VadPostprocessor with the event compaction (vadx_marblenet_serve_step),
+    replayed as a CUDA graph.  Its result (serve.MarbleNetServeTick) is a compact list of (slot, kind, value) events, each
+    emitted as soon as it is certain: kind 0 = a segment starts at frame a, 1 = it ends before frame b (max-speech cuts
+    included), 2 = it was open when the stream ended (the value is the reference's float32 end).  host_seconds() /
+    host_indices() give exactly run_vad's timestamps.  Frames count from the stream's first window as int32, so a
+    stream may run 2^31 frames.
+
+    `post` is the post-processor's configuration (the reference's module constants by default).  Inputs go through the
+    static buffers `chunk`, `n_samples`, `last`: step() copies the arguments it is given into them (non-blocking from
+    pinned host memory), or a producer writes them and calls step() with no arguments.  `probs` is the tick's active
+    probabilities fp32 [n_slots, F] (a view of the forward's static output).  The session stays usable between ticks."""
+
+    def __init__(self, session: MarbleNetSession, n_slots: int, window_samples: int = 16000,
+                 post: PP.FramePostConfig = POST_DEFAULT, device=None, graph: bool = True):
+        import torch
+        if not isinstance(session, MarbleNetSession):
+            raise ValueError("StreamServer needs a MarbleNetSession")
+        if session.in_sample_rate != IN_SAMPLE_RATE:
+            raise ValueError(f"StreamServer: the session must take {IN_SAMPLE_RATE} Hz audio, not {session.in_sample_rate}")
+        S, L = int(n_slots), int(window_samples)
+        if S < 1:
+            raise ValueError(f"StreamServer: n_slots must be at least 1, got {n_slots}")
+        if L < 1:
+            raise ValueError(f"StreamServer: window_samples must be at least 1, got {window_samples}")
+        T = session.frames(L)
+        F = T - 1
+        if F < 1:
+            raise ValueError(f"StreamServer: a {L}-sample window gives no frame (signal_len = {F})")
+        if post.tail_adds_frame_length:
+            raise ValueError("StreamServer: MarbleNet's open tail ends at n * frame_shift (post.tail_adds_frame_length "
+                             "must be False)")
+        self.session, self.L, self.T, self.F, self.post = session, L, T, F, post
+        super().__init__(S, L, device, graph)
+        self.scores = torch.zeros((2, S, T), dtype=torch.float32, device=self.device)   # the forward's static output
+        with torch.cuda.device(self.device):
+            self.seg = serve.MarbleNetSlotSegmenter(post, S, F, L, self.device)
+
+    def _tick(self, i: int):
+        """the tick body on the static buffers; only libvadx launches (the model keeps no state, so i is unused)"""
+        lib.check(lib.load().vadx_stream_serve_zero_tail(self.chunk.data_ptr(), self.L, self.n_samples.data_ptr(), self.S,
+                                                         self.L, self.L, lib.stream_ptr()))
+        self.session.run_batch(self.chunk, out=self.scores)
+        self.seg.enqueue(self._tick_probs(), self.n_samples, self.last, i)
+
+    def _tick_probs(self):
+        return self.scores[1, :, :self.F]
 
 
 def run_vad(audio, session: MarbleNetSession, post: PP.FramePostConfig = POST_DEFAULT, normalize: bool = False,

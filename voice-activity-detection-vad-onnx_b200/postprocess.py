@@ -19,8 +19,8 @@ import numpy as np
 from . import lib
 # The slot servers' host side lives in serve.py; its public names stay importable from here, where callers found them.
 from .serve import (SERVE_END, SERVE_END_OF_STREAM, SERVE_ERR_RANGE, SERVE_ERR_SHORT, SERVE_START,  # noqa: F401
-                    FsmnServeTick, FsmnSlotSegmenter, ServeTick, ServeTickError, SileroServeTick, SileroSlotSegmenter,
-                    StreamSlotSegmenter, load_tick_inputs)
+                    FsmnServeTick, FsmnSlotSegmenter, MarbleNetServeTick, MarbleNetSlotSegmenter, ServeTick,
+                    ServeTickError, SileroServeTick, SileroSlotSegmenter, StreamSlotSegmenter, load_tick_inputs)
 
 
 @dataclass(frozen=True)

@@ -1,6 +1,6 @@
-"""Host side of the slot servers (firered_vad, silero_vad and fsmn_vad.StreamServer): the control words and their
-checks, the segmenters with their two parities of event buffers, the tick handles, and the CUDA-graph runner of a tick
-body.  The device side is the vadx_*_serve_* entry points of csrc/postproc.cu (include/vadx.h)."""
+"""Host side of the slot servers (firered_vad, silero_vad, fsmn_vad and marblenet_vad.StreamServer): the control words
+and their checks, the segmenters with their two parities of event buffers, the tick handles, and the CUDA-graph runner
+of a tick body.  The device side is the vadx_*_serve_* entry points of csrc/postproc.cu (include/vadx.h)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -314,6 +314,79 @@ class FsmnSlotSegmenter(_SlotSegmenter):
         return self._step(score, n_samples, last, stream, score, noisy_dB)
 
 
+class MarbleNetServeTick(ServeTick):
+    """One tick of the MarbleNet slot server (MarbleNetSlotSegmenter).  As ServeTick, but `events` hold (slot, kind,
+    value): a frame for START / END, the bit pattern of the reference's float32 end for END_OF_STREAM.  host_seconds /
+    host_indices give the reference's timestamps (VadPostprocessor.decision_to_segment)."""
+
+    def _seconds(self, kind, v):
+        """round(float32(frame) * float32(frame_shift), 3), or the float32 end of an open last segment"""
+        if kind == SERVE_END_OF_STREAM:
+            return round(float(np.array(v, np.int32).view(np.float32)), 3)
+        return round(float(np.float32(v) * self._owner.fs), 3)
+
+    def host_seconds(self):
+        """-> [(slot, kind, seconds)].  Pairing one stream's starts and ends gives its marblenet_vad.run_vad timestamps.
+        A ServeTickError carries its events in seconds."""
+        return self._converted(self._seconds)
+
+    def host_indices(self):
+        """-> [(slot, kind, sample)], int(seconds * 16000) as the reference's indices file writes them"""
+        return self._converted(lambda k, v: int(self._seconds(k, v) * 16000))
+
+
+class MarbleNetSlotSegmenter(_SlotSegmenter):
+    """The reference's VadPostprocessor, online, and the slot lifecycle of the MarbleNet slot server
+    (vadx_marblenet_serve_step) for n_slots slots of F frames per tick: state (vadx_marblenet_serve_state_words int32 per
+    slot), scratch, and two sets of event buffers (device and pinned host) used by alternate ticks.  `step` runs it on
+    given probabilities fp32 [n_slots, >= F], without a model; a fed slot consumes all F frames (a short last chunk is
+    zero-padded to the window).  `post` is a postprocess.FramePostConfig whose open tail ends at n * frame_shift."""
+
+    tick_class = MarbleNetServeTick
+
+    def __init__(self, post, n_slots: int, n_frames: int, window_samples: int, device=None):
+        if post.tail_adds_frame_length:
+            raise ValueError("MarbleNetSlotSegmenter: the open tail of MarbleNet's post-processor ends at n * frame_shift "
+                             "(post.tail_adds_frame_length must be False)")
+        self.cfg = post.c_struct()
+        self.fs = np.float32(post.frame_shift_s)
+        self.S, self.F, self.L = int(n_slots), int(n_frames), int(window_samples)
+        L = lib.load()
+        words = L.vadx_marblenet_serve_state_words(C.byref(self.cfg))
+        if words < 0:
+            lib.check(words)
+        need = C.c_size_t()
+        lib.check(L.vadx_marblenet_serve_step(None, self.F, self.F, None, None, self.S, self.L, C.byref(self.cfg),
+                                              float(self.fs), None, None, None, None, None, None, None, 0, C.byref(need),
+                                              None))
+        self.events_per_slot = 2 * (self.F + self.delay) + 2
+        super().__init__(words, need.value, self.events_per_slot, device)
+
+    @property
+    def delay(self) -> int:
+        """frames after which a decision before the max-speech split is final (include/vadx.h)"""
+        c = self.cfg
+        d2 = 0 if c.min_speech_frame <= 0 and c.min_silence_frame <= 0 else max(c.min_speech_frame, 1)
+        return d2 + (c.smooth_window if c.smooth_window > 1 else 0) + max(c.merge_silence_frame - 1, 0) + \
+            max(c.extend_speech_frame, 0)
+
+    def enqueue(self, probs, n_samples, last, parity: int, stream=None):
+        """Enqueue vadx_marblenet_serve_step for one tick (no checks beyond pointers: the server checks shapes once)."""
+        lib.check(lib.load().vadx_marblenet_serve_step(
+            probs.data_ptr(), probs.stride(0), self.F, n_samples.data_ptr(), last.data_ptr(), self.S, self.L,
+            C.byref(self.cfg), float(self.fs), self.state.data_ptr(), *self._outputs(parity), lib.stream_ptr(stream)))
+
+    def step(self, probs, n_samples, last, stream=None) -> MarbleNetServeTick:
+        """One tick on given CUDA tensors: probs fp32 [n_slots, >= F] with contiguous rows, n_samples int32 [n_slots]
+        (in [0, window_samples]), last bool / uint8 [n_slots]."""
+        import torch
+        if not (torch.is_tensor(probs) and probs.is_cuda and probs.dtype == torch.float32 and probs.dim() == 2
+                and probs.shape[0] == self.S and probs.shape[1] >= self.F and probs.stride(1) == 1):
+            raise ValueError(f"MarbleNetSlotSegmenter.step: probs must be CUDA fp32 [{self.S}, >= {self.F}] with "
+                             "contiguous rows")
+        return self._step(probs, n_samples, last, stream, probs)
+
+
 def load_tick_inputs(who, chunk, n_samples, last, dst_chunk, dst_n_samples, dst_last, device, check_short: bool = True):
     """A slot server's step(chunk, n_samples, last): checks the arguments against the static buffers and copies them in
     (non-blocking from pinned host memory).  Host control words are checked here, before anything is copied; control
@@ -383,7 +456,7 @@ class _StreamGraphRunner:
 
 
 class SlotServer:
-    """What the three StreamServers share: the device, the static input buffers `chunk` int16 [n_slots, chunk width],
+    """What the four StreamServers share: the device, the static input buffers `chunk` int16 [n_slots, chunk width],
     `n_samples` int32 [n_slots] and `last` uint8 [n_slots], the optional graph runner and step().  A family sets `seg`
     (its segmenter) and defines _tick(i), the tick body on the static buffers with model state parity i (only libvadx
     launches, so it can be captured), and _tick_probs(), the tensor a tick's handle exposes as `probs`."""

@@ -512,8 +512,9 @@ class MarbleNetSession:
         """T' = frames emitted; the graph's `signal_len` output is T' - 1."""
         return self._e.output_frames(n_samples)
 
-    def run_batch(self, audio, stream=None):
-        """audio cuda int16 [S, L] -> scores cuda fp32 [2, S, T'] (plane 0 silence, plane 1 active)."""
+    def run_batch(self, audio, stream=None, out=None):
+        """audio cuda int16 [S, L] -> scores cuda fp32 [2, S, T'] (plane 0 silence, plane 1 active).  out: an optional
+        contiguous CUDA fp32 [2, S, T'] the scores are written to (a static output, so a call can be captured)."""
         import torch
         if not (torch.is_tensor(audio) and audio.is_cuda and audio.dtype == torch.int16 and audio.dim() == 2
                 and audio.is_contiguous()):
@@ -522,16 +523,26 @@ class MarbleNetSession:
         if L < 1:
             raise ValueError("InvalidArgument: empty audio")
         T = self.frames(L)
-        out = torch.empty((2, S, T), dtype=torch.float32, device=audio.device)
+        if out is None:
+            out = torch.empty((2, S, T), dtype=torch.float32, device=audio.device)
+            fresh = True
+        else:
+            if not (torch.is_tensor(out) and out.device == audio.device and out.dtype == torch.float32
+                    and tuple(out.shape) == (2, S, T) and out.is_contiguous()):
+                raise ValueError(f"run_batch: out must be a contiguous fp32 tensor [2, {S}, {T}] on {audio.device}")
+            fresh = False
         step = self.MAX_STREAMS_PER_CALL
         if S <= step:
             self._e.forward([audio], [out[0], out[1]], [], S, L, stream)
             return out
         for s0 in range(0, S, step):
             s1 = min(S, s0 + step)
-            part = torch.empty((2, s1 - s0, T), dtype=torch.float32, device=audio.device)
-            self._e.forward([audio[s0:s1]], [part[0], part[1]], [], s1 - s0, L, stream)
-            out[:, s0:s1] = part
+            if fresh:
+                part = torch.empty((2, s1 - s0, T), dtype=torch.float32, device=audio.device)
+                self._e.forward([audio[s0:s1]], [part[0], part[1]], [], s1 - s0, L, stream)
+                out[:, s0:s1] = part
+            else:                                    # the planes' row ranges are contiguous: no temporary
+                self._e.forward([audio[s0:s1]], [out[0, s0:s1], out[1, s0:s1]], [], s1 - s0, L, stream)
         return out
 
     def run(self, output_names, input_feed: dict):
